@@ -4,7 +4,7 @@
 Workload (BASELINE.json configs[1]): 80-dim Kaldi fbank + SpecAugment (2 time + 2 frequency masks) +
 per-utterance CMVN on a batch of 256 x 8-s 16 kHz utterances per GPU (synthetic, seeded).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -21,6 +21,10 @@ global CMVN = accumulate -> ONE all-reduce of 161 doubles -> apply, the all-redu
 region).  `cpu_baseline` = the reference path (torchaudio's kaldi.fbank + masking transforms, as
 lid/audio_processor.py calls them) on the box's host cores (rank 0, N=1 only), all cores and one core.
 --impl reference times that CPU path as the reference arm.
+
+--dump-outputs DIR writes what the headline's last timed step returned (rank 0): DIR/features.npy, float32
+[128, 798, 80], the features of a fixed seeded sample of 128 of the batch's 256 utterances (the whole batch is 65 MB).
+The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +48,7 @@ ALG_BYTES_PER_FRAME = 160 * 4 + N_MELS * 4             # SURVEY.md §8(d): 640 B
 ALG_FLOP_PER_FRAME = 15.0e3                            # SURVEY.md §8(d)
 METRIC = "audio-sec/sec 80-dim fbank+SpecAugment+CMVN"
 WORKLOAD = "cfg2: 80-dim kaldi fbank + SpecAugment(t_mask=0.05,f_mask=27,x2) + per-utterance CMVN, 256 x 8-s utterances per GPU"
+DUMP_UTTS, DUMP_SEED = 128, 0
 
 
 # ------------------------------------------------------------------------------------------------
@@ -154,6 +159,20 @@ def emit(line):
     out = _JSON_OUT if _JSON_OUT is not None else sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
+
+
+def dump_pick():
+    """The utterances --dump-outputs keeps: a fixed seeded sample of DUMP_UTTS of the B_UTTS, in batch order."""
+    import torch
+    return torch.randperm(B_UTTS, generator=torch.Generator().manual_seed(DUMP_SEED))[:DUMP_UTTS].sort().values
+
+
+def write_outputs(out_dir, arrays):
+    """DIR/<name>.npy per array, float32 as computed."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().numpy())
 
 
 def config_dict(world):
@@ -310,6 +329,10 @@ def run_gpu_arm(args):
     ms_total = ev0.elapsed_time(ev1)
     launches = lib.lidfe_launch_count() - launches0
     kernel_ms = fe.profile_end()
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # taken now: the sections below overwrite the rotating output sets
+        dump = {"features": outs[(args.warmup + args.steps - 1) % NBUF].index_select(0, dump_pick().to(dev)).cpu()}
 
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -485,6 +508,8 @@ def run_gpu_arm(args):
             cfg5 = cfg5_device.run(B=128, n_check=8, steps=3)
             if cfg5 is not None:
                 cfg5.pop("consumer", None)
+            else:
+                cfg5 = {"unavailable": "the reference's model source is not staged in baseline/_ref/lid"}
         except Exception as ex:       # the consumer is not the product: never let it take the bench line down
             cfg5 = {"unavailable": "%s: %s" % (type(ex).__name__, ex)}
 
@@ -576,6 +601,8 @@ def run_gpu_arm(args):
             "gpu_launches": int(launches),
             "roofline": roofline,
             "cpu_baseline": cpu}
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -676,7 +703,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the features of the last timed step (a fixed sample of the batch) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     keep_stdout_clean()
     if args.impl == "reference":

@@ -515,3 +515,24 @@ def test_cfg5_reference_consumer_on_device():
     assert r["consumer_worst_abs_diff"] <= 1e-3, r["consumer"]
     assert r["consumer_min_argmax_agreement"] >= 0.995, r["consumer"]
     assert 0.0 < r["frontend_share"] < 1.0
+
+
+@gpu
+def test_cfg5_conformer_consumer_on_device():
+    """Row A10 where the reference's model source is not staged: the same consumer check through a stand-in Conformer of
+    the reference model's shape (tools/cfg5_device.stand_in_model: torchaudio.models.Conformer, random init, eval).  The
+    oracle's features are pinned to the reference's own outputs (tests/golden/), so this still compares the kernel with
+    the reference's arithmetic as seen by a Conformer consumer; the convolutions run in plain fp32 (no TF32), so that
+    only the two feature sets differ."""
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    import cfg5_device
+    tf32 = torch.backends.cudnn.allow_tf32
+    torch.backends.cudnn.allow_tf32 = False
+    try:
+        r = cfg5_device.run(B=16, n_check=8, steps=1, model=cfg5_device.stand_in_model())
+    finally:
+        torch.backends.cudnn.allow_tf32 = tf32
+    assert r["features_norm_rel_vs_oracle"] <= 3e-4
+    assert r["consumer_worst_abs_diff"] <= 1e-3, r["consumer"]
+    assert r["consumer_min_argmax_agreement"] >= 0.995, r["consumer"]
+    assert 0.0 < r["frontend_share"] < 1.0

@@ -349,3 +349,27 @@ def test_pack_host_gathers_and_zeroes_gaps():
         assert lib.lidfe_pack_host(dst.data_ptr(), ptrs, ll(offs[::-1]), ll(lens), len(ws), eb, total, 1) == _lib.E_OFFSETS
         assert lib.lidfe_pack_host(dst.data_ptr(), ptrs, ll(offs), ll(lens), len(ws), eb, pos - 1000, 1) == _lib.E_OFFSETS
         assert lib.lidfe_pack_host(None, ptrs, ll(offs), ll(lens), len(ws), eb, total, 1) == _lib.E_NULL
+
+
+def test_bench_dump_outputs_sample_and_files(tmp_path):
+    """bench.py --dump-outputs: the same utterances every run (two builds are compared on them), float32 .npy files
+    named after the arrays, under 64 MB for the whole dump; bad arguments are refused before any device work."""
+    import subprocess
+    import sys
+    import bench
+    pick = bench.dump_pick()
+    assert torch.equal(pick, bench.dump_pick())
+    assert pick.numel() == bench.DUMP_UTTS == 128 and torch.equal(pick, pick.unique())
+    assert 0 <= int(pick[0]) and int(pick[-1]) < bench.B_UTTS
+    assert pick[:8].tolist() == [0, 1, 2, 3, 5, 7, 8, 10] and int(pick.sum()) == 15379
+    frames = 1 + (bench.N_SAMPLES - 400) // 160
+    assert bench.DUMP_UTTS * frames * bench.N_MELS * 4 <= 64 * 10 ** 6
+    feats = torch.randn(bench.B_UTTS, 7, bench.N_MELS).index_select(0, pick)
+    bench.write_outputs(str(tmp_path / "d"), {"features": feats})
+    got = np.load(str(tmp_path / "d" / "features.npy"))
+    assert got.dtype == np.float32 and got.shape == (128, 7, bench.N_MELS)
+    assert np.array_equal(got, feats.numpy())
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "r")]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + bad, capture_output=True, text=True)
+        assert r.returncode == 2 and "error" in r.stderr, bad
+    assert not (tmp_path / "r").exists()

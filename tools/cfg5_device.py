@@ -42,11 +42,36 @@ def load_reference_model():
     return ConformerMutiLangModel
 
 
-def run(B=128, n_check=16, steps=5):
+def stand_in_model():
+    """A consumer of the reference model's shape (SURVEY.md 3.5) built from torchaudio.models.Conformer, for the consumer
+    check where the reference's model source is not staged: Conv1d subsampling (k=3, s=2, p=1), 14 Conformer blocks,
+    one CTC head per language (vocab + blank) and a language-id head on the time-averaged encoding.  Not the reference
+    model: it checks that the kernel's features drive a Conformer like the oracle's (the reference's arithmetic) do."""
+    import torch
+    from torchaudio.models import Conformer
+
+    class StandInConformerLid(torch.nn.Module):
+        def __init__(self, lang2vocab, lang2index, dim=176, **_):
+            super().__init__()
+            self.sub = torch.nn.Conv1d(80, dim, 3, stride=2, padding=1)
+            self.enc = Conformer(input_dim=dim, num_heads=4, ffn_dim=4 * dim, num_layers=14, depthwise_conv_kernel_size=31)
+            self.ctc = torch.nn.ModuleDict({k: torch.nn.Linear(dim, v + 1) for k, v in lang2vocab.items()})
+            self.lid = torch.nn.Linear(dim, len(lang2index))
+
+        def forward(self, x, sample_rate, lang):
+            h = self.sub(x.transpose(1, 2)).transpose(1, 2)
+            h, _ = self.enc(h, torch.full((h.shape[0],), h.shape[1], device=h.device))
+            return {k: head(h).log_softmax(-1) for k, head in self.ctc.items()}, self.lid(h.mean(1)).softmax(-1)
+
+    return StandInConformerLid
+
+
+def run(B=128, n_check=16, steps=5, model=None):
+    """model: the consumer's class; default the staged reference model (None is returned when it is not staged)."""
     import torch
     import speech_lid_b200 as lid
     from oracle import frontend_oracle as O
-    Model = load_reference_model()
+    Model = model or load_reference_model()
     if Model is None:
         return None
     dev = torch.device("cuda:0")
@@ -111,7 +136,8 @@ def run(B=128, n_check=16, steps=5):
     fe_ms /= steps
     tot_ms /= steps
     audio_s = B * N / 16000.0
-    return dict(workload="cfg5: %d x 8-s utterances -> fused fbank -> reference ConformerMutiLangModel forward (random init, eval, fp32) on one B200" % B,
+    consumer = "reference ConformerMutiLangModel" if model is None else Model.__name__
+    return dict(workload="cfg5: %d x 8-s utterances -> fused fbank -> %s forward (random init, eval, fp32) on one B200" % (B, consumer),
                 features_norm_rel_vs_oracle=feat_err, consumer_worst_abs_diff=worst, consumer_min_argmax_agreement=agree,
                 checked_utterances=n_check, consumer=detail, ms_per_batch=round(tot_ms, 3), frontend_ms=round(fe_ms, 4),
                 frontend_share=round(fe_ms / tot_ms, 5), e2e_audio_s_per_s=round(audio_s / (tot_ms * 1e-3), 1),
