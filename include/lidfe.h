@@ -188,8 +188,10 @@ long long lidfe_plan_frames(lidfe_plan p, int i);
 /* -- the hot path --------------------------------------------------------------------------------- */
 
 /*
- * ONE kernel for every cmvn_mode: with LIDFE_CMVN_PER_UTT / LIDFE_POST_TOPDB the CTA that completes an utterance's
- * statistics normalises (clamps) its rows while they are still in L2 -- there is no second pass over HBM.
+ * One fbank kernel for every cmvn_mode.  With LIDFE_CMVN_PER_UTT / LIDFE_POST_TOPDB it also hands each utterance's
+ * statistics (sums / extrema) over to global memory, and a second kernel, cmvn_apply_kernel, normalises (clamps) the
+ * rows in place: it reads them back, mostly out of L2, where the fbank kernel has just written them.
+ * lidfe_set_precision changes which kernels this call launches: it mutates the handle and must not race with launches.
  * Replaces, for a whole batch in one call:
  *   wav2mel(x, use_kaildi=True)            ref: lid/audio_processor.py:8-69   (n_ceps == 0)
  *   torchaudio.compliance.kaldi.mfcc       ta: compliance/kaldi.py:669-813    (n_ceps > 0; not in the reference)

@@ -9,7 +9,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# LIDFE_LIB_PATH: development only (kernel variants built next to the product library by tools/build_variants.py)
+# LIDFE_LIB_PATH: development only (load a library built elsewhere, e.g. from another commit, to compare the two)
 LIB_PATH = os.environ.get("LIDFE_LIB_PATH") or os.path.join(_HERE, "liblidfe.so")
 
 # include/lidfe.h

@@ -3,7 +3,6 @@
 // CPU compute path.
 #include <cuda_runtime.h>
 #include <math.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -29,16 +28,16 @@ using namespace lidfe;
 // batches (a new length signature every step, ref: lid/raw_datasets.py:345-365) allocate nothing in steady state.
 //
 // Layout (sized by CAPACITY, so the at-rest state survives re-use with another batch size):
-//   workspace  sched[2] + ictl[2] int | utt_done[2][Bc] int | utt_max[2][Bc] u32 (0) | utt_min[2][Bc] u32 (~0) |
-//              utt_stats[2][Bc][2][n_out] f64 (0) | utt_wnorm[Bc] float2       ([2] = launch parity, see FbankParams::items)
+//   workspace  sched[2] int | utt_max[2][Bc] u32 (0) | utt_min[2][Bc] u32 (~0) | utt_stats[2][Bc][2][n_out] f64 (0) |
+//              utt_wnorm[Bc] float2                                ([2] = launch parity, see FbankParams::utt_stats)
 //   tables     frames[Bc] i64 | out_rows[Bc] i64 | offsets[Bc] i64 | lengths[Bc] i64 | first_tile[Bc] i64 |
-//              items[Ic] int4 | spans[Sc] | tiles[Tc] (MFCC two-kernel path only)
+//              spans[Sc] | w_first[W + 1] int | warp spans[Wc] | tiles[Tc] (MFCC two-kernel path only)
 struct PlanBlock {
   unsigned char* d_base;
   unsigned char* h_tables;      // pinned mirror of the tables section
   size_t ws_bytes, tab_bytes;
   int Bc;
-  long long Sc, Tc, Ic, Wc;     // capacities: spans, tiles, items, warp spans
+  long long Sc, Tc, Wc;         // capacities: spans, tiles, warp spans
   cudaEvent_t ev;               // last use on the device (kernels or the upload)
   float* d_logmel;              // tile-blocked log-mel workspace of the two-kernel MFCC path (grown on demand)
   long long logmel_tiles;
@@ -65,17 +64,7 @@ struct lidfe_ctx {
   int warp_ok;        // configuration inside its scope (KALDI framing, no in-kernel dither, std_mel 0/1)
   int w_grid;         // resident CTAs of that kernel
   int w_tab_bytes;    // shared-memory bytes in front of the per-warp areas
-  int w_static_pct;       // share of the quads dealt out as static per-warp runs (LIDFE_WSTATIC, default 90)
-  int w_pool_quads;       // quads per span of the dynamically claimed pool (LIDFE_WPOOL, default 1)
-  int w_fused;            // per-utterance CMVN: second stage inside the warp kernel (LIDFE_WFUSED, default 1) instead of a second launch
-  int w_groups;           // fused second stage: the static runs are dealt out in this many utterance groups (LIDFE_WGROUPS)
   size_t w_smem;      // dynamic shared memory per CTA
-  int apply_rows; // rows per CTA of cmvn_apply_kernel (LIDFE_APPLY_ROWS, read once)
-  int span_tiles; // LIDFE_SPAN_TILES override (0 = automatic)
-  int fused_apply;  // LIDFE_FUSED_APPLY=1: per-utterance second stage inside the fbank kernel (service CTAs) instead of a second kernel
-  int service_ctas; // LIDFE_SERVICE_CTAS override (0 = automatic)
-  int dbg;         // LIDFE_DBG development switches (see FbankParams::dbg)
-  int apply_block; // rows per claimed block of the in-kernel second stage (LIDFE_APPLY_BLOCK, default 128)
   std::vector<PlanBlock*>* pool;      // free blocks
   std::mutex* pool_mu;
   long long blocks_allocated;         // device/pinned block allocations made for plans so far (lidfe_pool_stats)
@@ -86,7 +75,7 @@ struct lidfe_ctx {
   int prof_used;
   int prof_stride;   // bracket every prof_stride-th featurize call (event records between kernels cost a few us)
   int prof_calls;
-  int dct_mma;     // two-kernel MFCC path: DCT on the tensor cores (lidfe_mfcc_mma.cuh) when the shapes fit; LIDFE_DCT_MMA=0 disables
+  int dct_mma;     // two-kernel MFCC path: DCT on the tensor cores (lidfe_mfcc_mma.cuh) when the shapes fit (n_mels % 8 == 0)
   // precise mode (lidfe_set_precision, lidfe_fbank_precise.cuh): fp64 arithmetic on the reference's fp32 tables
   int precise;
   int k0_off, melw_off, total_taps;   // the segment-form mel plan inside the blob (the precise kernel reads it from there)
@@ -102,21 +91,16 @@ struct lidfe_plan_s {
   PlanBlock* blk;
   // views into blk->d_base
   int* d_sched;
-  int* d_utt_done;
   unsigned* d_utt_max;
   unsigned* d_utt_min;
   double* d_utt_stats;
   float2* d_utt_wnorm;
-  int4* d_items;
-  int n_items;
   int parity;             // per-utterance launches on this plan so far, mod 2 (host-side toggle)
   long long* d_frames;    // [B]
   long long* d_out_rows;  // [B]
   long long* d_offsets;   // [B]
   long long* d_lengths;   // [B]
   long long* d_utt_first_tile;   // [B]
-  int* d_first_item;             // [B + 1] first second-stage item of every utterance
-  int* d_wq;                     // ready queue of the warp kernel's fused second stage ([4 + Ic] int, at rest = 0)
   Span* d_spans;
   Span* d_wspans;         // warp spans (NULL when the handle cannot use the warp kernel)
   long long n_wspans;
@@ -129,8 +113,6 @@ struct lidfe_plan_s {
 };
 
 static std::atomic<long long> g_launches{0};
-static long long* g_dbg_buf = nullptr;
-extern "C" int lidfe_dbg_read(long long* host, int n) { return g_dbg_buf ? (int)cudaMemcpy(host, g_dbg_buf, sizeof(long long) * n, cudaMemcpyDeviceToHost) : -1; }
 
 #define CU_TRY(expr)                      \
   do {                                    \
@@ -484,10 +466,8 @@ int lidfe_h2d_gather(void* dst_dev, const void* const* src_host, const long long
   }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   unsigned char* const dst = static_cast<unsigned char*>(dst_dev);
-  // kernel path: every source 16-byte aligned and device-accessible, every destination 16-byte aligned;
-  // LIDFE_H2D_KERNEL=0 keeps the copy engine
-  static const int use_kernel = [] { const char* env = getenv("LIDFE_H2D_KERNEL"); return env ? atoi(env) : 1; }();
-  bool kernel_ok = use_kernel && B >= 4 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
+  // kernel path: every source 16-byte aligned and device-accessible, every destination 16-byte aligned
+  bool kernel_ok = B >= 4 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
   for (int i = 0; i < B && kernel_ok; ++i)
     kernel_ok = (reinterpret_cast<uintptr_t>(src_host[i]) & 15) == 0 && ((offsets[i] * elem_bytes) & 15) == 0;
   for (int k = 0; k < B && kernel_ok; ++k) {       // (~0.5 us per query: a source the device cannot read would be a fault, not an error code)
@@ -729,23 +709,6 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
     lidfe_destroy(c);
     return LIDFE_E_NOMEM;
   }
-  c->apply_rows = kApplyRowsDefault;
-  if (const char* env = getenv("LIDFE_APPLY_ROWS")) {      // tuning knobs are read once, here
-    const int v = atoi(env);
-    if (v >= 8 && v <= 65536) c->apply_rows = v;
-  }
-  if (const char* env = getenv("LIDFE_DBG")) c->dbg = atoi(env);
-  c->apply_block = 128;
-  if (const char* env = getenv("LIDFE_SERVICE_CTAS")) c->service_ctas = atoi(env);
-  if (const char* env = getenv("LIDFE_FUSED_APPLY")) c->fused_apply = atoi(env) != 0;
-  if (const char* env = getenv("LIDFE_APPLY_BLOCK")) {
-    const int v = atoi(env);
-    if (v >= 16 && v <= 4096) c->apply_block = v;
-  }
-  if (const char* env = getenv("LIDFE_SPAN_TILES")) {
-    const int v = atoi(env);
-    if (v >= 1 && v <= kMaxSpanTiles) c->span_tiles = v;
-  }
   cudaError_t e = cudaGetDevice(&c->device);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&c->num_sms, cudaDevAttrMultiProcessorCount, c->device);
   if (e == cudaSuccess) e = upload(&c->d_blob, blob.data(), blob.size());
@@ -765,7 +728,6 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
       if (e == cudaSuccess)
         e = cudaFuncSetAttribute(mfcc_dct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->smem_bytes_dct));
       c->dct_mma = (cfg->n_mels % 8 == 0) ? 1 : 0;
-      if (const char* env = getenv("LIDFE_DCT_MMA")) c->dct_mma = c->dct_mma && atoi(env) != 0;
       if (e == cudaSuccess && c->dct_mma)
         e = cudaFuncSetAttribute(mfcc_dct_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMmSmemBytes);
     }
@@ -786,15 +748,8 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
   // of 4 samples so that interior quads stay 16-byte aligned)
   c->warp_ok = ((cfg->framing == LIDFE_FRAMING_KALDI && cfg->dither == 0.f && c->std_mel != 2) ||
                 (cfg->framing == LIDFE_FRAMING_CENTER && cfg->dither == 0.f && c->std_mel == 2 && cfg->pad % 4 == 0 && cfg->n_ceps == 0)) ? 1 : 0;
+  // test selector: LIDFE_WARP_KERNEL=0 keeps fbank_kernel, the reference the warp kernel is tested against
   if (const char* env = getenv("LIDFE_WARP_KERNEL")) c->warp_ok = c->warp_ok && atoi(env) != 0;
-  c->w_static_pct = 90;
-  c->w_pool_quads = 1;
-  if (const char* env = getenv("LIDFE_WSTATIC")) { const int v = atoi(env); if (v >= 0 && v <= 100) c->w_static_pct = v; }
-  if (const char* env = getenv("LIDFE_WPOOL")) { const int v = atoi(env); if (v >= 1 && v <= 64) c->w_pool_quads = v; }
-  c->w_fused = 0;
-  c->w_groups = 1;
-  if (const char* env = getenv("LIDFE_WFUSED")) c->w_fused = atoi(env) != 0;
-  if (const char* env = getenv("LIDFE_WGROUPS")) { const int v = atoi(env); if (v >= 1 && v <= 64) c->w_groups = v; }
   if (e == cudaSuccess && c->warp_ok) {
     c->w_tab_bytes = static_cast<int>((kWTabOff + c->blob_bytes_fbank + kMaxMels * 8 + 127) / 128 * 128);
     const size_t per_warp = (cfg->in_dtype == LIDFE_IN_I16) ? WarpLayout<short>::kWarpBytes : WarpLayout<float>::kWarpBytes;
@@ -859,19 +814,17 @@ int lidfe_destroy(lidfe_handle h) {
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 struct BlockLayout {
-  size_t sched, utt_done, utt_max, utt_min, utt_stats, utt_wnorm, wq, ws_bytes;
-  size_t frames, out_rows, offsets, lengths, first_tile, first_item, items, spans, wfirst, wspans, tiles, tab_bytes;   // tables: relative to ws_bytes
+  size_t sched, utt_max, utt_min, utt_stats, utt_wnorm, ws_bytes;
+  size_t frames, out_rows, offsets, lengths, first_tile, spans, wfirst, wspans, tiles, tab_bytes;   // tables: relative to ws_bytes
 };
-static BlockLayout block_layout(int Bc, long long Sc, long long Tc, long long Ic, long long Wc, int n_out, long long n_warps) {
+static BlockLayout block_layout(int Bc, long long Sc, long long Tc, long long Wc, int n_out, long long n_warps) {
   BlockLayout L;
   size_t o = 0;
   L.sched = o; o += 16;
-  L.utt_done = o; o = align_up(o + 2 * static_cast<size_t>(Bc) * 4, 16);          // [2 launch parities][Bc]
-  L.utt_max = o; o = align_up(o + 2 * static_cast<size_t>(Bc) * 4, 16);
+  L.utt_max = o; o = align_up(o + 2 * static_cast<size_t>(Bc) * 4, 16);          // [2 launch parities][Bc]
   L.utt_min = o; o = align_up(o + 2 * static_cast<size_t>(Bc) * 4, 16);
   L.utt_stats = o; o = align_up(o + 2 * static_cast<size_t>(Bc) * 2 * n_out * 8, 16);
   L.utt_wnorm = o; o = align_up(o + static_cast<size_t>(Bc) * 8, 256);
-  L.wq = o; o = align_up(o + (static_cast<size_t>(Ic) + 4) * 4, 256);
   L.ws_bytes = o;
   o = 0;
   L.frames = o; o += static_cast<size_t>(Bc) * 8;
@@ -879,8 +832,6 @@ static BlockLayout block_layout(int Bc, long long Sc, long long Tc, long long Ic
   L.offsets = o; o += static_cast<size_t>(Bc) * 8;
   L.lengths = o; o += static_cast<size_t>(Bc) * 8;
   L.first_tile = o; o = align_up(o + static_cast<size_t>(Bc) * 8, 32);
-  L.first_item = o; o = align_up(o + (static_cast<size_t>(Bc) + 1) * 4, 32);
-  L.items = o; o = align_up(o + static_cast<size_t>(Ic) * 16, 32);
   L.spans = o; o += static_cast<size_t>(Sc) * sizeof(Span);
   L.wfirst = o; o = align_up(o + (Wc > 0 ? static_cast<size_t>(n_warps) + 1 : 0) * 4, 32);
   L.wspans = o; o += static_cast<size_t>(Wc) * sizeof(Span);
@@ -896,7 +847,7 @@ static long long pow2_at_least(long long v, long long lo) {
 
 // a block with room for (B, spans, tiles): from the pool if one fits, else a new allocation (the only place that
 // allocates; the workspace is put to rest once, here -- the kernels leave it at rest)
-static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_tiles, long long n_items, long long n_wspans, PlanBlock** out) {
+static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_tiles, long long n_wspans, PlanBlock** out) {
   *out = nullptr;
   {
     // first choice: a block that fits and whose previous work has finished (no waiting); second: while the handle owns
@@ -907,7 +858,7 @@ static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_til
     int busy = -1;
     for (size_t i = 0; i < h->pool->size(); ++i) {
       PlanBlock* b = (*h->pool)[i];
-      if (b->Bc >= B && b->Sc >= n_spans && b->Tc >= n_tiles && b->Ic >= n_items && b->Wc >= n_wspans) {
+      if (b->Bc >= B && b->Sc >= n_spans && b->Tc >= n_tiles && b->Wc >= n_wspans) {
         if (cudaEventQuery(b->ev) == cudaSuccess) {
           h->pool->erase(h->pool->begin() + i);
           *out = b;
@@ -932,9 +883,8 @@ static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_til
   b->Bc = static_cast<int>(pow2_at_least(B, 64));
   b->Sc = pow2_at_least(n_spans, 256);
   b->Tc = n_tiles > 0 ? pow2_at_least(n_tiles, 256) : 0;
-  b->Ic = pow2_at_least(n_items, 256);
   b->Wc = n_wspans > 0 ? pow2_at_least(n_wspans, 256) : 0;
-  const BlockLayout L = block_layout(b->Bc, b->Sc, b->Tc, b->Ic, b->Wc, h->n_out, static_cast<long long>(h->w_grid) * kWWarps);
+  const BlockLayout L = block_layout(b->Bc, b->Sc, b->Tc, b->Wc, h->n_out, static_cast<long long>(h->w_grid) * kWWarps);
   b->ws_bytes = L.ws_bytes;
   b->tab_bytes = L.tab_bytes;
   cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&b->d_base), L.ws_bytes + L.tab_bytes);
@@ -987,13 +937,10 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   //      dynamic claiming balances (>= ~10), as long as possible otherwise (a span end costs two CTA barriers, and in
   //      the per-utterance modes a hand-over of 2 x n_out sums); the spans of the last stretch of the batch are single
   //      tiles so that the CTAs run dry together.
-  int span_tiles = h->span_tiles;
-  if (span_tiles <= 0) {
-    const long long per_cta_tiles = n_tiles / (h->grid_cap > 0 ? h->grid_cap : 1);
-    span_tiles = static_cast<int>(per_cta_tiles / 10);
-    if (span_tiles < 1) span_tiles = 1;
-    if (span_tiles > kMaxSpanTiles) span_tiles = kMaxSpanTiles;
-  }
+  const long long per_cta_tiles = n_tiles / (h->grid_cap > 0 ? h->grid_cap : 1);
+  int span_tiles = static_cast<int>(per_cta_tiles / 10);
+  if (span_tiles < 1) span_tiles = 1;
+  if (span_tiles > kMaxSpanTiles) span_tiles = kMaxSpanTiles;
   const long long tail_tiles = static_cast<long long>(h->grid_cap) * span_tiles;   // ~ one round of spans
   std::vector<Span> spans;
   std::vector<Tile> tiles;
@@ -1063,25 +1010,9 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
     const long long end = out_rows_host[i] + ((pad_rows_host && pad_rows_host[i] > frames[i]) ? pad_rows_host[i] : frames[i]);
     if (end > p->max_row) p->max_row = end;
   }
-  // items of the in-kernel second stage: <= apply_block rows of one utterance each, utterance-major
-  std::vector<int4> items;
-  std::vector<int> first_item(static_cast<size_t>(B) + 1, 0);
-  for (int i = 0; i < B; ++i) {
-    const long long T = frames[i];
-    first_item[static_cast<size_t>(i)] = static_cast<int>(items.size());
-    for (long long r = 0; r < T; r += h->apply_block)
-      items.push_back(make_int4(i, static_cast<int>(r), static_cast<int>(T - r < h->apply_block ? T - r : h->apply_block),
-                                static_cast<int>(T)));
-  }
-  if (items.size() > 0x7fffffffull) {
-    delete p;
-    return LIDFE_E_ARG;
-  }
-  p->n_items = static_cast<int>(items.size());
-  first_item[static_cast<size_t>(B)] = p->n_items;
   // ---- warp spans (lidfe_fbank_warp.cuh).  The quads (4 frames) of the batch, utterance-major, are dealt out as
-  //      W contiguous STATIC runs of s = floor(f Q / W) quads, one per warp (cut into spans where the utterance changes),
-  //      followed by a POOL of short spans (zero-fill runs first, then the last Q - W s quads) that the warps claim one at
+  //      W contiguous STATIC runs of s = floor(0.9 Q / W) quads, one per warp (cut into spans where the utterance changes),
+  //      followed by a POOL of one-quad spans (zero-fill runs first, then the last Q - W s quads) that the warps claim one at
   //      a time when their own run is done.  w_first[w] .. w_first[w + 1] are warp w's static spans.
   std::vector<Span> wspans;
   std::vector<int> w_first;
@@ -1091,7 +1022,7 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
     long long n_quads = 0;
     for (int i = 0; i < B; ++i) n_quads += (frames[i] + kQuadFrames - 1) / kQuadFrames;
     const long long W = static_cast<long long>(h->w_grid) * kWWarps;
-    const long long s_run = (n_quads * h->w_static_pct) / (100 * W);          // static quads per warp
+    const long long s_run = (n_quads * 90) / (100 * W);                     // static quads per warp
     const long long static_quads = s_run * W;
     std::vector<Span> pool;
     // CENTER framing: frame f covers p[160 f - 200, 160 f + 200) of the constant-padded signal (see the span builder above);
@@ -1143,64 +1074,27 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
         }
       }
     }
-    // Utterance GROUPS (w_groups > 1, for the fused per-utterance second stage): the batch is cut into G runs of whole
-    // utterances with about Q / G quads each, and every warp's static run is the concatenation of its share of group 0,
-    // its share of group 1, ...: all warps work on group g at about the same time, so the utterances of group g are
-    // complete -- and their second stage can start -- while groups g + 1 ... are still being computed.  Groups before
-    // the last are dealt out completely (shares differ by at most one quad, the longer ones rotate over the warps);
-    // the last group keeps the static / pool split that balances the tail.  G = 1 is the plain schedule.
-    long long G = h->w_groups;
-    while (G > 1 && n_quads / G < 4 * W) --G;
-    std::vector<int> group_of(static_cast<size_t>(B), 0);
-    std::vector<long long> group_quads(static_cast<size_t>(G), 0);
-    {
-      long long before = 0;
-      for (int i = 0; i < B; ++i) {
-        long long g = n_quads > 0 ? (before * G) / n_quads : 0;
-        if (g > G - 1) g = G - 1;
-        group_of[static_cast<size_t>(i)] = static_cast<int>(g);
-        const long long q = (frames[i] + kQuadFrames - 1) / kQuadFrames;
-        group_quads[static_cast<size_t>(g)] += q;
-        before += q;
-      }
-    }
     std::vector<std::vector<Span>> per_warp(static_cast<size_t>(W));
-    long long rot = 0;          // warp that takes the first run of the group
-    int i_next = 0;             // first utterance of the group
-    for (long long g = 0; g < G; ++g) {
-      const long long Qg = group_quads[static_cast<size_t>(g)];
-      const bool last = (g == G - 1);
-      const long long base = last ? (Qg * h->w_static_pct) / (100 * W) : Qg / W;
-      const long long extra = last ? 0 : Qg % W;           // the first `extra` runs are one quad longer
-      const long long static_q = last ? base * W : Qg;
-      long long quad_no = 0;      // quads of this group dealt out so far
-      long long k = 0;            // run being filled
-      long long run_end = base + (0 < extra ? 1 : 0);      // quad_no at which run k ends
-      for (int i = i_next; i < B && group_of[static_cast<size_t>(i)] == g; ++i, i_next = i) {
-        const long long T = frames[i];
-        for (long long f = 0; f < T;) {
-          const long long left_q = (T - f + kQuadFrames - 1) / kQuadFrames;      // quads left in this utterance
-          if (quad_no < static_q) {
-            while (quad_no >= run_end) {
-              ++k;
-              run_end += base + (k < extra ? 1 : 0);
-            }
-            long long q = run_end - quad_no;                                      // quads left in this run
-            if (q > left_q) q = left_q;
-            const long long nf = (T - f) < q * kQuadFrames ? (T - f) : q * kQuadFrames;
-            push_frames(per_warp[static_cast<size_t>((k + rot) % W)], i, f, nf);
-            quad_no += q;
-            f += nf;
-          } else {
-            long long q = h->w_pool_quads < left_q ? h->w_pool_quads : left_q;
-            const long long nf = (T - f) < q * kQuadFrames ? (T - f) : q * kQuadFrames;
-            push_frames(pool, i, f, nf);
-            quad_no += q;
-            f += nf;
-          }
+    long long quad_no = 0;      // quads dealt out so far
+    for (int i = 0; i < B; ++i) {
+      const long long T = frames[i];
+      for (long long f = 0; f < T;) {
+        const long long left_q = (T - f + kQuadFrames - 1) / kQuadFrames;        // quads left in this utterance
+        if (quad_no < static_quads) {
+          const long long k = quad_no / s_run;                                  // run being filled
+          long long q = (k + 1) * s_run - quad_no;                              // quads left in this run
+          if (q > left_q) q = left_q;
+          const long long nf = (T - f) < q * kQuadFrames ? (T - f) : q * kQuadFrames;
+          push_frames(per_warp[static_cast<size_t>(k)], i, f, nf);
+          quad_no += q;
+          f += nf;
+        } else {
+          const long long nf = (T - f) < kQuadFrames ? (T - f) : kQuadFrames;
+          push_frames(pool, i, f, nf);
+          quad_no += 1;
+          f += nf;
         }
       }
-      rot = (rot + extra) % W;
     }
     w_first.assign(static_cast<size_t>(W) + 1, 0);
     for (long long w = 0; w < W; ++w) {
@@ -1218,8 +1112,7 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   p->n_wspans = static_cast<long long>(wspans.size());
   p->all_aligned = all_aligned;
   PlanBlock* b = nullptr;
-  const int rc = acquire_block(h, B, p->n_spans, static_cast<long long>(tiles.size()), static_cast<long long>(items.size()),
-                               p->n_wspans, &b);
+  const int rc = acquire_block(h, B, p->n_spans, static_cast<long long>(tiles.size()), p->n_wspans, &b);
   if (rc != LIDFE_OK) {
     delete p;
     return rc;
@@ -1229,23 +1122,19 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
     std::lock_guard<std::mutex> g(*h->pool_mu);
     ++h->live_plans;
   }
-  const BlockLayout L = block_layout(b->Bc, b->Sc, b->Tc, b->Ic, b->Wc, h->n_out, static_cast<long long>(h->w_grid) * kWWarps);
+  const BlockLayout L = block_layout(b->Bc, b->Sc, b->Tc, b->Wc, h->n_out, static_cast<long long>(h->w_grid) * kWWarps);
   unsigned char* ws = b->d_base;
   unsigned char* tab = b->d_base + L.ws_bytes;
   p->d_sched = reinterpret_cast<int*>(ws + L.sched);
-  p->d_utt_done = reinterpret_cast<int*>(ws + L.utt_done);
   p->d_utt_max = reinterpret_cast<unsigned*>(ws + L.utt_max);
   p->d_utt_min = reinterpret_cast<unsigned*>(ws + L.utt_min);
   p->d_utt_stats = reinterpret_cast<double*>(ws + L.utt_stats);
   p->d_utt_wnorm = reinterpret_cast<float2*>(ws + L.utt_wnorm);
-  p->d_items = reinterpret_cast<int4*>(tab + L.items);
   p->d_frames = reinterpret_cast<long long*>(tab + L.frames);
   p->d_out_rows = reinterpret_cast<long long*>(tab + L.out_rows);
   p->d_offsets = reinterpret_cast<long long*>(tab + L.offsets);
   p->d_lengths = reinterpret_cast<long long*>(tab + L.lengths);
   p->d_utt_first_tile = reinterpret_cast<long long*>(tab + L.first_tile);
-  p->d_first_item = reinterpret_cast<int*>(tab + L.first_item);
-  p->d_wq = reinterpret_cast<int*>(ws + L.wq);
   p->d_spans = reinterpret_cast<Span*>(tab + L.spans);
   p->d_wspans = wspans.empty() ? nullptr : reinterpret_cast<Span*>(tab + L.wspans);
   p->d_w_first = wspans.empty() ? nullptr : reinterpret_cast<int*>(tab + L.wfirst);
@@ -1257,8 +1146,6 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   memcpy(ht + L.offsets, wav_offsets_host, static_cast<size_t>(B) * 8);
   memcpy(ht + L.lengths, wav_lengths_host, static_cast<size_t>(B) * 8);
   memcpy(ht + L.first_tile, utt_first_tile.data(), static_cast<size_t>(B) * 8);
-  memcpy(ht + L.first_item, first_item.data(), (static_cast<size_t>(B) + 1) * 4);
-  memcpy(ht + L.items, items.data(), items.size() * sizeof(int4));
   memcpy(ht + L.spans, spans.data(), spans.size() * sizeof(Span));
   if (!wspans.empty()) {
     memcpy(ht + L.wspans, wspans.data(), wspans.size() * sizeof(Span));
@@ -1342,11 +1229,10 @@ static int launch_apply(lidfe_ctx* h, lidfe_plan p, float* feats, long long ld, 
     A.utt_max = p->d_utt_max + parity * Bc;
     A.utt_min = p->d_utt_min + parity * Bc;
     A.rest_stats = p->d_utt_stats + static_cast<long long>(op) * Bc * 2 * h->n_out;
-    A.rest_done = p->d_utt_done + op * Bc;
     A.rest_max = p->d_utt_max + op * Bc;
     A.rest_min = p->d_utt_min + op * Bc;
   }
-  A.rows_per_cta = h->apply_rows;
+  A.rows_per_cta = kApplyRows;
   const long long chunks = (p->max_frames + A.rows_per_cta - 1) / A.rows_per_cta;
   if (chunks > 65535) return LIDFE_E_ARG;
   dim3 grid(static_cast<unsigned>(p->B), static_cast<unsigned>(chunks));
@@ -1406,26 +1292,10 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
   P.spans = p->d_spans;
   P.n_spans = static_cast<int>(p->n_spans);
   P.sched = p->d_sched;
-  P.utt_done = p->d_utt_done;
-  P.ictl = p->d_sched + 2;
-  P.items = p->d_items;
-  P.n_items = p->n_items;
   P.parity = p->parity;
   P.b_cap = p->blk->Bc;
-  P.n_utts = p->B;
   if (cmvn_mode == LIDFE_CMVN_PER_UTT || cmvn_mode == LIDFE_POST_TOPDB) p->parity ^= 1;
-  P.dbg = h->dbg;
-  if (h->dbg & 16) {
-    static long long* g_dbg = nullptr;
-    if (!g_dbg) cudaMalloc(reinterpret_cast<void**>(&g_dbg), 8 * 8 * 4096);
-    P.dbg_buf = g_dbg;
-    g_dbg_buf = g_dbg;
-  }
-  P.utt_frames = p->d_frames;
-  P.utt_out_row = p->d_out_rows;
   P.utt_first_tile = p->d_utt_first_tile;
-  P.utt_first_item = p->d_first_item;
-  P.wq = p->d_wq;
   P.const_blob = h->d_blob;
   P.const_bytes = h->blob_bytes;
   for (int b = 0; b < kBands; ++b) P.band_taps[b] = h->band_taps[b];
@@ -1495,7 +1365,7 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
     Q.mode = cmvn_mode;
     Q.utt_stats = p->d_utt_stats + static_cast<long long>(P.parity & 1) * P.b_cap * 2 * h->n_out;
     Q.stats_out = stats_out_dev;
-    long long gp = p->n_spans * kMaxSpanTiles < static_cast<long long>(h->num_sms) * LIDFE_PRECISE_CTAS ? p->n_spans * kMaxSpanTiles : static_cast<long long>(h->num_sms) * LIDFE_PRECISE_CTAS;
+    long long gp = p->n_spans * kMaxSpanTiles < static_cast<long long>(h->num_sms) * kPCtasPerSm ? p->n_spans * kMaxSpanTiles : static_cast<long long>(h->num_sms) * kPCtasPerSm;
     if (gp < 1) gp = 1;
     {
       void (*pk)(const PreciseParams) =
@@ -1514,7 +1384,7 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
   }
 
   // the warp-autonomous kernel takes every call inside its scope (see lidfe_fbank_warp.cuh)
-  const bool use_warp = h->warp_ok && !raw && p->d_wspans != nullptr && !h->fused_apply &&
+  const bool use_warp = h->warp_ok && !raw && p->d_wspans != nullptr &&
                         (cmvn_mode != LIDFE_POST_TOPDB || h->std_mel == 2);
   auto launch_warp = [&](FbankParams& F, bool profile) -> int {
     F.wspans = p->d_wspans;
@@ -1566,14 +1436,12 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
     F.mode = LIDFE_CMVN_NONE;
     F.ws_blocked = 1;
     F.const_bytes = h->blob_bytes_fbank;
-    F.n_compute = static_cast<int>(p->n_spans < static_cast<long long>(h->num_sms) * 4 ? p->n_spans : static_cast<long long>(h->num_sms) * 4);
-    if (F.n_compute < 1) F.n_compute = 1;
-    F.k_static = static_cast<int>((p->n_spans / F.n_compute) * 85 / 100);
-    if (F.k_static < 1) F.k_static = 1;
     fbank_fn f2 = (h->cfg.in_dtype == LIDFE_IN_I16) ? pick_kernel_t<short>(false, h->std_mel)
                                                      : pick_kernel_t<float>(false, h->std_mel);
     long long g2 = p->n_spans < static_cast<long long>(h->num_sms) * 4 ? p->n_spans : static_cast<long long>(h->num_sms) * 4;
     if (g2 < 1) g2 = 1;
+    F.k_static = static_cast<int>((p->n_spans / g2) * 85 / 100);
+    if (F.k_static < 1) F.k_static = 1;
     if (use_warp) {
       const int rcw = launch_warp(F, true);
       if (rcw != LIDFE_OK) return rcw;
@@ -1622,41 +1490,20 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
   }
 
   if (use_warp && h->cfg.n_ceps == 0) {
-    const int launch_parity_w = P.parity;
-    // per-utterance CMVN: the second stage runs inside the kernel (w_fused), else as a second launch
-    const bool fused_w = LIDFE_WFUSED_BUILD && h->w_fused && cmvn_mode == LIDFE_CMVN_PER_UTT && p->n_items > 0;
-    if (!fused_w) P.n_items = 0;
     const int rcw = launch_warp(P, true);
     if (rcw != LIDFE_OK) return rcw;
     if (cmvn_mode == LIDFE_POST_TOPDB)
-      return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 2, launch_parity_w);
-    if (cmvn_mode == LIDFE_CMVN_PER_UTT && !fused_w)
-      return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 1, launch_parity_w);
+      return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 2, P.parity);
+    if (cmvn_mode == LIDFE_CMVN_PER_UTT)
+      return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 1, P.parity);
     CU_TRY(cudaEventRecord(p->blk->ev, st));
     return LIDFE_OK;
   }
 
-  // per-utterance modes: some of the resident CTAs are SERVICE CTAs (the second stage, see FbankParams::items)
-  P.n_compute = static_cast<int>(grid);
-  const bool per_utt = (cmvn_mode == LIDFE_CMVN_PER_UTT || cmvn_mode == LIDFE_POST_TOPDB);
-  const int launch_parity = P.parity;
-  if (per_utt && !h->fused_apply) P.n_items = 0;       // second stage as its own kernel (default, see DESIGN.md 4.2)
-  if (per_utt && h->fused_apply) {
-    long long service = h->service_ctas > 0 ? h->service_ctas : h->num_sms / 8;
-    if (service > grid / 4) service = grid / 4;
-    if (service < 1) service = 1;
-    long long compute = p->n_spans < h->grid_cap - service ? p->n_spans : h->grid_cap - service;
-    if (compute < 1) compute = 1;
-    P.n_compute = static_cast<int>(compute);
-    grid = compute + service;
-  }
-  // static head of the schedule: ~85 % of the spans are dealt out as consecutive runs (fused second stage: none, the
-  // utterances have to complete progressively)
+  // static head of the schedule: ~85 % of the spans are dealt out as consecutive runs
   {
-    const long long per = p->n_spans / (P.n_compute > 0 ? P.n_compute : 1);
-    long long ks = (per * 85) / 100;
-    if (ks < 1 || (per_utt && h->fused_apply)) ks = 1;
-    P.k_static = static_cast<int>(ks);
+    const long long ks = ((p->n_spans / grid) * 85) / 100;
+    P.k_static = static_cast<int>(ks < 1 ? 1 : ks);
   }
   fbank_fn fn = pick_kernel(h);
   bool prof = h->prof_events && (h->prof_used + 2 <= static_cast<int>(h->prof_events->size()));
@@ -1669,8 +1516,8 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
     CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used + 1], st));
     h->prof_used += 2;
   }
-  if (per_utt && !h->fused_apply)
-    return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, cmvn_mode == LIDFE_CMVN_PER_UTT ? 1 : 2, launch_parity);
+  if (cmvn_mode == LIDFE_CMVN_PER_UTT || cmvn_mode == LIDFE_POST_TOPDB)
+    return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, cmvn_mode == LIDFE_CMVN_PER_UTT ? 1 : 2, P.parity);
   CU_TRY(cudaEventRecord(p->blk->ev, st));
   return LIDFE_OK;
 }
@@ -1836,7 +1683,7 @@ struct lidfe_resampler_s {
   int K8, KS, use_mma;             // tensor-core path (nw % 16 == 0): taps padded to 8, shared-memory row stride
   float* d_w;                      // [nw][K8] row-major bank (tensor-core kernel)
   // tcgen05 path (lidfe_resample_tc.cuh): the bank as shared-memory images, one per (phase tile, 32-tap block, hi | lo)
-  int use_tc, tc_N, tc_tiles, tc_KB, tc_stages, tc_cols, tc_dbg;
+  int use_tc, tc_N, tc_tiles, tc_KB, tc_stages, tc_cols;
   size_t tc_smem;
   unsigned char* d_wimg;
 };
@@ -1888,6 +1735,7 @@ static int create_bank(lidfe_resampler* out, int orig, int nw, const float* kern
   r->K8 = (taps + 7) & ~7;
   r->KS = r->K8 + 4;
   r->d_w = nullptr;
+  // test selectors: LIDFE_RESAMPLE_MMA=0 / LIDFE_RESAMPLE_TC=0 keep the kernels the faster ones are tested against
   const char* ev = getenv("LIDFE_RESAMPLE_MMA");
   r->use_mma = (nw % 16 == 0) && !(ev && ev[0] == '0') &&
                static_cast<size_t>(kRmFrames) * r->KS * sizeof(float) <= 200 * 1024;
@@ -1902,7 +1750,6 @@ static int create_bank(lidfe_resampler* out, int orig, int nw, const float* kern
   }
   // tcgen05 path: phases in tiles of N (a multiple of 32 that divides nw, <= 256: 160 for both of the reference's rates)
   r->use_tc = 0;
-  r->tc_dbg = getenv("LIDFE_TC_DBG") != nullptr;      // development: per-role cycle counters of CTA 0 on stderr (synchronises)
   r->d_wimg = nullptr;
   {
     int N = 0;
@@ -1993,12 +1840,6 @@ int lidfe_resample(lidfe_resampler r, int B, const float* in_dev, const long lon
     const long long gxt = (fr + kTcM - 1) / kTcM;
     if (gxt > 0x7fffffffLL || B > 65535 || r->tc_tiles > 65535) return LIDFE_E_ARG;
     T.gx = static_cast<int>(gxt); T.B = B; T.n_tiles = r->tc_tiles;
-    T.dbg = nullptr;
-    static long long* g_tc_dbg = nullptr;
-    if (r->tc_dbg) {
-      if (!g_tc_dbg) { cudaMalloc(reinterpret_cast<void**>(&g_tc_dbg), 16 * 8); cudaMemset(g_tc_dbg, 0, 16 * 8); }
-      T.dbg = g_tc_dbg;
-    }
     const long long n_lin = gxt * B * r->tc_tiles;
     int dev = 0, sms = 0;
     CU_TRY(cudaGetDevice(&dev));
@@ -2007,13 +1848,6 @@ int lidfe_resample(lidfe_resampler r, int B, const float* in_dev, const long lon
     resample_tc_kernel<<<static_cast<unsigned>(grid), kTcThreads, r->tc_smem, static_cast<cudaStream_t>(stream)>>>(T);
     g_launches.fetch_add(1);
     CU_TRY(cudaGetLastError());
-    if (T.dbg) {
-      long long h[16];
-      cudaDeviceSynchronize();
-      cudaMemcpy(h, T.dbg, sizeof(h), cudaMemcpyDeviceToHost);
-      fprintf(stderr, "[tc dbg] CTA0: mma lane total %lld cyc, wait A %lld, wait B %lld, wait acc_empty %lld, issue %lld, tiles %lld | builder w4: wait empty %lld, publish %lld | w8: wait empty %lld, publish %lld | w4 load-wait %lld, stores %lld\n",
-              h[0], h[1], h[2], h[3], h[4], h[5], h[8], h[9], h[10], h[11], h[12], h[13]);
-    }
     return LIDFE_OK;
   }
   if (r->use_mma) {

@@ -50,10 +50,8 @@ struct PreciseParams {
   double* stats_out;        // [2 * n_out + 1]
 };
 
-#ifndef LIDFE_PRECISE_CTAS
-#define LIDFE_PRECISE_CTAS 4
-#endif
 constexpr int kPThreads = 128;
+constexpr int kPCtasPerSm = 4;
 constexpr int kPHalfWarps = kPThreads / 16;
 constexpr int kPRow = 17;                               // double2 elements per transposition row (conflict-free both ways)
 constexpr int kPPlane = 16 * kPRow;                     // double2 elements per half-warp plane (4352 bytes)
@@ -114,7 +112,7 @@ constexpr int kPOffPlane = kPOffMelR + kMaxMels * 4 + 64;
 constexpr int kPSmemBytes = kPOffPlane + kPHalfWarps * kPPlane * 16;
 
 template <typename TIn, bool kCenter>
-__global__ void __launch_bounds__(kPThreads, LIDFE_PRECISE_CTAS) fbank_precise_kernel(const PreciseParams P) {
+__global__ void __launch_bounds__(kPThreads, kPCtasPerSm) fbank_precise_kernel(const PreciseParams P) {
   extern __shared__ __align__(16) unsigned char psmem[];
   double2* const sm_tw1 = reinterpret_cast<double2*>(psmem);                       // [K1][t]: W256^(K1 t) = (cos, -sin)(2 pi K1 t / 256)
   double2* const sm_tw2 = reinterpret_cast<double2*>(psmem + kPOffTw2);            // W512^k = (cos, -sin)(2 pi k / 512), k = 0..127

@@ -34,31 +34,10 @@ namespace lidfe {
 
 constexpr int kQuadFrames = 4;
 constexpr int kQuadSamples = kFrameShift * kQuadFrames + (kFrameLen - kFrameShift);   // 880
-#ifndef LIDFE_WWARPS
-#define LIDFE_WWARPS 16
-#endif
-#ifndef LIDFE_WCTAS
-#define LIDFE_WCTAS 1
-#endif
-constexpr int kWWarps = LIDFE_WWARPS;            // warps per CTA (they only share the constant tables)
-constexpr int kWCtasPerSm = LIDFE_WCTAS;
+constexpr int kWWarps = 16;                      // warps per CTA (they only share the constant tables)
+constexpr int kWCtasPerSm = 1;
 constexpr int kWThreads = kWWarps * 32;
-#ifndef LIDFE_FOLD_QUADS
-#define LIDFE_FOLD_QUADS 32
-#endif
-constexpr int kFoldQuads = LIDFE_FOLD_QUADS;     // fp32 partial sums are folded into the fp64 accumulators this often
-#ifndef LIDFE_XPOSE_ST128
-#define LIDFE_XPOSE_ST128 1      // transposition stores: 1 = one STS.128 per point, 0 = two STS.64 halves
-#endif
-#ifndef LIDFE_PRE_SHARE
-#define LIDFE_PRE_SHARE 0        // unit pre-emphasis: 1 = frames A and B share the 18 "previous sample" shuffles in EVERY variant (the statistics variant always does)
-#endif
-#ifndef LIDFE_TW2_REGS
-#define LIDFE_TW2_REGS 1           // 1: instantiations without CMVN sums keep the 8 split twiddles of a lane in registers
-#endif
-#ifndef LIDFE_WFUSED_BUILD
-#define LIDFE_WFUSED_BUILD 0      // 1: build the in-kernel per-utterance second stage (then LIDFE_WFUSED=1 selects it)
-#endif
+constexpr int kFoldQuads = 32;                   // fp32 partial sums are folded into the fp64 accumulators this often
 constexpr int kWTabOff = 128;                    // tables start here (the tables' mbarrier sits in front)
 
 // per half-warp transposition plane: 16 rows of 17 elements of 16 bytes (re_A, re_B, im_A, im_B); reused for the 257
@@ -80,87 +59,6 @@ struct WSpanRegs {     // the fields of a span a warp needs per quad, read from 
   long long wav_off, out_row;
   int nframes, utt, t0, aux;
 };
-
-// ---- fused per-utterance second stage (mode 1, P.n_items > 0), out of line: none of its state lives in the quad loop ----
-// Every hand-over announces its frames on the utterance's counter; the warp whose hand-over makes the count complete
-// publishes the utterance's items (<= apply_block rows each) in the ready queue.  A warp that has run out of spans takes
-// items by ticket (one atomicAdd each) until all have been handed out: the rows are rewritten out of L2 by the warps that
-// finish first while the others still compute, and by all of them at the end.
-// MEASURED (cfg2, one B200, tools/dev_fused.py): correct (equal to the two-launch path to 1 ulp on every case) and
-// SLOWER -- 155 us per step against 130 us for fbank_warp_kernel + cmvn_apply_kernel: an item is a chain of dependent
-// round trips (ticket, queue slot, descriptor, sums, rows) that 1.4 items per warp cannot hide, where the stand-alone
-// kernel has 1280 CTAs in flight.  Taking items INSIDE the span loop (to overlap them with the FFTs) makes ptxas keep
-// the quad loop's statistics registers on the stack whether the call is inlined or not (~30 local accesses per quad;
-// 174 us with the span body moved out of line instead, because kernel parameters then stop being constant-bank
-// operands), and a compare-and-swap claim serialises at one item per L2 round trip (3.3 ms).  Hence a build switch
-// (LIDFE_WFUSED_BUILD), off by default; the two-launch path stays the product.
-__device__ __noinline__ void announce_frames_warp(const FbankParams& P, int utt, int frames_held) {
-  const int lane = threadIdx.x & 31;
-  int* const done_cur = P.utt_done + (P.parity & 1) * P.b_cap;
-  __threadfence();       // release: this warp's rows and sums before its frames are announced
-  __syncwarp();
-  int complete = 0;
-  if (lane == 0) complete = (atomicAdd(&done_cur[utt], frames_held) + frames_held == static_cast<int>(__ldg(P.utt_frames + utt)));
-  complete = __shfl_sync(0xffffffffu, complete, 0);
-  if (!complete) return;
-  const int first = __ldg(P.utt_first_item + utt), n = __ldg(P.utt_first_item + utt + 1) - first;
-  int base = 0;
-  if (lane == 0) {
-    done_cur[utt] = 0;                                    // back to rest: nobody adds to a complete utterance
-    base = atomicAdd(&P.wq[0], n);
-  }
-  base = __shfl_sync(0xffffffffu, base, 0);
-  __threadfence();
-  for (int i = lane; i < n; i += 32) st_volatile_i(&P.wq[4 + base + i], first + i + 1);
-}
-
-__device__ __noinline__ void second_stage_warp(const FbankParams& P, unsigned char* scratch, int n_out) {
-  const int lane = threadIdx.x & 31;
-  float4* const c4 = reinterpret_cast<float4*>(scratch);                          // mean | inv | lo: 60 float4
-  float* const cf = reinterpret_cast<float*>(c4);
-  int* const amasks = reinterpret_cast<int*>(cf + 3 * kMaxMels);                   // [kMaxMasks][4]
-  const double* const stats_cur = P.utt_stats + static_cast<long long>(P.parity & 1) * P.b_cap * 2 * n_out;
-  for (;;) {
-    int e = -1;
-    if (lane == 0) {
-      // a ticket per item: the warp has no spans left, so waiting for a slot that other warps have yet to publish costs
-      // nothing (and cannot dead-lock: whoever still computes does not wait for anything)
-      const int slot = atomicAdd(&P.wq[1], 1);
-      if (slot < P.n_items) {
-        while ((e = ld_volatile_i(&P.wq[4 + slot])) == 0) __nanosleep(64);
-        P.wq[4 + slot] = 0;                               // the slot goes back to rest
-        __threadfence();                                  // acquire: the utterance's sums and rows
-        e -= 1;
-      }
-    }
-    e = __shfl_sync(0xffffffffu, e, 0);
-    if (e < 0) return;
-    const int4 item = __ldg(&P.items[e]);                 // (utt, first row, rows, frames of the utterance)
-    const int utt = item.x;
-    for (int d = lane; d < n_out; d += 32) {
-      const double n = static_cast<double>(item.w);
-      const double sm = __ldcg(stats_cur + (static_cast<long long>(utt) * 2 + 0) * n_out + d);
-      const double ss = __ldcg(stats_cur + (static_cast<long long>(utt) * 2 + 1) * n_out + d);
-      const double mu = sm / n;
-      double var = (ss - sm * mu) / (n - 1.0);            // n == 1 -> NaN, as torch.std of one sample
-      var = var > 0.0 ? var : (var == var ? 0.0 : var);
-      const float mean = static_cast<float>(mu);
-      cf[d] = mean;
-      cf[kMaxMels + d] = static_cast<float>(1.0 / (sqrt(var) + 1e-9));
-      cf[2 * kMaxMels + d] = static_cast<float>(-(mu - static_cast<double>(mean)) / (sqrt(var) + 1e-9));
-    }
-    if (P.n_masks > 0 && lane < P.n_masks * 4) amasks[lane] = __ldg(P.masks + static_cast<long long>(utt) * P.n_masks * 4 + lane);
-    if (item.y == 0) {         // first item of the utterance: the other launch parity's sums go back to rest
-      double* os = P.utt_stats + (static_cast<long long>((P.parity & 1) ^ 1) * P.b_cap + utt) * 2 * n_out;
-      for (int q = lane; q < 2 * n_out; q += 32) os[q] = 0.0;
-    }
-    __syncwarp();
-    const bool fast = (n_out == 80) && (P.out_ld % 4 == 0) && ((reinterpret_cast<uintptr_t>(P.out) & 15) == 0);
-    apply_rows_warp(P.out + (__ldg(P.utt_out_row + utt) + item.y) * P.out_ld, P.out_ld, n_out, P.n_masks, fast, item.y, item.z,
-                    1, 0.f, c4, amasks);
-    __syncwarp();              // the scratch is free again
-  }
-}
 
 // kStats: 0 = no statistics, 1 = sums for per-utterance / global CMVN, 2 = per-utterance extrema for AmplitudeToDB(top_db)
 template <typename TIn, int kStdMel, int kStats>
@@ -320,11 +218,6 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
   int frames_acc = 0;                  // mode 3: frames of the spans this warp has processed
   float ex_max = -INFINITY, ex_min = INFINITY;      // kExt: extrema of held_utt's features seen by this lane
   int held_utt = -1;                   // mode 1: whose sums the accumulators hold
-  int frames_held = 0;                 // mode 1, fused second stage: frames of held_utt in the accumulators
-
-  // per-utterance second stage inside this kernel: compiled in only with -DLIDFE_WFUSED_BUILD=1 (see the note above
-  // announce_frames_warp: it is slower than the second launch, and its mere presence costs the statistics variant 4 us)
-  const bool fused2 = LIDFE_WFUSED_BUILD && kSums && mode == 1 && P.n_items > 0;
 
   while (have_cur) {
     // the next span's descriptor travels into the other slot while this span runs
@@ -400,7 +293,7 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
       const int n_quads = (sp_nframes + kQuadFrames - 1) / kQuadFrames;
       // the statistics-free instantiations have the registers the sums would take: the lane's 8 split twiddles stay
       // resident for the span (16 wavefronts per quad less on the shared-memory pipe)
-      constexpr bool kTw2Regs = LIDFE_TW2_REGS && (kStats != 1);
+      constexpr bool kTw2Regs = (kStats != 1);
       float2 tw2r[8];
       if constexpr (kTw2Regs) {
     #pragma unroll
@@ -447,7 +340,7 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
           }
 
           float mA = 0.f, mB = 0.f;
-          if ((kStdMel == 1 && !LIDFE_UNIT_SHORTCUT) || (kStdMel == 0 && P.remove_dc)) {
+          if (kStdMel == 0 && P.remove_dc) {
             f2 sA = make_float2(0.f, 0.f), sB = make_float2(0.f, 0.f);
     #pragma unroll
             for (int j = 0; j < 13; ++j) {
@@ -466,27 +359,6 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
             mB = __fdiv_rn(sum.y, static_cast<float>(kFrameLen));
           }
           const float c = P.preemph;
-          auto frame_pass = [&](auto unit_tag) {
-            constexpr bool kUnit = decltype(unit_tag)::value;
-            f2 to_prev = make_float2(0.f, 0.f);
-    #pragma unroll
-            for (int j = 0; j < 13; ++j) {
-              const int n = t + 16 * j;
-              const float2 w = *reinterpret_cast<const float2*>(sm_window + 2 * n);
-              const f2 te = make_float2(__fsub_rn(x[j].x, mA), __fsub_rn(x[j + 5].x, mB));   // x[2n]   - mean
-              const f2 to = make_float2(__fsub_rn(x[j].y, mA), __fsub_rn(x[j + 5].y, mB));   // x[2n+1] - mean
-              const f2 send = (t == 15) ? to_prev : to;
-              f2 tp;
-              tp.x = __shfl_sync(0xffffffffu, send.x, up_lane);
-              tp.y = __shfl_sync(0xffffffffu, send.y, up_lane);
-              if (j == 0 && t == 0) tp = te;
-              to_prev = to;
-              const f2 se = kUnit ? sub2(te, tp) : sub2(te, mul2(tp, bc(c)));
-              const f2 so = kUnit ? sub2(to, te) : sub2(to, mul2(te, bc(c)));
-              R[j] = mul2(se, bc(w.x));
-              I[j] = mul2(so, bc(w.y));
-            }
-          };
           if (kStdMel == 2) {
             // the reference's torch.stft call: window only; the (A, B) pairs are formed by the scalar multiplies themselves
     #pragma unroll
@@ -495,7 +367,7 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
               R[j] = make_float2(__fmul_rn(x[j].x, w.x), __fmul_rn(x[j + 5].x, w.x));
               I[j] = make_float2(__fmul_rn(x[j].y, w.y), __fmul_rn(x[j + 5].y, w.y));
             }
-          } else if (kStdMel == 1 && LIDFE_UNIT_SHORTCUT) {
+          } else if (kStdMel == 1) {
             // The reference's call (DC removal, then pre-emphasis with coefficient 1.0, replicate-left): every output is
             // (x[n] - m) - (x[n-1] - m), and y[0] = (x[0] - m) - (x[0] - m) = 0.  The frame mean m only enters through the
             // rounding of the two inner differences; x[n] - x[n-1] rounded ONCE is the same value with less round-off (the
@@ -505,7 +377,7 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
             // shuffles can serve both frames (13 + 13 otherwise); only B's first sample (replicate-left) differs.  Same
             // values either way.  The shared form holds 18 floats at once: it pays in the statistics variant (-2 us on the
             // per-utterance CMVN step) and spills in the statistics-free one, hence the choice per instantiation.
-            constexpr bool kPreShare = LIDFE_PRE_SHARE || (kStats == 1);
+            constexpr bool kPreShare = (kStats == 1);
             if constexpr (kPreShare) {
               float q[18];
     #pragma unroll
@@ -540,8 +412,26 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
                 I[j] = mul2(so, bc(w.y));
               }
             }
-          } else if (kStdMel == 1) frame_pass(std::true_type{});
-          else frame_pass(std::false_type{});
+          } else {
+            f2 to_prev = make_float2(0.f, 0.f);
+    #pragma unroll
+            for (int j = 0; j < 13; ++j) {
+              const int n = t + 16 * j;
+              const float2 w = *reinterpret_cast<const float2*>(sm_window + 2 * n);
+              const f2 te = make_float2(__fsub_rn(x[j].x, mA), __fsub_rn(x[j + 5].x, mB));   // x[2n]   - mean
+              const f2 to = make_float2(__fsub_rn(x[j].y, mA), __fsub_rn(x[j + 5].y, mB));   // x[2n+1] - mean
+              const f2 send = (t == 15) ? to_prev : to;
+              f2 tp;
+              tp.x = __shfl_sync(0xffffffffu, send.x, up_lane);
+              tp.y = __shfl_sync(0xffffffffu, send.y, up_lane);
+              if (j == 0 && t == 0) tp = te;
+              to_prev = to;
+              const f2 se = sub2(te, mul2(tp, bc(c)));
+              const f2 so = sub2(to, mul2(te, bc(c)));
+              R[j] = mul2(se, bc(w.x));
+              I[j] = mul2(so, bc(w.y));
+            }
+          }
           if (t >= 8) R[12] = I[12] = make_float2(0.f, 0.f);
           R[13] = R[14] = R[15] = I[13] = I[14] = I[15] = make_float2(0.f, 0.f);
         }
@@ -552,16 +442,8 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
           // (re_A, re_B) and (im_A, im_B) of a point go out as the two halves of its 16-byte element; the twiddle of point
           // p + 2 is requested before point p is multiplied, so that its shared-memory latency hides behind two complex
           // multiplications instead of stalling each one
-    #if !LIDFE_XPOSE_ST128
-          f2* const X2 = reinterpret_cast<f2*>(X_pl);
-    #endif
           float2 wa = sm_tw1[rev4(1) * 16 + t], wb = sm_tw1[rev4(2) * 16 + t];
-    #if LIDFE_XPOSE_ST128
           X_pl[t] = make_float4(R[0].x, R[0].y, I[0].x, I[0].y);
-    #else
-          X2[2 * t] = R[0];
-          X2[2 * t + 1] = I[0];
-    #endif
     #pragma unroll
           for (int p = 1; p < 16; ++p) {
             const int K1 = rev4(p);
@@ -569,12 +451,7 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
             wa = wb;
             if (p + 2 < 16) wb = sm_tw1[rev4(p + 2) * 16 + t];
             cmul2(R[p], I[p], w.x, w.y);
-    #if LIDFE_XPOSE_ST128
             X_pl[K1 * kXRow + t] = make_float4(R[p].x, R[p].y, I[p].x, I[p].y);
-    #else
-            X2[2 * (K1 * kXRow + t)] = R[p];
-            X2[2 * (K1 * kXRow + t) + 1] = I[p];
-    #endif
           }
         }
         __syncwarp();
@@ -750,7 +627,6 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
         // order of the fp64 additions)
         if (quads_since_fold) fold();
         frames_acc += sp_nframes;
-        frames_held += sp_nframes;
         held_utt = read_span(cur).utt;
       }
     }
@@ -797,10 +673,6 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
           if (a != 0.0) atomicAdd(g + e, a);
           if (b2 != 0.0) atomicAdd(g + n_out + e, b2);
         }
-        if (fused2) {
-          announce_frames_warp(P, held_utt, frames_held);
-        }
-        frames_held = 0;
         held_utt = -1;
       }
     }
@@ -813,9 +685,6 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
     }
     nxt_idx = __shfl_sync(0xffffffffu, nxt_idx, 0);
   }
-
-  // ---- out of spans: the second stage of whatever is (or becomes) ready ------------------------------------------------
-  if (fused2) second_stage_warp(P, wbase + WL::off_plane, n_out);
 
   // ---- out of work: global sums leave the CTA once; the last CTA puts the claim counter back to rest ----------------
   if (kSums && mode == 3) {
@@ -835,10 +704,6 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
     if (atomicAdd(&P.sched[1], 1) == static_cast<int>(gridDim.x) - 1) {
       P.sched[0] = 0;
       P.sched[1] = 0;
-      if (fused2) {
-        P.wq[0] = 0;
-        P.wq[1] = 0;
-      }
     }
   }
 }

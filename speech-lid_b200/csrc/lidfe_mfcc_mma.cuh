@@ -20,20 +20,14 @@
 // of a launch are 18.5 us by themselves; 8 warps per SM with two tiles per pass were slower (47 us), 16 warps with one
 // tile per pass are what is kept.  The HBM floor (15 us) would need the tcgen05 path (resample_tc_kernel's machinery
 // plus a K-major workspace), not built.
-// Scope: n_mels % 8 == 0, n_ceps <= 40; other shapes stay with mfcc_dct_kernel (LIDFE_DCT_MMA=0 forces it).
+// Scope: n_mels % 8 == 0, n_ceps <= 40; other shapes stay with mfcc_dct_kernel.
 #pragma once
 #include "lidfe_kernels.cuh"
 
 namespace lidfe {
 
-#ifndef LIDFE_MM_TM
-#define LIDFE_MM_TM 1          // tiles per pass and warp
-#endif
-#ifndef LIDFE_MM_THREADS
-#define LIDFE_MM_THREADS 256
-#endif
-constexpr int kMmTM = LIDFE_MM_TM;
-constexpr int kMmThreads = LIDFE_MM_THREADS;
+constexpr int kMmTM = 1;                        // tiles per pass and warp
+constexpr int kMmThreads = 256;
 constexpr int kMmWarps = kMmThreads / 32;
 constexpr int kMmMaxKS = kMaxMels / 8;          // k-steps (8 mel bins each)
 constexpr int kMmMaxNT = kDctMaxCeps / 8;       // 8-column blocks of cepstra

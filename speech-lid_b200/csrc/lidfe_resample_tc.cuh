@@ -23,9 +23,6 @@
 
 namespace lidfe {
 
-#ifndef LIDFE_TC_ABL
-#define LIDFE_TC_ABL 0      // development: 1 = gather from a 4 KB region (no memory latency), 2 = no MMAs, 4 = no B copies
-#endif
 constexpr int kTcM = 128;            // frames per CTA = rows of A = TMEM lanes
 constexpr int kTcKB = 32;            // taps per pipeline stage = one 128-byte swizzle row
 constexpr int kTcThreads = 512;      // warp 0: B loader, 1: MMA issuer + TMEM owner, 4-11: A builders, 12-15: epilogue
@@ -42,7 +39,6 @@ struct ResampleTcParams {
   int orig, nw, K, KB, width;        // KB = ceil(K / 32) tap blocks
   int N, stages, tmem_cols;          // phases per CTA (multiple of 32, <= 256), pipeline depth, allocated TMEM columns (2 buffers)
   int gx, B, n_tiles;                // tile grid: frame tiles per utterance (of the longest), utterances, phase tiles
-  long long* dbg;                    // development (LIDFE_TC_DBG): per-role cycle counters of CTA 0, else NULL
 };
 
 template <bool kRelaxed = false>
@@ -151,7 +147,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
         for (int kb = 0; kb < P.KB; ++kb, ++item) {
           const uint32_t s = item % P.stages, u = item / P.stages;
           if (u > 0) tc_wait<true>(&empty[s], (u - 1) & 1u);
-          if (LIDFE_TC_ABL & 4) { mbar_arrive(&full_b[s]); continue; }
           mbar_expect_tx(&full_b[s], static_cast<uint32_t>(2 * b_bytes));
           tma_bulk_g2s_plain(base + s * stage_bytes + 2 * kTcABytes, src + static_cast<long long>(kb) * 2 * b_bytes,
                              static_cast<uint32_t>(2 * b_bytes), &full_b[s]);
@@ -165,41 +160,31 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
       const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(P.N >> 3) << 17) |
                              (static_cast<uint32_t>(kTcM >> 4) << 24);
       uint32_t item = 0, seq = 0;
-      long long t_wa = 0, t_wb = 0, t_we = 0, t_iss = 0, t_all = clock64();
       for (long long L = next_live(blockIdx.x); L < n_lin; L = next_live(L + gridDim.x), ++seq) {
         const uint32_t a = seq & 1u;
         if (seq >= 2) {                                            // the epilogue has drained this buffer's previous tile
-          const long long c0 = clock64();
           tc_wait(&acc_empty[a], ((seq >> 1) - 1) & 1u);
-          t_we += clock64() - c0;
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         }
         const uint32_t d_addr = tmem_d + a * acc_stride;
         for (int kb = 0; kb < P.KB; ++kb, ++item) {
           const uint32_t s = item % P.stages, u = item / P.stages;
-          const long long c0 = clock64();
           tc_wait(&full_a[s], u & 1u);
-          const long long c1 = clock64();
           tc_wait(&full_b[s], u & 1u);
-          const long long c2 = clock64();
-          t_wa += c1 - c0; t_wb += c2 - c1;
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t a_hi = smem_u32(base + s * stage_bytes), a_lo = a_hi + kTcABytes;
           const uint32_t b_hi = a_hi + 2 * kTcABytes, b_lo = b_hi + b_bytes;
 #pragma unroll
           for (int j = 0; j < kTcKB / 8; ++j) {                    // K = 8 tf32 = 32 bytes per instruction
             const uint32_t off = 32u * j;
-            if (LIDFE_TC_ABL & 2) continue;
             tc_mma_tf32(d_addr, tc_smem_desc(a_lo + off), tc_smem_desc(b_hi + off), idesc, (kb | j) ? 1u : 0u);
             tc_mma_tf32(d_addr, tc_smem_desc(a_hi + off), tc_smem_desc(b_lo + off), idesc, 1u);
             tc_mma_tf32(d_addr, tc_smem_desc(a_hi + off), tc_smem_desc(b_hi + off), idesc, 1u);
           }
           tc_commit(&empty[s]);                                    // the stage is free once these MMAs have read it
-          t_iss += clock64() - c2;
         }
         tc_commit(&acc_full[a]);
       }
-      if (P.dbg && blockIdx.x == 0) { P.dbg[0] = clock64() - t_all; P.dbg[1] = t_wa; P.dbg[2] = t_wb; P.dbg[3] = t_we; P.dbg[4] = t_iss; P.dbg[5] = seq; }
     }
   } else if (warp >= 4 && warp < 12) {
     // ---- A builders: warps 4-7 take the even pipeline items, warps 8-11 the odd ones; warp (set, q) gathers rows
@@ -234,10 +219,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
       const float* const src = p.x + j0;
       if (j0 >= 0 && j0 + 31ll * P.orig < p.n_in && p.kb * kTcKB + 31 < P.K) {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) v[i] = __ldg(src + ((LIDFE_TC_ABL & 1) ? ((i * P.orig) & 1023) - j0 + (j0 & 1023) : i * P.orig));
+        for (int i = 0; i < 32; ++i) v[i] = __ldg(src + i * P.orig);
         // a row moves on by one 128-byte line per tap block: ask L2 for the line this warp's NEXT-BUT-ONE block will
         // touch (its own next block is already being loaded into the other register buffer) -- the builders' exposed
-        // DRAM latency was 40 % of the tile (cycle counters, LIDFE_TC_DBG)
+        // DRAM latency was 40 % of the tile (clock64 cycle counters)
         if (lane == 0 && j0 + 31ll * P.orig + 5 * kTcKB < p.n_in) {
 #pragma unroll
           for (int i = 0; i < 32; ++i) asm volatile("prefetch.global.L2 [%0];" ::"l"(src + i * P.orig + 4 * kTcKB + 31));
@@ -252,19 +237,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
     };
     const uint32_t a_lane = static_cast<uint32_t>(32 * q * 128 + ((lane & 3) << 2));   // row 32 q, this lane's word in a chunk
     const uint32_t chunk = static_cast<uint32_t>(lane >> 2);
-    long long t_be = 0, t_bp = 0, t_bg = 0, t_st = 0;
     auto publish = [&](uint32_t item, const float (&v)[32]) {
       const uint32_t s = item % P.stages, u = item / P.stages;
-      const long long c0 = clock64();
       if (u > 0) tc_wait(&empty[s], (u - 1) & 1u);
-      const long long c1 = clock64();
-      t_be += c1 - c0;
       const uint32_t a_hi = smem_u32(base + s * stage_bytes) + a_lane;
-      if (P.dbg) { float acc = 0.f;
-#pragma unroll
-        for (int i = 0; i < 32; ++i) acc += v[i];
-        if (acc == 1.2345e-30f) t_bg += 1; t_bg += clock64() - c1; }
-      const long long c1b = clock64();
 #pragma unroll
       for (int i = 0; i < 32; ++i) {                               // row 32 q + i: chunk c goes to position c ^ (row % 8)
         uint32_t hi, lo;
@@ -273,11 +249,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
         asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(hi) : "memory");
         asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr + kTcABytes), "r"(lo) : "memory");
       }
-      const long long c1c = clock64();
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> visible to the tensor core
       __syncwarp();
       if (lane == 0) mbar_arrive(&full_a[s]);                      // (128 arrivals on one mbarrier cost 0.26 us per item)
-      t_bp += clock64() - c1; t_st += c1c - c1b;
     };
     Pos p;
     p.L = next_live(blockIdx.x);
@@ -300,8 +274,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
       if (p.L < n_lin) gather(p, va);
       publish(ib, vb);
     }
-    if (P.dbg && blockIdx.x == 0 && warp == 4 && lane == 0) { P.dbg[8] = t_be; P.dbg[9] = t_bp; P.dbg[12] = t_bg; P.dbg[13] = t_st; }
-    if (P.dbg && blockIdx.x == 0 && warp == 8 && lane == 0) { P.dbg[10] = t_be; P.dbg[11] = t_bp; }
   } else if (warp >= 12) {
     // ---- epilogue: TMEM lane = frame, column = phase; the buffer goes back to the MMA warp as soon as it is in registers --
     const int q = warp - 12;

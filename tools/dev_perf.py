@@ -1,6 +1,5 @@
 #!/usr/bin/env python
-"""Kernel-time probe used during development: cfg2 shapes (256 x 8 s), CUDA events, per cmvn mode.
-env: LIDFE_SPAN_TILES, LIDFE_APPLY_BLOCK are read at FrontEnd creation."""
+"""Kernel-time probe used during development: cfg2 shapes (256 x 8 s), CUDA events, per cmvn mode."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -34,22 +33,4 @@ for mode in modes:
         fe.featurize_packed(ins[i % 3], plan, out=outs[i % 3], **kw)
     e1.record()
     torch.cuda.synchronize()
-    print("span_tiles=%s apply_block=%s spans=%d mode=%-13s %.1f us/step" % (
-        os.environ.get("LIDFE_SPAN_TILES", "auto"), os.environ.get("LIDFE_APPLY_BLOCK", "64"), spans, mode,
-        e0.elapsed_time(e1) / n * 1e3), flush=True)
-if int(os.environ.get("LIDFE_DBG", "0")) & 16:
-    import ctypes, numpy as np
-    torch.cuda.synchronize()
-    buf = (ctypes.c_longlong * (8 * 592))()
-    fe.lib.lidfe_dbg_read.argtypes = [ctypes.c_void_p, ctypes.c_int]
-    print("rc", fe.lib.lidfe_dbg_read(buf, 8 * 592))
-    a = np.array(buf[:]).reshape(592, 8)
-    t0 = a[:, 0].min()
-    sp = (a[:, 1] - t0) / 1e3
-    en = (a[:, 2] - t0) / 1e3
-    st = (a[:, 0] - t0) / 1e3
-    print("start  us: min %.1f max %.1f" % (st.min(), st.max()))
-    print("spans done us: min %.1f p50 %.1f p90 %.1f max %.1f" % (sp.min(), np.percentile(sp, 50), np.percentile(sp, 90), sp.max()))
-    print("end us: min %.1f max %.1f" % (en.min(), en.max()))
-    print("spans/CTA: min %d max %d mean %.1f; blocks/CTA min %d max %d sum %d; drain iters mean %.1f max %d" % (
-        a[:, 3].min(), a[:, 3].max(), a[:, 3].mean(), a[:, 4].min(), a[:, 4].max(), a[:, 4].sum(), a[:, 5].mean(), a[:, 5].max()))
+    print("spans=%d mode=%-13s %.1f us/step" % (spans, mode, e0.elapsed_time(e1) / n * 1e3), flush=True)
