@@ -57,7 +57,6 @@ struct lidfe_ctx {
   int blob_bytes_fbank;    // prefix without dct / lifter (the fbank-only kernel variant of the two-kernel MFCC path)
   int dct_off, lifter_off; // byte offsets of those sections inside the blob
   size_t smem_bytes_fbank;
-  size_t smem_bytes_dct;
   size_t smem_bytes;
   int grid_cap;   // resident CTAs of the fbank kernel on this device
   // warp-autonomous kernel (lidfe_fbank_warp.cuh): used whenever the configuration and the call are inside its scope
@@ -75,7 +74,6 @@ struct lidfe_ctx {
   int prof_used;
   int prof_stride;   // bracket every prof_stride-th featurize call (event records between kernels cost a few us)
   int prof_calls;
-  int dct_mma;     // two-kernel MFCC path: DCT on the tensor cores (lidfe_mfcc_mma.cuh) when the shapes fit (n_mels % 8 == 0)
   // precise mode (lidfe_set_precision, lidfe_fbank_precise.cuh): fp64 arithmetic on the reference's fp32 tables
   int precise;
   int k0_off, melw_off, total_taps;   // the segment-form mel plan inside the blob (the precise kernel reads it from there)
@@ -716,19 +714,14 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
   if (e == cudaSuccess) {
     c->smem_bytes = smem_for(*cfg, total_taps);
     if (cfg->n_ceps > 0 && cfg->n_ceps <= kDctMaxCeps) {
-      // two-kernel MFCC path: fbank-only variant into a log-mel workspace, then mfcc_dct_kernel
+      // two-kernel MFCC path: fbank-only variant into a log-mel workspace, then mfcc_dct_mma_kernel
       lidfe_config fb = *cfg;
       fb.n_ceps = 0;
       c->smem_bytes_fbank = smem_for(fb, total_taps);
       fbank_fn f2 = (cfg->in_dtype == LIDFE_IN_I16) ? pick_kernel_t<short>(false, c->std_mel)
                                                       : pick_kernel_t<float>(false, c->std_mel);
       e = cudaFuncSetAttribute(f2, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->smem_bytes_fbank));
-      c->smem_bytes_dct = (static_cast<size_t>(kDctStages) * kDctMaxTiles * kDctThreads * 4 +
-                           static_cast<size_t>(cfg->n_mels) * kDctMaxCeps + kDctMaxCeps + 2 * kDctMaxCeps) * sizeof(float);
       if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(mfcc_dct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->smem_bytes_dct));
-      c->dct_mma = (cfg->n_mels % 8 == 0) ? 1 : 0;
-      if (e == cudaSuccess && c->dct_mma)
         e = cudaFuncSetAttribute(mfcc_dct_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMmSmemBytes);
     }
     fbank_fn fn = pick_kernel(c);
@@ -915,7 +908,7 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   const size_t in_elt = (h->cfg.in_dtype == LIDFE_IN_I16) ? 2 : 4;
   const bool center = h->cfg.framing == LIDFE_FRAMING_CENTER;
   const long long cpad_w = h->cfg.pad;
-  const bool need_tiles = h->cfg.n_ceps > 0 && h->cfg.n_ceps <= kDctMaxCeps && h->cfg.n_mels % 4 == 0;   // mfcc_dct_kernel's table
+  const bool need_tiles = h->cfg.n_ceps > 0 && h->cfg.n_ceps <= kDctMaxCeps && h->cfg.n_mels % 4 == 0;   // mfcc_dct_mma_kernel's table
   std::vector<long long> frames(B), utt_first_tile(B);
   long long total = 0, n_tiles = 0, max_frames = 0;
   for (int i = 0; i < B; ++i) {
@@ -1415,7 +1408,7 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
   long long grid = p->n_spans < h->grid_cap ? p->n_spans : h->grid_cap;
   if (grid < 1) grid = 1;
   if (mfcc2) {
-    // MFCC without statistics: fbank-only kernel into the log-mel workspace, then the register-tiled DCT kernel
+    // MFCC without statistics: fbank-only kernel into the log-mel workspace, then the tensor-core DCT kernel
     PlanBlock* b = p->blk;
     if (b->logmel_tiles < p->n_tiles) {      // grown on demand, kept with the pooled block
       CU_TRY(cudaStreamSynchronize(st));
@@ -1470,19 +1463,11 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
     D.n_masks = masks_dev ? n_masks : 0;
     D.mode = cmvn_mode;
     D.stats_in = stats_in_dev;
-    // 4 CTAs of 128 threads per SM resident; the tiles are dealt out evenly inside the kernel (one per warp at least)
-    long long groups = (p->n_tiles + 3) / 4;
-    long long gd = groups < static_cast<long long>(h->num_sms) * 4 ? groups : static_cast<long long>(h->num_sms) * 4;
-    if (gd < 1) gd = 1;
-    if (h->dct_mma) {
-      // tensor-core DCT: every warp walks its own contiguous range of tiles; 2 CTAs of 8 warps per SM
-      long long gm = (p->n_tiles + kMmTM * kMmWarps - 1) / (kMmTM * kMmWarps);
-      if (gm > static_cast<long long>(h->num_sms) * 2) gm = static_cast<long long>(h->num_sms) * 2;
-      if (gm < 1) gm = 1;
-      mfcc_dct_mma_kernel<<<static_cast<unsigned>(gm), kMmThreads, kMmSmemBytes, st>>>(D);
-    } else {
-      mfcc_dct_kernel<<<static_cast<unsigned>(gd), kDctThreads, h->smem_bytes_dct, st>>>(D);
-    }
+    // every warp walks its own contiguous range of tiles; 2 CTAs of 8 warps per SM
+    long long gm = (p->n_tiles + kMmTM * kMmWarps - 1) / (kMmTM * kMmWarps);
+    if (gm > static_cast<long long>(h->num_sms) * 2) gm = static_cast<long long>(h->num_sms) * 2;
+    if (gm < 1) gm = 1;
+    mfcc_dct_mma_kernel<<<static_cast<unsigned>(gm), kMmThreads, kMmSmemBytes, st>>>(D);
     g_launches.fetch_add(1);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaEventRecord(p->blk->ev, st));
@@ -1680,8 +1665,6 @@ int lidfe_fp32_probe(float ms_budget, double* tflops_out, void* stream) {
 struct lidfe_resampler_s {
   int orig, nw, K, K4, width;      // frequencies already divided by their gcd
   float* d_wt;                     // [K4][nw] transposed bank (FP32 kernel)
-  int K8, KS, use_mma;             // tensor-core path (nw % 16 == 0): taps padded to 8, shared-memory row stride
-  float* d_w;                      // [nw][K8] row-major bank (tensor-core kernel)
   // tcgen05 path (lidfe_resample_tc.cuh): the bank as shared-memory images, one per (phase tile, 32-tap block, hi | lo)
   int use_tc, tc_N, tc_tiles, tc_KB, tc_stages, tc_cols;
   size_t tc_smem;
@@ -1732,29 +1715,17 @@ static int create_bank(lidfe_resampler* out, int orig, int nw, const float* kern
   cudaError_t e = upload(&r->d_wt, wt.data(), wt.size());
   const size_t smem = static_cast<size_t>(kRsFrames) * r->K4 * sizeof(float);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(resample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-  r->K8 = (taps + 7) & ~7;
-  r->KS = r->K8 + 4;
-  r->d_w = nullptr;
-  // test selectors: LIDFE_RESAMPLE_MMA=0 / LIDFE_RESAMPLE_TC=0 keep the kernels the faster ones are tested against
-  const char* ev = getenv("LIDFE_RESAMPLE_MMA");
-  r->use_mma = (nw % 16 == 0) && !(ev && ev[0] == '0') &&
-               static_cast<size_t>(kRmFrames) * r->KS * sizeof(float) <= 200 * 1024;
-  if (e == cudaSuccess && r->use_mma) {
-    std::vector<float> w(static_cast<size_t>(nw) * r->K8, 0.f);
-    for (int p = 0; p < nw; ++p)
-      for (int k = 0; k < taps; ++k) w[static_cast<size_t>(p) * r->K8 + k] = kernel_host[static_cast<size_t>(p) * taps + k];
-    e = upload(&r->d_w, w.data(), w.size());
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(resample_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               static_cast<int>(static_cast<size_t>(kRmFrames) * r->KS * sizeof(float)));
-  }
-  // tcgen05 path: phases in tiles of N (a multiple of 32 that divides nw, <= 256: 160 for both of the reference's rates)
+  // tcgen05 path: phases in tiles of N, the largest multiple of 32 that divides nw and is <= 256 (160 for both of the
+  // reference's rates), else the largest such multiple of 16 (M = 128 takes any N % 16 == 0 up to 256)
   r->use_tc = 0;
   r->d_wimg = nullptr;
   {
     int N = 0;
-    for (int c = 256; c >= 32; c -= 32)
-      if (nw % c == 0) { N = c; break; }
+    for (int c = 256; c >= 32 && N == 0; c -= 32)
+      if (nw % c == 0) N = c;
+    for (int c = 240; c >= 16 && N == 0; c -= 16)
+      if (nw % c == 0) N = c;
+    // test selector: LIDFE_RESAMPLE_TC=0 keeps resample_kernel, the FP32 reference the tensor-core kernel is tested against
     const char* et = getenv("LIDFE_RESAMPLE_TC");
     int dev = 0, cc_major = 0;
     cudaGetDevice(&dev);
@@ -1763,45 +1734,43 @@ static int create_bank(lidfe_resampler* out, int orig, int nw, const float* kern
       r->tc_N = N;
       r->tc_tiles = nw / N;
       r->tc_KB = (taps + kTcKB - 1) / kTcKB;
+      if (r->tc_KB < 2) r->tc_KB = 2;                         // the builder warps' two sets: a second block of zeros
       const size_t stage = 2 * static_cast<size_t>(kTcABytes) + 2 * static_cast<size_t>(N) * 128;
-      int stages = static_cast<int>((220 * 1024) / stage);
+      int stages = static_cast<int>((220 * 1024) / stage);    // >= 2: a stage is at most 96 KB (N <= 256)
       if (stages > 4) stages = 4;
       if (stages > r->tc_KB) stages = r->tc_KB;
       r->tc_stages = stages;
+      // two accumulator buffers of tc_cols / 2 >= round_up(N, 32) columns each: the epilogue reads 32 columns at a time
       r->tc_cols = 32;
-      while (r->tc_cols < 2 * N) r->tc_cols <<= 1;            // two accumulator buffers of tc_cols / 2 >= N columns each
-      if (r->tc_cols / 2 < N) r->tc_cols = 0;
+      while (r->tc_cols < 2 * ((N + 31) & ~31)) r->tc_cols <<= 1;
       r->tc_smem = stages * stage + 1024 + (3 * static_cast<size_t>(stages) + 5) * 8;
-      if (stages >= 2 && r->tc_cols >= 32 && r->tc_cols <= 512 && r->tc_KB >= 2) {
-        // image of (tile t, block kb, part h): row n (phase t N + n) holds taps 32 kb .. 32 kb + 31 in 128 bytes, its eight
-        // 16-byte chunks XOR-swizzled by n % 8 (the layout tcgen05.mma reads with a SWIZZLE_128B K-major descriptor)
-        const size_t img = static_cast<size_t>(N) * 128;
-        std::vector<float> buf(static_cast<size_t>(r->tc_tiles) * r->tc_KB * 2 * (img / 4), 0.f);
-        for (int t = 0; t < r->tc_tiles; ++t)
-          for (int kb = 0; kb < r->tc_KB; ++kb)
-            for (int n = 0; n < N; ++n)
-              for (int kk = 0; kk < kTcKB; ++kk) {
-                const int k = kb * kTcKB + kk;
-                const float w = (k < taps) ? kernel_host[static_cast<size_t>(t * N + n) * taps + k] : 0.f;
-                const float hi = tf32_rna_host(w), lo = w - hi;
-                const size_t off = (static_cast<size_t>(n) * 128 + ((((kk >> 2) ^ (n & 7)) << 4) | ((kk & 3) << 2))) / 4;
-                const size_t base = (static_cast<size_t>(t) * r->tc_KB + kb) * 2 * (img / 4);
-                buf[base + off] = hi;
-                buf[base + img / 4 + off] = lo;
-              }
-        float* dimg = nullptr;
-        e = upload(&dimg, buf.data(), buf.size());
-        r->d_wimg = reinterpret_cast<unsigned char*>(dimg);
-        if (e == cudaSuccess)
-          e = cudaFuncSetAttribute(resample_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(r->tc_smem));
-        r->use_tc = (e == cudaSuccess);
-      }
+      // image of (tile t, block kb, part h): row n (phase t N + n) holds taps 32 kb .. 32 kb + 31 in 128 bytes, its eight
+      // 16-byte chunks XOR-swizzled by n % 8 (the layout tcgen05.mma reads with a SWIZZLE_128B K-major descriptor)
+      const size_t img = static_cast<size_t>(N) * 128;
+      std::vector<float> buf(static_cast<size_t>(r->tc_tiles) * r->tc_KB * 2 * (img / 4), 0.f);
+      for (int t = 0; t < r->tc_tiles; ++t)
+        for (int kb = 0; kb < r->tc_KB; ++kb)
+          for (int n = 0; n < N; ++n)
+            for (int kk = 0; kk < kTcKB; ++kk) {
+              const int k = kb * kTcKB + kk;
+              const float w = (k < taps) ? kernel_host[static_cast<size_t>(t * N + n) * taps + k] : 0.f;
+              const float hi = tf32_rna_host(w), lo = w - hi;
+              const size_t off = (static_cast<size_t>(n) * 128 + ((((kk >> 2) ^ (n & 7)) << 4) | ((kk & 3) << 2))) / 4;
+              const size_t base = (static_cast<size_t>(t) * r->tc_KB + kb) * 2 * (img / 4);
+              buf[base + off] = hi;
+              buf[base + img / 4 + off] = lo;
+            }
+      float* dimg = nullptr;
+      e = upload(&dimg, buf.data(), buf.size());
+      r->d_wimg = reinterpret_cast<unsigned char*>(dimg);
+      if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(resample_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(r->tc_smem));
+      r->use_tc = (e == cudaSuccess);
     }
   }
   if (e != cudaSuccess) {
     cudaGetLastError();
     cudaFree(r->d_wt);
-    cudaFree(r->d_w);
     cudaFree(r->d_wimg);
     delete r;
     return static_cast<int>(e);
@@ -1813,7 +1782,6 @@ static int create_bank(lidfe_resampler* out, int orig, int nw, const float* kern
 int lidfe_resampler_destroy(lidfe_resampler r) {
   if (!r) return LIDFE_E_NULL;
   cudaFree(r->d_wt);
-  cudaFree(r->d_w);
   cudaFree(r->d_wimg);
   delete r;
   return LIDFE_OK;
@@ -1846,20 +1814,6 @@ int lidfe_resample(lidfe_resampler r, int B, const float* in_dev, const long lon
     CU_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const long long grid = n_lin < sms ? n_lin : sms;         // persistent: one CTA per SM walks the tiles
     resample_tc_kernel<<<static_cast<unsigned>(grid), kTcThreads, r->tc_smem, static_cast<cudaStream_t>(stream)>>>(T);
-    g_launches.fetch_add(1);
-    CU_TRY(cudaGetLastError());
-    return LIDFE_OK;
-  }
-  if (r->use_mma) {
-    ResampleMmaParams M;
-    M.in = in_dev; M.in_off = in_off_dev; M.in_len = in_len_dev;
-    M.out = out_dev; M.out_off = out_off_dev; M.out_len = out_len_dev;
-    M.w = r->d_w; M.orig = r->orig; M.nw = r->nw; M.K = r->K; M.K8 = r->K8; M.KS = r->KS; M.width = r->width;
-    const long long fr = (max_out_len + r->nw - 1) / r->nw;
-    const long long gxm = (fr + kRmFrames - 1) / kRmFrames;
-    if (gxm > 0x7fffffffLL || B > 65535) return LIDFE_E_ARG;
-    resample_mma_kernel<<<dim3(static_cast<unsigned>(gxm), static_cast<unsigned>(B)), kRmWarps * 32,
-                          static_cast<size_t>(kRmFrames) * r->KS * sizeof(float), static_cast<cudaStream_t>(stream)>>>(M);
     g_launches.fetch_add(1);
     CU_TRY(cudaGetLastError());
     return LIDFE_OK;

@@ -1,10 +1,14 @@
 // lidfe_mfcc_mma.cuh -- the DCT-II + lifter of the two-kernel MFCC path (row A5; ta: compliance/kaldi.py:648-666, 669-813) on
 // the tensor cores.
 //
-// [rows x n_mels] . [n_mels x n_ceps] is 6.4 kflop per frame: as FP32 FMAs (mfcc_dct_kernel) it costs 47 us per 512 x 4 s
-// against an HBM floor of 15 us (65 MB of log-mels in, 33 MB of cepstra out).  Here the product runs as 3xTF32
+// The in-kernel DCT epilogue of fbank_kernel re-reads the n_mels x n_ceps matrix from shared memory for every frame pair
+// (+65 % shared-memory wavefronts on a kernel that is bound by exactly that pipe); when no statistics are needed (cmvn
+// none / global apply) the fbank kernel writes the log-mels to a tile-blocked workspace (FbankParams::ws_blocked) and this
+// kernel finishes the job.  [rows x n_mels] . [n_mels x n_ceps] is 6.4 kflop per frame: as FP32 FMAs (a register-tiled
+// kernel, measured, then removed; see git history) it cost 47 us per 512 x 4 s against an HBM floor of 15 us (65 MB of
+// log-mels in, 33 MB of cepstra out).  Here the product runs as 3xTF32
 // (hi = tf32(v), lo = v - hi; D += A_lo B_hi + A_hi B_lo + A_hi B_hi with fp32 accumulation: ~21 mantissa bits per
-// product, the decomposition of the resampler kernels) on mma.sync.m16n8k8 -- 150 MMAs per 16-frame tile:
+// product, the decomposition of resample_tc_kernel) on mma.sync.m16n8k8 -- 150 MMAs per 16-frame tile:
 //   * the tile-blocked log-mel workspace [tile][mel / 4][16 frames][4] IS the A-fragment order: a0 of the 32 lanes for
 //     k-step ks is the 128 contiguous bytes at (2 ks) * 256, a1 the next 128, a2 / a3 the 256 bytes after that;
 //   * every warp owns a contiguous range of tiles; a tile (16 frames, 5 KB) arrives by ONE TMA bulk copy
@@ -14,17 +18,41 @@
 //     per lane, k-step and 8-column block);
 //   * the three partial products are three SWEEPS over the column-block accumulators, so that consecutive MMAs are
 //     independent (a dependent chain of three per accumulator ran at the MMA latency: slower than the FP32 kernel).
-// Epilogue as mfcc_dct_kernel: lifter, global CMVN, SpecAugment zero-fill, stores of two adjacent cepstra per lane.
-// MEASURED (cfg3, 512 x 4 s, one B200): 35-37 us against 47 us for mfcc_dct_kernel (cfg3 step 148 -> 136 us).  ncu: the
+// Epilogue: lifter, global CMVN, SpecAugment zero-fill, stores of two adjacent cepstra per lane.
+// MEASURED (cfg3, 512 x 4 s, one B200): 35-37 us against 47 us for the FP32 kernel (cfg3 step 148 -> 136 us).  ncu: the
 // tensor pipe is 49 % busy -- the legacy mma.sync TF32 path retires an m16n8k8 in 2.8 cycles per SM, so the 1.92 M MMAs
 // of a launch are 18.5 us by themselves; 8 warps per SM with two tiles per pass were slower (47 us), 16 warps with one
 // tile per pass are what is kept.  The HBM floor (15 us) would need the tcgen05 path (resample_tc_kernel's machinery
 // plus a K-major workspace), not built.
-// Scope: n_mels % 8 == 0, n_ceps <= 40; other shapes stay with mfcc_dct_kernel.
+// Scope: n_mels % 4 == 0, n_ceps <= 40 (when n_mels % 8 == 4 the last k-step has half its mel bins, the other half is
+// zero on both sides).
 #pragma once
 #include "lidfe_kernels.cuh"
 
 namespace lidfe {
+
+constexpr int kDctMaxCeps = 40;                 // n_ceps <= 40 takes the two-kernel path
+
+struct DctParams {
+  const float* logmel;      // workspace [n_tiles][n_mels / 4][16][4]
+  float* out;
+  long long out_ld;
+  const Tile* tiles;
+  int n_tiles;
+  int n_mels, n_ceps;       // n_mels % 4 == 0
+  const float* dct;         // [n_mels][n_ceps] device copy
+  const float* lifter;      // [n_ceps]
+  const int* masks;
+  int n_masks;
+  int mode;                 // 0 none, 2 global apply
+  const double* stats_in;   // [2*n_ceps+1] (mode 2)
+};
+
+__device__ __forceinline__ void mma_tf32(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
 
 constexpr int kMmTM = 1;                        // tiles per pass and warp
 constexpr int kMmThreads = 256;
@@ -52,7 +80,7 @@ __global__ void __launch_bounds__(kMmThreads, 2) mfcc_dct_mma_kernel(const __gri
   unsigned char* const bufs = msm + kMmOffBuf + warp * 2 * kMmPairBytes;
 
   const int nm = P.n_mels, nc = P.n_ceps;
-  const int KS = nm >> 3, NT = (nc + 7) >> 3;
+  const int KS = (nm + 7) >> 3, NT = (nc + 7) >> 3;
   const int tile_bytes = kTileFrames * nm * 4;
 
   // ---- this warp's contiguous range of tiles; its first copy goes out before anything else, so that it flies under the
@@ -80,11 +108,11 @@ __global__ void __launch_bounds__(kMmThreads, 2) mfcc_dct_mma_kernel(const __gri
   }
 
   // ---- B images: element (k, n) of the DCT matrix for lane (g, c): b0 = (8 ks + c, 8 nt + g), b1 = (8 ks + c + 4, 8 nt + g)
-  for (int e = tid; e < KS * kMmMaxNT * 64; e += kMmThreads) {      // (column blocks beyond n_ceps are zeros)
+  for (int e = tid; e < KS * kMmMaxNT * 64; e += kMmThreads) {      // (column blocks beyond n_ceps, rows beyond n_mels are zeros)
     const int which = e & 1, ln = (e >> 1) & 31, blk = e >> 6;
     const int ks = blk / kMmMaxNT, nt = blk - ks * kMmMaxNT;
     const int k = 8 * ks + (ln & 3) + 4 * which, n = 8 * nt + (ln >> 2);
-    const float v = (n < nc) ? __ldg(P.dct + k * nc + n) : 0.f;
+    const float v = (n < nc && k < nm) ? __ldg(P.dct + k * nc + n) : 0.f;
     uint32_t hi, lo;
     split_tf32(v, hi, lo);
     s_bhi[e] = __uint_as_float(hi);
@@ -128,13 +156,16 @@ __global__ void __launch_bounds__(kMmThreads, 2) mfcc_dct_mma_kernel(const __gri
 #pragma unroll 2
     for (int ks = 0; ks < KS; ++ks) {
       uint32_t ahi[kMmTM][4], alo[kMmTM][4];
+      // mel bins 8 ks + 4 .. 8 ks + 7 lie past the tile when n_mels % 8 == 4 and this is the last k-step: a2 / a3 must be
+      // zeros, not the stale bytes behind the tile (a NaN there times the zero rows of B is still NaN)
+      const bool quad2 = 8 * ks + 4 < nm;
 #pragma unroll
       for (int i = 0; i < kMmTM; ++i) {
         const float* a = A + i * (kTileFrames * nm) + ks * 128 + lane;
         split_tf32(a[0], ahi[i][0], alo[i][0]);
         split_tf32(a[32], ahi[i][1], alo[i][1]);
-        split_tf32(a[64], ahi[i][2], alo[i][2]);
-        split_tf32(a[96], ahi[i][3], alo[i][3]);
+        split_tf32(quad2 ? a[64] : 0.f, ahi[i][2], alo[i][2]);
+        split_tf32(quad2 ? a[96] : 0.f, ahi[i][3], alo[i][3]);
       }
       // B fragments of the k-step for every column block, then the three partial products as three SWEEPS over the
       // (tile, column block) accumulators: consecutive MMAs are independent (a dependent chain of three per accumulator

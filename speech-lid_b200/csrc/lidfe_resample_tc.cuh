@@ -5,9 +5,9 @@
 // view of the waveform).  One CTA computes 128 consecutive frames of one utterance for N phases:
 //   D[128 frames x N phases] (fp32, in TMEM) = A[128 x K] . B[N x K]^T,  both operands K-major in shared memory,
 // as 3 x TF32: every fp32 value is split once into hi = tf32(v) and lo = v - hi, and D += A_lo.B_hi + A_hi.B_lo + A_hi.B_hi
-// (the product of the two low parts is below fp32 resolution) -- the same decomposition, to the same 1e-5 parity bar,
-// as resample_mma_kernel, but with tcgen05.mma issued by one thread, accumulators in tensor memory, and the operands
-// staged through a 3-stage mbarrier pipeline:
+// (the product of the two low parts is below fp32 resolution), to the 1e-5 parity bar of the FP32 resample_kernel, with
+// tcgen05.mma issued by one thread, accumulators in tensor memory, and the operands staged through a 3-stage mbarrier
+// pipeline:
 //   * B (the FIR bank) is constant: the host lays every (phase tile, 32-tap block) out as the exact shared-memory image
 //     -- rows of 128 bytes, 16-byte chunks XOR-swizzled by (row % 8), hi image then lo image -- so one 1-D TMA bulk copy
 //     (cp.async.bulk, complete_tx on the stage's mbarrier) brings a block in;
@@ -18,6 +18,8 @@
 //     stage back with tcgen05.commit; a last commit tells the builder warps, which double as the epilogue, that the
 //     accumulators are complete: tcgen05.ld (32 lanes x 32 columns per warp and turn) -> registers -> global.
 // SASS of this kernel: UTCHMMA / UTCBAR / LDTM / UBLKCP (profiles/r2_resample_tc_sass.txt).
+// Scope: nw % 16 == 0, any number of taps (fewer than 33 run as two blocks, the second all zeros); resample_kernel takes
+// every other rate pair.
 #pragma once
 #include "lidfe_kernels.cuh"
 
@@ -36,8 +38,8 @@ struct ResampleTcParams {
   const long long* out_off;
   const long long* out_len;
   const unsigned char* wimg;         // [n_tiles][KB][2][N * 128 bytes] shared-memory images of the FIR bank (hi, lo)
-  int orig, nw, K, KB, width;        // KB = ceil(K / 32) tap blocks
-  int N, stages, tmem_cols;          // phases per CTA (multiple of 32, <= 256), pipeline depth, allocated TMEM columns (2 buffers)
+  int orig, nw, K, KB, width;        // KB = max(2, ceil(K / 32)) tap blocks
+  int N, stages, tmem_cols;          // phases per CTA (multiple of 16, <= 256), pipeline depth, allocated TMEM columns (2 buffers)
   int gx, B, n_tiles;                // tile grid: frame tiles per utterance (of the longest), utterances, phase tiles
 };
 
@@ -287,7 +289,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       float* const y = P.out + P.out_off[bb];
       const long long o_row = (f0 + 32 * q + lane) * P.nw + static_cast<long long>(nt) * P.N;
-      for (int c = 0; c < P.N; c += 32) {
+      for (int c = 0; c < P.N; c += 32) {                           // (a buffer is at least round_up(N, 32) columns wide)
         uint32_t r[32];
         const uint32_t taddr = tmem_d + a * acc_stride + (static_cast<uint32_t>(32 * q) << 16) + static_cast<uint32_t>(c);
         asm volatile(
@@ -307,7 +309,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
           if (lane == 0) mbar_arrive(&acc_empty[a]);
         }
         const long long o = o_row + c;
-        if (o + 32 <= n_out && ((reinterpret_cast<uintptr_t>(y + o) & 15) == 0)) {
+        const int nv = P.N - c < 32 ? P.N - c : 32;                // valid columns of this chunk
+        if (nv == 32 && o + 32 <= n_out && ((reinterpret_cast<uintptr_t>(y + o) & 15) == 0)) {
 #pragma unroll
           for (int e = 0; e < 32; e += 4)
             *reinterpret_cast<float4*>(y + o + e) = make_float4(__uint_as_float(r[e]), __uint_as_float(r[e + 1]),
@@ -315,7 +318,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) resample_tc_kernel(const __grid
         } else {
 #pragma unroll
           for (int e = 0; e < 32; ++e)
-            if (o + e < n_out) y[o + e] = __uint_as_float(r[e]);
+            if (e < nv && o + e < n_out) y[o + e] = __uint_as_float(r[e]);
         }
       }
     }

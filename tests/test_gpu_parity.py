@@ -44,6 +44,16 @@ def _norm_rel(got, want):
     return float((got - want).abs().max() / want.abs().max())
 
 
+def _cuda_kernels(fn):
+    """Names of the CUDA kernels that fn() launches (torch.profiler, CUDA activities)."""
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        out = fn()
+        torch.cuda.synchronize()
+    return out, {e.name for e in prof.events()}
+
+
 LOW_BINS = 3            # mel bins 0..2: cancellation dominated for white noise through the 1.0 pre-emphasis
 NORM_REL_LOW = 3e-4
 DEEP_NULL = 9.2         # nepers (40 dB) below the mel bin's median energy over the utterance
@@ -243,6 +253,43 @@ def test_generic_kernel_variant_configs(lid):
         assert torch.allclose(norm[i, :T].cpu(), want, rtol=1e-4, atol=2e-4), (norm[i, :T].cpu() - want).abs().max()
         full = O.cmvn_per_utt(O.kaldi_mfcc(w))
         assert torch.allclose(norm[i, :T].cpu(), full, rtol=1e-3, atol=5e-3), (norm[i, :T].cpu() - full).abs().max()
+    # MFCC of n_mels % 8 == 4 mel bins through the two-kernel path (the tensor-core DCT's last k-step has four mel bins):
+    # ragged padded batch, masks, global CMVN with the raw cepstra's own statistics.  Against the oracle chain, and
+    # against the device's own log-mels times the DCT and lifter in fp64 (the bound of the cfg3 linearity test).  Both
+    # bounds are relative to the range of the raw cepstra, so the normalised output's error is taken back to cepstral
+    # units first: global CMVN multiplies column j's error by 1 / std_j, and a high cepstrum's std is far below the range
+    from speech_lid_b200 import tables
+    for n_mels, n_ceps in ((60, 40), (20, 13)):
+        mf, fb = lid.FrontEnd(n_mels=n_mels, n_ceps=n_ceps), lid.FrontEnd(n_mels=n_mels)
+        lens = (48000, 7000, 20000)
+        wavs = [O.synth_speechlike(n, 970 + i) for i, n in enumerate(lens)]
+        frames = [O.kaldi_num_frames(n) for n in lens]
+        plan, plan_f = mf.make_plan(lens, padded=True), fb.make_plan(lens, padded=True)
+        packed = mf.pack(wavs, plan)
+        raw = mf.featurize_packed(packed, plan).cpu()
+        stats = O.cmvn_stats([raw[i, :T] for i, T in enumerate(frames)]).cuda()
+        torch.manual_seed(13)
+        masks = lid.draw_masks(frames, n_ceps, 0.05, n_ceps // 4, 2).cuda()
+        got, names = _cuda_kernels(lambda: mf.featurize_packed(packed, plan, masks=masks, cmvn="global_apply",
+                                                               stats_in=stats).cpu())
+        assert any("mfcc_dct_mma_kernel" in n for n in names), names
+        logmel = fb.featurize_packed(fb.pack(wavs, plan_f), plan_f).double()
+        lin = ((logmel @ tables.dct_matrix(n_ceps, n_mels).cuda().double()) * tables.lifter(n_ceps, 22.0).cuda().double()).cpu()
+        mean, std = O.cmvn_finalize(stats.cpu())
+        for i, (w, T) in enumerate(zip(wavs, frames)):
+            b = [tuple(int(v) for v in masks[i, q]) for q in range(masks.shape[1])]
+            mask = lambda x: O.apply_mask_bounds(x.T.unsqueeze(0), b)[0].T        # noqa: E731
+            ceps = O.kaldi_mfcc(w, num_ceps=n_ceps, n_mels=n_mels)
+            rel = float((raw[i, :T].double() - lin[i, :T]).abs().max() / lin[i, :T].abs().max())
+            assert rel < 2e-6, (n_mels, i, rel)
+            assert _norm_rel(raw[i, :T], ceps) <= NORM_REL, (n_mels, i, _norm_rel(raw[i, :T], ceps))
+            want64 = mask((lin[i, :T] - mean) / (std + O.CMVN_EPS))
+            rel = float(((got[i, :T].double() - want64).abs() * (std + O.CMVN_EPS)).max() / lin[i, :T].abs().max())
+            assert rel < 2e-6, (n_mels, i, rel)
+            want = mask(O.cmvn_apply(ceps, mean, std)).double()
+            rel = float(((got[i, :T].double() - want).abs() * (std + O.CMVN_EPS)).max() / ceps.abs().max())
+            assert rel <= NORM_REL, (n_mels, i, rel)
+            assert torch.all(got[i, T:] == 0)
 
 
 def test_specaug_masks_bit_exact(fe, lid, golden_dir):

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Device-resident throughput of the other BASELINE configs / branches on one GPU (CUDA events, rotating buffers):
-cfg1 (32 x 3 s fbank), cfg2 without CMVN, cfg3 (512 x 4 s MFCC-40 of 80), the default MelSpectrogram+dB branch on the
-cfg2 shape, int16 input.  One JSON line each; informational (bench.py carries the headline)."""
+cfg1 (32 x 3 s fbank), cfg2 without CMVN, cfg3 (512 x 4 s MFCC-40 of 80) and MFCC-40 of 60 mel, the default
+MelSpectrogram+dB branch on the cfg2 shape, int16 input, the resampler.  One JSON line each; informational (bench.py carries the headline)."""
 import json
 import os
 import sys
@@ -56,6 +56,7 @@ def main():
     run("cfg2: kaldi fbank + SpecAugment + per-utterance CMVN, 256 x 8 s", fb, 256, 128000, masks=masks, cmvn="utt")
     mf = lid.FrontEnd(n_mels=80, n_ceps=40)
     run("cfg3: 40 MFCC of 80 mel (DCT epilogue), 512 x 4 s", mf, 512, 64000)
+    run("MFCC-40 of 60 mel (n_mels % 8 == 4: half a last k-step in the DCT), 512 x 4 s", lid.FrontEnd(n_mels=60, n_ceps=40), 512, 64000)
     ms = lid.FrontEnd(kind="melspec_db", pad=16)
     run("default branch: MelSpectrogram + AmplitudeToDB(top_db=80), pad 16, 256 x 8 s (white noise: nothing to clamp)", ms, 256, 128000)
     run("default branch, last quarter of every utterance 100 dB down (clamp active in a quarter of the row blocks)", ms, 256,
@@ -70,6 +71,7 @@ def main():
         256, 128000)
     run_resample("resample 44.1 kHz -> 16 kHz (475-tap polyphase FIR), 256 x 8 s", 44100, 256, 8.0)
     run_resample("resample 22.05 kHz -> 16 kHz (459-tap polyphase FIR), 256 x 8 s", 22050, 256, 8.0)
+    run_resample("resample 25 kHz -> 16 kHz (45-tap polyphase FIR, 16 phases), 256 x 8 s", 25000, 256, 8.0)
 
 
 def run_resample(name, orig, B, seconds, steps=None, warmup=5):

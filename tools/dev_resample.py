@@ -1,6 +1,5 @@
 #!/usr/bin/env python
-"""Development: the three resampler kernels (tcgen05 / mma.sync / FP32, selected by LIDFE_RESAMPLE_TC / LIDFE_RESAMPLE_MMA
-at Resampler creation) against an fp64 evaluation of the same polyphase sum, on ragged batches, and their timings on
+"""Development: the two resampler kernels (tcgen05 / FP32, selected by LIDFE_RESAMPLE_TC at Resampler creation) against an fp64 evaluation of the same polyphase sum, on ragged batches, and their timings on
 256 x 8 s.  Run under `timeout`."""
 import ctypes as C, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -10,7 +9,6 @@ import speech_lid_b200 as lid
 
 def make(kind, orig):
     os.environ["LIDFE_RESAMPLE_TC"] = "1" if kind == "tc" else "0"
-    os.environ["LIDFE_RESAMPLE_MMA"] = "0" if kind == "fp32" else "1"
     return lid.Resampler(orig, 16000)
 
 
@@ -32,7 +30,7 @@ for orig in ((44100, 22050) if CHECK else ()):
     lens = [int(orig * s) for s in (0.05, 0.31, 1.0, 2.57, 0.011)] + [441, 1, 44101]
     wavs = [torch.randn(n, generator=g) for n in lens]
     ref = None
-    for kind in ("tc", "mma", "fp32"):
+    for kind in ("tc", "fp32"):
         rs = make(kind, orig)
         outs = rs.resample_list([w.cuda() for w in wavs])
         torch.cuda.synchronize()
@@ -49,7 +47,7 @@ for orig in (44100, 22050):
     n = int(orig * seconds)
     gg = torch.Generator(device="cuda").manual_seed(2)
     packed = torch.randn(B * n, device="cuda", generator=gg)
-    for kind in ("tc", "mma", "fp32"):
+    for kind in ("tc", "fp32"):
         rs = make(kind, orig)
         n_out = rs.out_len(n)
         stride = (n_out + 3) // 4 * 4
