@@ -257,6 +257,30 @@ int lidfe_wave_stages(lidfe_handle h, lidfe_plan p, const float* wav_in_dev, flo
 int lidfe_wave_stages_i16(lidfe_handle h, lidfe_plan p, const short* pcm_in_dev, float in_scale, float* wav_out_dev,
                           int normalize, float dither, const float* noise_dev, float preemph, void* stream);
 
+/*
+ * Additive noise at a per-utterance SNR (torchaudio.functional.add_noise), then optionally normalize_wav, per utterance
+ * of the plan, out-of-place (wav_out_dev must not alias wav_in_dev).  in_i16 = 1: wav_in_dev holds int16 PCM, scaled
+ * by in_scale first; 0: float32 samples.  For utterance u with samples x_i, i < n, and noise nu_i:
+ *   a_u = sqrt(E_x / E_nu * 10^(-snr_db_dev[u] / 10)),  E_x = sum x_i^2, E_nu = sum nu_i^2 (fp64, a_u rounded to fp32)
+ *   y_i = fl(x_i + fl(a_u * nu_i))                                   (torchaudio's operation order)
+ * snr = +inf, E_x = 0 or E_nu = 0 give a_u = 0 and y = x bit for bit (torchaudio returns NaN for E_nu = 0).  NaN or
+ * -inf SNRs are not meant to reach the device (the Python layer rejects them); they make the utterance non-finite.
+ * Noise source:
+ *   bank_dev != NULL : nu_i = bank_dev[off_u + (start_u + i) mod len_u], the clip repeating when it is shorter than the
+ *                      utterance.  noise_tab_dev is int64 [3][B]: off_u, len_u, start_u.  An entry that does not
+ *                      satisfy 0 <= off_u, 0 < len_u, off_u + len_u <= bank_len, 0 <= start_u < len_u is never read
+ *                      from: that utterance's output is NaN.
+ *   bank_dev == NULL : nu_i ~ N(0,1), Philox4x32-10 keyed by `seed`, counter (i >> 2, (i >> 2) >> 32, u, 1); the
+ *                      block's words (x, y) and (z, w) are two Box-Muller pairs, u1 = ((r >> 8) + 1) 2^-24,
+ *                      u2 = (r >> 8) 2^-24, sample 4b + 2k takes sqrt(-2 ln u1) cospi(2 u2), 4b + 2k + 1 the sinpi term.
+ *                      noise_tab_dev and bank_len are not read.
+ * normalize != 0 : normalize_wav of y afterwards, the same bits as lidfe_wave_stages(normalize = 1) on y.
+ * snr_db_dev is float32 [B].  Nothing but wav_out_dev is written; gaps between utterances are left as they are.
+ */
+int lidfe_add_noise(lidfe_handle h, lidfe_plan p, const void* wav_in_dev, int in_i16, float in_scale, float* wav_out_dev,
+                    const float* bank_dev, long long bank_len, const long long* noise_tab_dev, const float* snr_db_dev,
+                    unsigned long long seed, int normalize, void* stream);
+
 /* -- measurement --------------------------------------------------------------------------------
  * Between lidfe_profile_begin and lidfe_profile_end every lidfe_featurize call brackets its fused fbank kernel with
  * a CUDA event pair on the launching stream (up to max_launches calls).  lidfe_profile_end synchronises on them and

@@ -28,7 +28,7 @@ EXPORTS = (
     "lidfe_abi_version", "lidfe_launch_count", "lidfe_profile_begin", "lidfe_profile_end", "lidfe_profile_set_stride", "lidfe_mel_plan", "lidfe_mel_plan_expand",
     "lidfe_resampler_create", "lidfe_resampler_destroy", "lidfe_resample_out_len", "lidfe_resample",
     "lidfe_plan_create_async", "lidfe_plan_num_spans", "lidfe_featurize_raw", "lidfe_fp32_probe", "lidfe_pool_stats", "lidfe_pack_host", "lidfe_h2d_gather", "lidfe_wgemm_create", "lidfe_stft_mel_db",
-    "lidfe_set_precision",
+    "lidfe_set_precision", "lidfe_add_noise",
 )
 
 
@@ -127,6 +127,8 @@ def load_library() -> C.CDLL:
     lib.lidfe_resample.restype = i32
     lib.lidfe_wave_stages_i16.argtypes = [vp, vp, vp, f32, vp, i32, f32, vp, f32, vp]
     lib.lidfe_wave_stages_i16.restype = i32
+    lib.lidfe_add_noise.argtypes = [vp, vp, vp, i32, f32, vp, vp, ll, vp, vp, C.c_ulonglong, i32, vp]
+    lib.lidfe_add_noise.restype = i32
     lib.lidfe_strerror.argtypes = [i32]
     lib.lidfe_strerror.restype = C.c_char_p
     lib.lidfe_abi_version.argtypes = []

@@ -35,8 +35,13 @@ def collate_host_part(batch: Sequence[Tuple], lang2index: Dict[str, int]):
 
 class DeviceCollate:
     def __init__(self, frontend, lang2index: Dict[str, int], train: bool = False, t_mask: float = 0.05,
-                 f_mask: int = 27, mask_times: int = 0, cmvn: str = "none"):
+                 f_mask: int = 27, mask_times: int = 0, cmvn: str = "none", noise=None):
+        """``noise``: a ``NoiseAugment`` mixed into the waveforms of training batches (``train=True``) only; its draws
+        come from its own generator, so the SpecAugment masks are the same with noise on or off."""
+        if noise is not None and frontend.in_dtype != torch.float32:
+            raise ValueError("noise augmentation needs a float32 FrontEnd")
         self.frontend = frontend
+        self.noise = noise
         self.lang2index = dict(lang2index)
         self.train = bool(train)
         self.t_mask, self.f_mask, self.mask_times = float(t_mask), int(f_mask), int(mask_times)
@@ -51,6 +56,7 @@ class DeviceCollate:
             # drawn inside featurize once the H2D copies of the waveforms are under way (same RNG consumption)
             def masks(frames):
                 return draw_masks(frames, self.frontend.n_out, self.t_mask, self.f_mask, self.mask_times)
-        feats, wav_percents = self.frontend.featurize(wavs, masks=masks, cmvn=self.cmvn, cache_plan=False)
+        feats, wav_percents = self.frontend.featurize(wavs, masks=masks, cmvn=self.cmvn, cache_plan=False,
+                                                      noise=self.noise if self.train else None)
         texts, text_percents, audio_paths, langs = collate_host_part(batch, self.lang2index)
         return feats, texts, wav_percents.to(torch.float32).cpu(), text_percents, audio_paths, langs

@@ -1236,6 +1236,19 @@ static int launch_apply(lidfe_ctx* h, lidfe_plan p, float* feats, long long ld, 
   return LIDFE_OK;
 }
 
+// noise: kNoiseNone / kNoiseBank / kNoiseGauss (the wave_stages_kernel instantiation)
+static int run_wave(lidfe_plan p, const WaveParams& W, int noise, void* stream) {
+  const dim3 grid(static_cast<unsigned>(p->B) * kWaveCluster);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (noise == kNoiseBank) wave_stages_kernel<kNoiseBank><<<grid, kWaveThreads, 0, st>>>(W);
+  else if (noise == kNoiseGauss) wave_stages_kernel<kNoiseGauss><<<grid, kWaveThreads, 0, st>>>(W);
+  else wave_stages_kernel<kNoiseNone><<<grid, kWaveThreads, 0, st>>>(W);
+  g_launches.fetch_add(1);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaEventRecord(p->blk->ev, st));
+  return LIDFE_OK;
+}
+
 static int launch_wave(lidfe_handle h, lidfe_plan p, const void* in, int in_i16, float in_scale, float* out, float2* norm_out,
                        int normalize, float dither, const float* noise_dev, float preemph, void* stream) {
   if (!h || !p || !in) return LIDFE_E_NULL;
@@ -1254,11 +1267,12 @@ static int launch_wave(lidfe_handle h, lidfe_plan p, const void* in, int in_i16,
   W.noise = noise_dev;
   W.seed = h->cfg.seed;
   W.preemph = preemph;
-  wave_stages_kernel<<<static_cast<unsigned>(p->B) * kWaveCluster, kWaveThreads, 0, static_cast<cudaStream_t>(stream)>>>(W);
-  g_launches.fetch_add(1);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaEventRecord(p->blk->ev, static_cast<cudaStream_t>(stream)));
-  return LIDFE_OK;
+  W.bank = nullptr;
+  W.bank_len = 0;
+  W.noise_tab = nullptr;
+  W.snr_db = nullptr;
+  W.noise_seed = 0;
+  return run_wave(p, W, kNoiseNone, stream);
 }
 
 static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, float* out_dev, long long out_ld,
@@ -1602,6 +1616,30 @@ int lidfe_wave_stages_i16(lidfe_handle h, lidfe_plan p, const short* pcm_in_dev,
                           int normalize, float dither, const float* noise_dev, float preemph, void* stream) {
   if (!wav_out_dev) return LIDFE_E_NULL;
   return launch_wave(h, p, pcm_in_dev, 1, in_scale, wav_out_dev, nullptr, normalize, dither, noise_dev, preemph, stream);
+}
+
+int lidfe_add_noise(lidfe_handle h, lidfe_plan p, const void* wav_in_dev, int in_i16, float in_scale, float* wav_out_dev,
+                    const float* bank_dev, long long bank_len, const long long* noise_tab_dev, const float* snr_db_dev,
+                    unsigned long long seed, int normalize, void* stream) {
+  if (!h || !p || !wav_in_dev || !wav_out_dev || !snr_db_dev) return LIDFE_E_NULL;
+  if (bank_dev && !noise_tab_dev) return LIDFE_E_NULL;
+  if (p->ctx != h || wav_in_dev == static_cast<const void*>(wav_out_dev) || (in_i16 != 0 && in_i16 != 1)) return LIDFE_E_ARG;
+  if (bank_dev && (bank_len <= 0 || bank_dev == wav_out_dev)) return LIDFE_E_ARG;
+  WaveParams W;
+  memset(&W, 0, sizeof(W));
+  W.in = wav_in_dev;
+  W.in_i16 = in_i16;
+  W.in_scale = in_scale;
+  W.out = wav_out_dev;
+  W.offsets = p->d_offsets;
+  W.lengths = p->d_lengths;
+  W.normalize = normalize ? 1 : 0;
+  W.bank = bank_dev;
+  W.bank_len = bank_len;
+  W.noise_tab = noise_tab_dev;
+  W.snr_db = snr_db_dev;
+  W.noise_seed = seed;
+  return run_wave(p, W, bank_dev ? kNoiseBank : kNoiseGauss, stream);
 }
 
 // ---- FP32 ceiling, measured (bench.py's roofline denominator) -----------------------------------------------------

@@ -16,6 +16,7 @@ from typing import List, Optional, Sequence, Tuple, Union
 import torch
 
 from . import _lib, tables
+from .noise import NoiseAugment, NoiseBank, NoiseDraw, noise_table
 
 CMVN_MODES = {"none": _lib.CMVN_NONE, "utt": _lib.CMVN_PER_UTT, "global_apply": _lib.CMVN_APPLY_GLOBAL,
               "global_accum": _lib.CMVN_ACCUM_GLOBAL, "topdb": _lib.POST_TOPDB}
@@ -495,6 +496,42 @@ class FrontEnd:
                                                       st.cuda_stream))
         return out
 
+    def add_noise(self, packed: torch.Tensor, plan: Plan, draw: NoiseDraw, bank: Optional[NoiseBank] = None,
+                  normalize: bool = False, out: Optional[torch.Tensor] = None,
+                  stream: Optional[torch.cuda.Stream] = None, pcm_scale: float = 1.0 / 32768.0) -> torch.Tensor:
+        """Additive noise at each utterance's SNR (``torchaudio.functional.add_noise``; ``noise.py``), then
+        ``normalize_wav`` when ``normalize``: the evaluation chain "load -> add noise -> read_audio(normalize=True)".
+        ``draw`` comes from ``draw_noise`` (with the same ``bank``; ``bank=None`` mixes N(0,1) drawn on the device from
+        ``draw.seed``).  ``packed`` is float32 or int16 PCM (scaled by ``pcm_scale`` first).  Returns a new packed
+        float32 buffer with zeroed gaps (or fills ``out``).  Unlike torchaudio, a zero-energy noise window leaves the
+        utterance clean instead of NaN."""
+        if packed.dtype not in (torch.float32, torch.int16):
+            raise ValueError("add_noise works on float32 samples or int16 PCM")
+        if not packed.is_cuda or not packed.is_contiguous() or packed.numel() < plan.total_samples:
+            raise ValueError("packed must be a contiguous CUDA buffer covering the plan's extent")
+        if out is not None and (out.dtype != torch.float32 or not out.is_cuda or not out.is_contiguous()
+                                or out.numel() < plan.total_samples):
+            raise ValueError("out must be a contiguous float32 CUDA buffer covering the plan's extent")
+        if bank is not None and bank.data.device != packed.device:
+            raise ValueError("the noise bank lives on %s, the samples on %s" % (bank.data.device, packed.device))
+        tab, snr = noise_table(draw, bank, plan.batch)
+        i16 = packed.dtype == torch.int16
+        st = stream if stream is not None else torch.cuda.current_stream(self.device)
+        # the output and the per-utterance tables are allocated and uploaded on the launching stream: nothing is
+        # ordered on another stream, so a side-stream caller needs no synchronisation
+        with torch.cuda.device(self.device), torch.cuda.stream(st):
+            if out is None:
+                out = torch.zeros(packed.numel(), dtype=torch.float32, device=packed.device)
+            snr_d = snr.pin_memory().to(self.device, non_blocking=True)
+            tab_d = tab.pin_memory().to(self.device, non_blocking=True) if tab is not None else None
+            _lib.check(self.lib.lidfe_add_noise(self.handle, plan.handle, packed.data_ptr(), int(i16),
+                                                float(pcm_scale) if i16 else 1.0, out.data_ptr(),
+                                                _ptr(bank.data) if bank is not None else None,
+                                                bank.data.numel() if bank is not None else 0, _ptr(tab_d),
+                                                snr_d.data_ptr(), int(draw.seed) & 0xFFFFFFFFFFFFFFFF, int(normalize),
+                                                st.cuda_stream))
+        return out
+
     def featurize_host(self, host_in: torch.Tensor, plan: Plan, host_out: torch.Tensor,
                        masks: Optional[torch.Tensor] = None, cmvn: str = "none", chunks: int = 8) -> torch.Tensor:
         """Host-buffer entry (what a CPU-side caller of the reference's ``wav2mel`` sees): ``host_in`` is the packed
@@ -557,14 +594,19 @@ class FrontEnd:
         return host_out
 
     def featurize(self, wavs: Sequence[torch.Tensor], masks: Optional[torch.Tensor] = None, cmvn: str = "none",
-                  padded: bool = True, cache_plan: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
+                  padded: bool = True, cache_plan: bool = True,
+                  noise: Optional[NoiseAugment] = None) -> Tuple[torch.Tensor, torch.Tensor]:
         """The batched public entry: list of waveforms -> ``(feats, wav_percents)`` with the collate contract
         (ref: lid/raw_datasets.py:345-365).  ``feats`` stays on the device -- that is where the model consumes it.
         ``cache_plan=False`` (ragged training batches: every batch has its own length signature): the plan is built for
         this call and handed straight back to the handle's pool -- the pool re-uses its block only after the work
         launched here has finished (an event per block), so nothing is allocated or freed in steady state.
         ``masks`` may be a callable ``frames -> int32 [B, n_masks, 4]``: it is evaluated after the H2D copies have been
-        issued (``DeviceCollate`` draws its SpecAugment bounds this way, under the DMA)."""
+        issued (``DeviceCollate`` draws its SpecAugment bounds this way, under the DMA).
+        ``noise``: a ``NoiseAugment``; every call draws its noise and mixes it into the packed waveforms
+        (``add_noise``) before the features are computed.  Needs a float32 FrontEnd."""
+        if noise is not None and self.in_dtype != torch.float32:
+            raise ValueError("noise augmentation needs a float32 FrontEnd (add_noise produces float32 samples)")
         lengths = [int(w.shape[-1]) for w in wavs]
         if cache_plan:
             plan = self.cached_plan(lengths, padded=padded)
@@ -580,6 +622,8 @@ class FrontEnd:
                 pos += (n + self.align - 1) // self.align * self.align
             packed = self.pack(wavs, _Layout(lengths=lengths, offsets=offsets, total_samples=pos))
             plan = self.make_plan(lengths, padded=padded, offsets=offsets)
+        if noise is not None:
+            packed = self.add_noise(packed, plan, noise.draw(plan.batch), bank=noise.bank, normalize=noise.normalize)
         if callable(masks):
             masks = masks(plan.frames)
         out = self.featurize_packed(packed, plan, masks=masks, cmvn=cmvn)
