@@ -340,19 +340,43 @@ def collate_features(specs: Sequence[torch.Tensor]) -> Tuple[torch.Tensor, torch
 # --------------------------------------------------------------------------------------
 # fp64 "truth" with the oracle's fp32 tables (SURVEY.md appendix A.3): calibrates tolerances.
 # --------------------------------------------------------------------------------------
-def truth64_fbank(wav: torch.Tensor, n_mels: int = 80, preemph: float = 1.0) -> torch.Tensor:
+def truth64_fbank(wav: torch.Tensor, n_mels: int = 80, preemph: float = 1.0, window_type: str = "povey",
+                  remove_dc: bool = True, in_scale: float = 1.0) -> torch.Tensor:
+    """``kaldi_fbank`` in float64 on the same fp32 tables: (m, n_mels).  ``in_scale`` multiplies the samples first
+    (int16 PCM); it is rounded to fp32, as the front-end's configuration holds it, and the product is exact in fp64."""
     if wav.dim() == 2:
         wav = wav[0]
-    w = wav.double()
+    w = wav.double() * float(torch.tensor(in_scale, dtype=torch.float32))
     m = kaldi_num_frames(w.numel())
     idx = torch.arange(m)[:, None] * 160 + torch.arange(400)[None]
     fr = w[idx]
-    fr = fr - fr.mean(1, keepdim=True)
-    fr = fr - preemph * torch.cat([fr[:, :1], fr[:, :-1]], 1)
-    fr = torch.nn.functional.pad(fr * povey_window(400).double(), (0, 112))
+    if remove_dc:
+        fr = fr - fr.mean(1, keepdim=True)
+    if preemph != 0.0:
+        fr = fr - preemph * torch.cat([fr[:, :1], fr[:, :-1]], 1)
+    fr = torch.nn.functional.pad(fr * kaldi_window(window_type, 400).double(), (0, 112))
     X = torch.fft.rfft(fr)
     mel = (X.real ** 2 + X.imag ** 2) @ kaldi_mel_banks(n_mels, 512, 16000.0).double().T
     return mel.clamp_min(EPS32).log()
+
+
+def truth64_melspec_db(x: torch.Tensor, pad: int = 0, top_db: Optional[float] = 80.0, n_mels: int = 80) -> torch.Tensor:
+    """``melspec_db`` -- the reference's default branch (ref: lid/audio_processor.py:72-105 -> torch.stft(center=True,
+    reflect), HTK mel, AmplitudeToDB(top_db)) -- in float64 on the fp32 tables: (T, n_mels).  ``top_db=None``: no clamp."""
+    w = x.reshape(-1).double()
+    if pad:
+        w = torch.nn.functional.pad(w, (pad, pad))
+    wp = torch.nn.functional.pad(w[None, None], (256, 256), mode="reflect")[0, 0]
+    T = 1 + w.numel() // 160
+    fr = wp[torch.arange(T)[:, None] * 160 + torch.arange(512)[None]]
+    win = torch.zeros(512, dtype=torch.float64)
+    win[56:456] = torch.hann_window(400).double()
+    X = torch.fft.rfft(fr * win)
+    mel = (X.real ** 2 + X.imag ** 2) @ htk_mel_fbanks(257, 0.0, 8000.0, n_mels, 16000).double()
+    db = 10.0 * torch.log10(mel.clamp_min(1e-10))
+    if top_db is None:
+        return db
+    return torch.maximum(db, db.max() - top_db)
 
 
 # --------------------------------------------------------------------------------------

@@ -738,9 +738,12 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
   }
   // warp-autonomous kernel: KALDI framing without in-kernel dither; the HTK / CENTER variant (std_mel 2) stays with fbank_kernel
   // ... and the reference's default branch as a whole (CENTER framing + HTK-80 bank + window-only framing, pad a multiple
-  // of 4 samples so that interior quads stay 16-byte aligned)
+  // of 16 bytes of input -- 4 float or 8 int16 samples -- so that the interior quads the span builder sends to the bulk
+  // copy stay 16-byte aligned; other pads run fbank_kernel, which checks every span's alignment)
+  const int in_elt = (cfg->in_dtype == LIDFE_IN_I16) ? 2 : 4;
   c->warp_ok = ((cfg->framing == LIDFE_FRAMING_KALDI && cfg->dither == 0.f && c->std_mel != 2) ||
-                (cfg->framing == LIDFE_FRAMING_CENTER && cfg->dither == 0.f && c->std_mel == 2 && cfg->pad % 4 == 0 && cfg->n_ceps == 0)) ? 1 : 0;
+                (cfg->framing == LIDFE_FRAMING_CENTER && cfg->dither == 0.f && c->std_mel == 2 &&
+                 (cfg->pad * in_elt) % 16 == 0 && cfg->n_ceps == 0)) ? 1 : 0;
   // test selector: LIDFE_WARP_KERNEL=0 keeps fbank_kernel, the reference the warp kernel is tested against
   if (const char* env = getenv("LIDFE_WARP_KERNEL")) c->warp_ok = c->warp_ok && atoi(env) != 0;
   if (e == cudaSuccess && c->warp_ok) {

@@ -142,23 +142,6 @@ def test_precise_scope_errors(lid):
         lid.FrontEnd(dither=1e-5, precise=True)       # the in-kernel dither draw stays with the fp32 kernels
 
 
-def _truth64_melspec_db(x, pad=0, top_db=80.0):
-    """The reference's default branch (ref: lid/audio_processor.py:72-105 -> torch.stft(center=True, reflect), HTK mel,
-    AmplitudeToDB(top_db)) in float64 on the fp32 tables: (T, 80)."""
-    w = x[0].double()
-    if pad:
-        w = torch.nn.functional.pad(w, (pad, pad))
-    wp = torch.nn.functional.pad(w[None, None], (256, 256), mode="reflect")[0, 0]
-    T = 1 + w.numel() // 160
-    fr = wp[torch.arange(T)[:, None] * 160 + torch.arange(512)[None]]
-    win = torch.zeros(512, dtype=torch.float64)
-    win[56:456] = torch.hann_window(400).double()
-    X = torch.fft.rfft(fr * win)
-    mel = (X.real ** 2 + X.imag ** 2) @ O.htk_mel_fbanks(257, 0.0, 8000.0, 80, 16000).double()
-    db = 10.0 * torch.log10(mel.clamp_min(1e-10))
-    return torch.maximum(db, db.max() - top_db)
-
-
 @gpu
 def test_precise_default_branch_melspec_db(lid):
     """The precise mode on the reference's DEFAULT branch (row A9): CENTER framing with reflection, periodic Hann window,
@@ -172,7 +155,7 @@ def test_precise_default_branch_melspec_db(lid):
         feats, _ = fe.featurize(wavs)
         feats = feats.cpu()
         for i, w in enumerate(wavs):
-            tru = _truth64_melspec_db(w, pad=pad)
+            tru = O.truth64_melspec_db(w, pad=pad)
             T = tru.shape[0]
             got = feats[i, :T]
             assert float((got.double() - tru).abs().max()) <= 1.0e-5, (pad, i)
