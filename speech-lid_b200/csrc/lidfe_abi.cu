@@ -43,6 +43,7 @@ struct PlanBlock {
   long long logmel_tiles;
 };
 
+// Created value-initialised (new lidfe_ctx()): every scalar member starts at zero.
 struct lidfe_ctx {
   lidfe_config cfg;
   int device;
@@ -59,18 +60,18 @@ struct lidfe_ctx {
   size_t smem_bytes_fbank;
   size_t smem_bytes;
   int grid_cap;   // resident CTAs of the fbank kernel on this device
-  // warp-autonomous kernel (lidfe_fbank_warp.cuh): used whenever the configuration and the call are inside its scope
-  int warp_ok;        // configuration inside its scope (KALDI framing, no in-kernel dither, std_mel 0/1)
-  int w_grid;         // resident CTAs of that kernel
+  // warp-autonomous kernel (lidfe_fbank_warp.cuh); route_for decides when it runs
+  bool warp_off;      // LIDFE_WARP_KERNEL=0 at creation
+  int w_grid;         // resident CTAs of that kernel (0 when the handle cannot use it)
   int w_tab_bytes;    // shared-memory bytes in front of the per-warp areas
   size_t w_smem;      // dynamic shared memory per CTA
-  std::vector<PlanBlock*>* pool;      // free blocks
-  std::mutex* pool_mu;
+  std::vector<PlanBlock*> pool;       // free blocks
+  std::mutex pool_mu;
   long long blocks_allocated;         // device/pinned block allocations made for plans so far (lidfe_pool_stats)
   int live_plans;                     // plans that still point at this handle (guarded by pool_mu)
   bool destroyed;                     // lidfe_destroy was called while plans were alive: the last plan frees the handle
   // optional per-launch timing of the fbank kernel (bench.py's roofline leg)
-  std::vector<cudaEvent_t>* prof_events;
+  std::vector<cudaEvent_t> prof_events;   // empty outside lidfe_profile_begin / lidfe_profile_end
   int prof_used;
   int prof_stride;   // bracket every prof_stride-th featurize call (event records between kernels cost a few us)
   int prof_calls;
@@ -100,12 +101,12 @@ struct lidfe_plan_s {
   long long* d_lengths;   // [B]
   long long* d_utt_first_tile;   // [B]
   Span* d_spans;
-  Span* d_wspans;         // warp spans (NULL when the handle cannot use the warp kernel)
+  Span* d_wspans;         // warp spans (NULL unless plan_can_warp)
   long long n_wspans;
   int n_wstatic;          // spans [0, n_wstatic) are the warps' static runs, the rest is the pool
   int* d_w_first;         // [W + 1] first static span of every warp
   bool all_aligned;       // every utterance starts on a 16-byte boundary (TMA-eligible)
-  Tile* d_tiles;          // MFCC two-kernel path, else NULL
+  Tile* d_tiles;          // MFCC two-kernel path (handle_has_dct_path), else NULL
   long long max_frames;
   long long max_row;      // rows of the output matrix this plan touches
 };
@@ -144,10 +145,8 @@ static fbank_fn pick_kernel_t(bool mfcc, int std_mel) {
   if (mfcc) return std_mel == 1 ? fbank_kernel<TIn, true, 1> : std_mel == 2 ? fbank_kernel<TIn, true, 2> : fbank_kernel<TIn, true, 0>;
   return std_mel == 1 ? fbank_kernel<TIn, false, 1> : std_mel == 2 ? fbank_kernel<TIn, false, 2> : fbank_kernel<TIn, false, 0>;
 }
-static fbank_fn pick_kernel(const lidfe_ctx* c) {
-  const bool mfcc = c->cfg.n_ceps > 0;
-  return c->cfg.in_dtype == LIDFE_IN_I16 ? pick_kernel_t<short>(mfcc, c->std_mel)
-                                         : pick_kernel_t<float>(mfcc, c->std_mel);
+static fbank_fn pick_kernel(int in_dtype, bool mfcc, int std_mel) {
+  return in_dtype == LIDFE_IN_I16 ? pick_kernel_t<short>(mfcc, std_mel) : pick_kernel_t<float>(mfcc, std_mel);
 }
 static size_t smem_for(const lidfe_config& c, int total_taps) {
   const bool mf = c.n_ceps > 0;
@@ -157,6 +156,64 @@ static size_t smem_for(const lidfe_config& c, int total_taps) {
   size_t extra = static_cast<size_t>(total_taps) * 32;   // (wa, wb) per step and lane
   if (c.n_ceps > 0) extra += ((static_cast<size_t>(c.n_mels) * c.n_ceps + 3) & ~static_cast<size_t>(3)) + ((c.n_ceps + 3) & ~3);
   return base + extra * sizeof(float);
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Routing: which kernels serve a featurize call.  route_for holds the rule; lidfe_create sets up, and
+// lidfe_plan_create_async builds the work lists for, whatever its predicates allow.
+// ------------------------------------------------------------------------------------------------------------------
+// fbank_warp_kernel's scope (lidfe_fbank_warp.cuh), as far as the configuration decides it: no in-kernel dither, and
+// KALDI framing with a generic or the Kaldi-80 bank, or the reference's default branch as a whole (CENTER framing,
+// HTK-80 bank, window-only framing, fbank output) with a pad of a multiple of 16 bytes of input (4 float or 8 int16
+// samples), so that the interior quads of a 16-byte aligned utterance stay on 16-byte boundaries
+static bool handle_can_warp(const lidfe_ctx* h) {
+  const lidfe_config& c = h->cfg;
+  const int in_elt = (c.in_dtype == LIDFE_IN_I16) ? 2 : 4;
+  const bool kaldi = c.framing == LIDFE_FRAMING_KALDI && h->std_mel != 2;
+  const bool center = c.framing == LIDFE_FRAMING_CENTER && h->std_mel == 2 && c.n_ceps == 0 && (c.pad * in_elt) % 16 == 0;
+  return c.dither == 0.f && (kaldi || center) && !h->warp_off;
+}
+// ... and every utterance of the plan starts on a 16-byte boundary (the kernel stages quads with bulk copies only)
+static bool plan_can_warp(const lidfe_ctx* h, bool aligned) { return aligned && handle_can_warp(h); }
+// MFCC without statistics may run as fbank into a log-mel workspace, then mfcc_dct_mma_kernel (its table: n_mels % 4 == 0)
+static bool handle_has_dct_path(const lidfe_ctx* h) {
+  return h->cfg.n_ceps > 0 && h->cfg.n_ceps <= kDctMaxCeps && h->cfg.n_mels % 4 == 0;
+}
+
+enum FbankKind { kFbPrecise, kFbWarp, kFbCta };
+// the cmvn_apply_kernel pass after the feature kernels: none, per-utterance normalisation or the top_db clamp (the
+// statistics of this launch's parity), global statistics, masks only
+enum ApplyPass { kApplyNone, kApplyUtt, kApplyTopDb, kApplyGlobal, kApplyMasks };
+struct Route {
+  FbankKind fbank;
+  fbank_fn fn;        // the warp or CTA instantiation (precise: launch_precise picks it)
+  bool dct;           // fbank into the tile-blocked log-mel workspace, then mfcc_dct_mma_kernel into the output
+  ApplyPass apply;
+};
+
+static Route route_for(const lidfe_ctx* h, const lidfe_plan_s* p, int mode, bool raw, bool masks) {
+  Route r = {kFbCta, nullptr, false, kApplyNone};
+  if (mode == LIDFE_CMVN_PER_UTT) r.apply = kApplyUtt;
+  if (mode == LIDFE_POST_TOPDB) r.apply = kApplyTopDb;
+  if (h->precise) {   // fbank_precise_kernel takes statistics but leaves global CMVN and masks to the apply pass
+    r.fbank = kFbPrecise;
+    if (mode == LIDFE_CMVN_APPLY_GLOBAL) r.apply = kApplyGlobal;
+    if (mode == LIDFE_CMVN_NONE && masks) r.apply = kApplyMasks;
+    return r;
+  }
+  const lidfe_config& c = h->cfg;
+  r.dct = handle_has_dct_path(h) && (mode == LIDFE_CMVN_NONE || mode == LIDFE_CMVN_APPLY_GLOBAL);
+  // the warp kernel has no fused normalize_wav load, no in-kernel DCT and takes extrema only in the std_mel 2 variant
+  const bool warp = !raw && plan_can_warp(h, p->all_aligned) && (c.n_ceps == 0 || r.dct) &&
+                    (mode != LIDFE_POST_TOPDB || h->std_mel == 2);
+  if (warp) {
+    const int stats = r.dct ? 0 : (mode == LIDFE_CMVN_PER_UTT || mode == LIDFE_CMVN_ACCUM_GLOBAL) ? 1 : mode == LIDFE_POST_TOPDB ? 2 : 0;
+    r.fbank = kFbWarp;
+    r.fn = pick_warp_kernel(c.in_dtype, h->std_mel, stats);
+  } else {
+    r.fn = pick_kernel(c.in_dtype, c.n_ceps > 0 && !r.dct, h->std_mel);
+  }
+  return r;
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -627,7 +684,6 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
 
   lidfe_ctx* c = new (std::nothrow) lidfe_ctx();
   if (!c) return LIDFE_E_NOMEM;
-  memset(c, 0, sizeof(*c));
   c->cfg = *cfg;
   c->n_out = cfg->n_ceps > 0 ? cfg->n_ceps : cfg->n_mels;
 
@@ -701,30 +757,25 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
   }
   c->blob_bytes = static_cast<int>(blob.size());
 
-  c->pool = new (std::nothrow) std::vector<PlanBlock*>();
-  c->pool_mu = new (std::nothrow) std::mutex();
-  if (!c->pool || !c->pool_mu) {
-    lidfe_destroy(c);
-    return LIDFE_E_NOMEM;
-  }
+  // test selector: LIDFE_WARP_KERNEL=0 keeps fbank_kernel, the reference the warp kernel is tested against
+  if (const char* env = getenv("LIDFE_WARP_KERNEL")) c->warp_off = atoi(env) == 0;
   cudaError_t e = cudaGetDevice(&c->device);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&c->num_sms, cudaDevAttrMultiProcessorCount, c->device);
   if (e == cudaSuccess) e = upload(&c->d_blob, blob.data(), blob.size());
   if (e == cudaSuccess) e = cudaDeviceSynchronize();   // the tables have landed whatever stream the caller launches on
   if (e == cudaSuccess) {
     c->smem_bytes = smem_for(*cfg, total_taps);
-    if (cfg->n_ceps > 0 && cfg->n_ceps <= kDctMaxCeps) {
+    if (handle_has_dct_path(c)) {
       // two-kernel MFCC path: fbank-only variant into a log-mel workspace, then mfcc_dct_mma_kernel
       lidfe_config fb = *cfg;
       fb.n_ceps = 0;
       c->smem_bytes_fbank = smem_for(fb, total_taps);
-      fbank_fn f2 = (cfg->in_dtype == LIDFE_IN_I16) ? pick_kernel_t<short>(false, c->std_mel)
-                                                      : pick_kernel_t<float>(false, c->std_mel);
-      e = cudaFuncSetAttribute(f2, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->smem_bytes_fbank));
+      e = cudaFuncSetAttribute(pick_kernel(cfg->in_dtype, false, c->std_mel), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               static_cast<int>(c->smem_bytes_fbank));
       if (e == cudaSuccess)
         e = cudaFuncSetAttribute(mfcc_dct_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMmSmemBytes);
     }
-    fbank_fn fn = pick_kernel(c);
+    fbank_fn fn = pick_kernel(cfg->in_dtype, cfg->n_ceps > 0, c->std_mel);
     if (e == cudaSuccess)
       e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(c->smem_bytes));
     if (e == cudaSuccess) {
@@ -736,17 +787,7 @@ int lidfe_create(lidfe_handle* out, const lidfe_config* cfg, const float* window
       }
     }
   }
-  // warp-autonomous kernel: KALDI framing without in-kernel dither; the HTK / CENTER variant (std_mel 2) stays with fbank_kernel
-  // ... and the reference's default branch as a whole (CENTER framing + HTK-80 bank + window-only framing, pad a multiple
-  // of 16 bytes of input -- 4 float or 8 int16 samples -- so that the interior quads the span builder sends to the bulk
-  // copy stay 16-byte aligned; other pads run fbank_kernel, which checks every span's alignment)
-  const int in_elt = (cfg->in_dtype == LIDFE_IN_I16) ? 2 : 4;
-  c->warp_ok = ((cfg->framing == LIDFE_FRAMING_KALDI && cfg->dither == 0.f && c->std_mel != 2) ||
-                (cfg->framing == LIDFE_FRAMING_CENTER && cfg->dither == 0.f && c->std_mel == 2 &&
-                 (cfg->pad * in_elt) % 16 == 0 && cfg->n_ceps == 0)) ? 1 : 0;
-  // test selector: LIDFE_WARP_KERNEL=0 keeps fbank_kernel, the reference the warp kernel is tested against
-  if (const char* env = getenv("LIDFE_WARP_KERNEL")) c->warp_ok = c->warp_ok && atoi(env) != 0;
-  if (e == cudaSuccess && c->warp_ok) {
+  if (e == cudaSuccess && handle_can_warp(c)) {
     c->w_tab_bytes = static_cast<int>((kWTabOff + c->blob_bytes_fbank + kMaxMels * 8 + 127) / 128 * 128);
     const size_t per_warp = (cfg->in_dtype == LIDFE_IN_I16) ? WarpLayout<short>::kWarpBytes : WarpLayout<float>::kWarpBytes;
     c->w_smem = static_cast<size_t>(c->w_tab_bytes) + kWWarps * per_warp;
@@ -781,15 +822,8 @@ static void free_block(PlanBlock* b) {
 
 static void destroy_now(lidfe_ctx* h) {
   cudaFree(h->d_blob);
-  if (h->pool) {
-    for (PlanBlock* b : *h->pool) free_block(b);
-    delete h->pool;
-  }
-  delete h->pool_mu;
-  if (h->prof_events) {
-    for (auto& ev : *h->prof_events) cudaEventDestroy(ev);
-    delete h->prof_events;
-  }
+  for (PlanBlock* b : h->pool) free_block(b);
+  for (cudaEvent_t ev : h->prof_events) cudaEventDestroy(ev);
   delete h;
 }
 
@@ -797,8 +831,8 @@ static void destroy_now(lidfe_ctx* h) {
 // and the last one to go frees it.
 int lidfe_destroy(lidfe_handle h) {
   if (!h) return LIDFE_E_NULL;
-  if (h->pool_mu) {
-    std::unique_lock<std::mutex> g(*h->pool_mu);
+  {
+    std::lock_guard<std::mutex> g(h->pool_mu);
     if (h->live_plans > 0) {
       h->destroyed = true;
       return LIDFE_OK;
@@ -850,13 +884,13 @@ static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_til
     // fewer than kPoolAsyncBlocks blocks, a new one (so that a loop that creates and destroys a plan per batch can run
     // ahead of the device); last: wait for a busy block that fits
     constexpr long long kPoolAsyncBlocks = 4;
-    std::lock_guard<std::mutex> g(*h->pool_mu);
+    std::lock_guard<std::mutex> g(h->pool_mu);
     int busy = -1;
-    for (size_t i = 0; i < h->pool->size(); ++i) {
-      PlanBlock* b = (*h->pool)[i];
+    for (size_t i = 0; i < h->pool.size(); ++i) {
+      PlanBlock* b = h->pool[i];
       if (b->Bc >= B && b->Sc >= n_spans && b->Tc >= n_tiles && b->Wc >= n_wspans) {
         if (cudaEventQuery(b->ev) == cudaSuccess) {
-          h->pool->erase(h->pool->begin() + i);
+          h->pool.erase(h->pool.begin() + i);
           *out = b;
           break;
         }
@@ -865,8 +899,8 @@ static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_til
       }
     }
     if (!*out && busy >= 0 && h->blocks_allocated >= kPoolAsyncBlocks) {
-      *out = (*h->pool)[busy];
-      h->pool->erase(h->pool->begin() + busy);
+      *out = h->pool[busy];
+      h->pool.erase(h->pool.begin() + busy);
     }
   }
   if (*out) {
@@ -895,12 +929,57 @@ static int acquire_block(lidfe_ctx* h, int B, long long n_spans, long long n_til
     return static_cast<int>(e);
   }
   {
-    std::lock_guard<std::mutex> g(*h->pool_mu);
+    std::lock_guard<std::mutex> g(h->pool_mu);
     ++h->blocks_allocated;
   }
   *out = b;
   return LIDFE_OK;
 }
+
+constexpr int kZeroRows = 4 * kTileFrames;   // output rows one zero-fill span clears
+
+// The spans of a plan, for both kernels' lists: where a run of frames of utterance i starts in the packed input, and
+// whether its samples may be bulk-copied (aux = 1): the first sample inside the buffer on a 16-byte boundary and, for
+// the warp kernel's quads under CENTER framing, none of them in the padding / reflection (`interior`).
+struct SpanMaker {
+  const long long* offsets;
+  const long long* out_rows;
+  long long in_elt, pad;
+  bool center;
+  // first sample of frame f relative to the utterance's first.  CENTER framing: frame f covers p[160 f - 200, 160 f + 200)
+  // of the constant-padded signal p (the Hann window sits at 56..455 of the 512-point buffer and |FFT|^2 does not see
+  // that shift)
+  long long rel(long long f) const { return center ? f * kFrameShift - kFrameLen / 2 - pad : f * kFrameShift; }
+  // the quad starting at frame q0 (<= 4 frames, never past the utterance's T-th) reads only the utterance's N samples
+  bool quad_interior(long long q0, long long T, long long N) const {
+    const long long fr = (T - q0) < kQuadFrames ? (T - q0) : kQuadFrames;
+    return rel(q0) >= 0 && rel(q0) + fr * kFrameShift + (kFrameLen - kFrameShift) <= N;
+  }
+  Span frames(int i, long long f, long long nf, bool interior) const {
+    Span sp;
+    sp.wav_off = offsets[i] + rel(f);
+    sp.out_row = out_rows[i] + f;
+    sp.nframes = static_cast<int>(nf);
+    sp.utt = i;
+    sp.t0 = static_cast<int>(f);
+    sp.aux = (interior && sp.wav_off >= 0 && (sp.wav_off * in_elt) % 16 == 0) ? 1 : 0;
+    return sp;
+  }
+  // pad_sequence's zeros behind utterance i's T frames (ref: lid/raw_datasets.py:347-350): spans of no frames that
+  // clear up to kZeroRows rows each (aux = rows)
+  void zero_fill(std::vector<Span>& dst, int i, long long T, long long pad_rows) const {
+    for (long long r = T; r < pad_rows; r += kZeroRows) {
+      Span sp;
+      sp.wav_off = 0;
+      sp.out_row = out_rows[i] + r;
+      sp.nframes = 0;
+      sp.utt = i;
+      sp.t0 = static_cast<int>(r);
+      sp.aux = static_cast<int>(pad_rows - r < kZeroRows ? pad_rows - r : kZeroRows);
+      dst.push_back(sp);
+    }
+  }
+};
 
 int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long long* wav_offsets_host,
                             const long long* wav_lengths_host, const long long* out_rows_host,
@@ -908,10 +987,9 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   if (!h || !out || !wav_offsets_host || !wav_lengths_host || !out_rows_host) return LIDFE_E_NULL;
   *out = nullptr;
   if (B <= 0) return LIDFE_E_ARG;
-  const size_t in_elt = (h->cfg.in_dtype == LIDFE_IN_I16) ? 2 : 4;
-  const bool center = h->cfg.framing == LIDFE_FRAMING_CENTER;
-  const long long cpad_w = h->cfg.pad;
-  const bool need_tiles = h->cfg.n_ceps > 0 && h->cfg.n_ceps <= kDctMaxCeps && h->cfg.n_mels % 4 == 0;   // mfcc_dct_mma_kernel's table
+  const SpanMaker mk = {wav_offsets_host, out_rows_host, (h->cfg.in_dtype == LIDFE_IN_I16) ? 2 : 4, h->cfg.pad,
+                       h->cfg.framing == LIDFE_FRAMING_CENTER};
+  const bool dct_path = handle_has_dct_path(h);
   std::vector<long long> frames(B), utt_first_tile(B);
   long long total = 0, n_tiles = 0, max_frames = 0;
   for (int i = 0; i < B; ++i) {
@@ -925,14 +1003,15 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
     max_frames = T > max_frames ? T : max_frames;
     utt_first_tile[i] = n_tiles;
     n_tiles += (T + kTileFrames - 1) / kTileFrames;
-    if (pad_rows_host && need_tiles) n_tiles += (pad_rows_host[i] - T + 4 * kTileFrames - 1) / (4 * kTileFrames);
+    if (pad_rows_host && dct_path) n_tiles += (pad_rows_host[i] - T + kZeroRows - 1) / kZeroRows;
   }
   if (n_tiles > 0x7fffffffLL) return LIDFE_E_ARG;
 
   // ---- spans: runs of <= span_tiles consecutive tiles of one utterance, utterance-major.  Enough spans per CTA that
   //      dynamic claiming balances (>= ~10), as long as possible otherwise (a span end costs two CTA barriers, and in
   //      the per-utterance modes a hand-over of 2 x n_out sums); the spans of the last stretch of the batch are single
-  //      tiles so that the CTAs run dry together.
+  //      tiles so that the CTAs run dry together.  Under CENTER framing fbank_kernel decides per tile which ones touch
+  //      the padding / reflection and stages those element-wise.
   const long long per_cta_tiles = n_tiles / (h->grid_cap > 0 ? h->grid_cap : 1);
   int span_tiles = static_cast<int>(per_cta_tiles / 10);
   if (span_tiles < 1) span_tiles = 1;
@@ -943,25 +1022,13 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   {
     long long tile_no = 0;
     for (int i = 0; i < B; ++i) {
-      const long long T = frames[i], N = wav_lengths_host[i], cpad = h->cfg.pad;
+      const long long T = frames[i];
       for (long long f = 0; f < T;) {
         const int st = (n_tiles - tile_no <= tail_tiles) ? 1 : span_tiles;
         const long long nf = (T - f) < static_cast<long long>(st) * kTileFrames ? (T - f) : static_cast<long long>(st) * kTileFrames;
-        Span sp;
-        sp.out_row = out_rows_host[i] + f;
-        sp.nframes = static_cast<int>(nf);
-        sp.utt = i;
-        sp.t0 = static_cast<int>(f);
-        // first sample of the span relative to the utterance's first sample.  CENTER framing: frame f covers
-        // p[160 f - 200, 160 f + 200) of the constant-padded signal p (the Hann window sits at 56..455 of the 512-point
-        // buffer and |FFT|^2 does not see that shift); tiles that touch the padding / reflection are staged element-wise
-        // (the kernel decides per tile; aux only says whether the span's samples are 16-byte aligned).
-        const long long rel = center ? f * kFrameShift - kFrameLen / 2 - cpad : f * kFrameShift;
-        sp.wav_off = wav_offsets_host[i] + rel;
-        sp.aux = (sp.wav_off >= 0 && ((static_cast<unsigned long long>(sp.wav_off) * in_elt) % 16ull) == 0ull) ? 1 : 0;
-        (void)N;
+        const Span sp = mk.frames(i, f, nf, true);
         spans.push_back(sp);
-        if (need_tiles) {
+        if (dct_path) {
           for (long long g = f; g < f + nf; g += kTileFrames) {
             Tile tl = sp;
             tl.wav_off = sp.wav_off + (g - f) * kFrameShift;
@@ -975,18 +1042,9 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
         f += nf;
       }
       if (pad_rows_host) {
-        for (long long r = T; r < pad_rows_host[i]; r += 4 * kTileFrames) {
-          Span sp;
-          sp.wav_off = 0;
-          sp.out_row = out_rows_host[i] + r;
-          sp.nframes = 0;
-          sp.utt = i;
-          sp.t0 = static_cast<int>(r);
-          const long long left = pad_rows_host[i] - r;
-          sp.aux = static_cast<int>(left < 4 * kTileFrames ? left : 4 * kTileFrames);
-          spans.push_back(sp);
-          if (need_tiles) tiles.push_back(sp);
-        }
+        const size_t z = spans.size();
+        mk.zero_fill(spans, i, T, pad_rows_host[i]);
+        if (dct_path) tiles.insert(tiles.end(), spans.begin() + z, spans.end());
       }
     }
   }
@@ -1013,63 +1071,35 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   std::vector<Span> wspans;
   std::vector<int> w_first;
   bool all_aligned = true;
-  for (int i = 0; i < B; ++i) all_aligned = all_aligned && ((static_cast<unsigned long long>(wav_offsets_host[i]) * in_elt) % 16ull) == 0ull;
-  if (h->warp_ok && all_aligned) {
+  for (int i = 0; i < B; ++i) all_aligned = all_aligned && ((wav_offsets_host[i] * mk.in_elt) % 16) == 0;
+  if (plan_can_warp(h, all_aligned)) {
     long long n_quads = 0;
     for (int i = 0; i < B; ++i) n_quads += (frames[i] + kQuadFrames - 1) / kQuadFrames;
     const long long W = static_cast<long long>(h->w_grid) * kWWarps;
     const long long s_run = (n_quads * 90) / (100 * W);                     // static quads per warp
     const long long static_quads = s_run * W;
     std::vector<Span> pool;
-    // CENTER framing: frame f covers p[160 f - 200, 160 f + 200) of the constant-padded signal (see the span builder above);
-    // a run is cut so that the quads that touch the padding / the reflection -- the first quad of an utterance and its last
-    // one or two -- are spans of their own with aux = 0 (staged element by element), everything else stays on TMA
-    auto push_one = [&](std::vector<Span>& dst, int i, long long f, long long nf, int aux) {
-      Span sp;
-      sp.wav_off = wav_offsets_host[i] + (center ? f * kFrameShift - kFrameLen / 2 - cpad_w : f * kFrameShift);
-      sp.out_row = out_rows_host[i] + f;
-      sp.nframes = static_cast<int>(nf);
-      sp.utt = i;
-      sp.t0 = static_cast<int>(f);
-      sp.aux = aux;
-      dst.push_back(sp);
-    };
+    // CENTER framing: a run is cut so that the quads that touch the padding / the reflection -- the first quad of an
+    // utterance and its last one or two -- are spans of their own with aux = 0 (staged element by element), everything
+    // else stays on TMA
     auto push_frames = [&](std::vector<Span>& dst, int i, long long f, long long nf) {
-      if (!center) {
-        push_one(dst, i, f, nf, 1);
+      if (!mk.center) {
+        dst.push_back(mk.frames(i, f, nf, true));
         return;
       }
-      const long long N = wav_lengths_host[i];
-      auto interior = [&](long long q0) {          // quad starting at frame q0 (<= 4 frames, never past the utterance's last)
-        const long long fr = (frames[i] - q0) < kQuadFrames ? (frames[i] - q0) : kQuadFrames;
-        const long long rel = q0 * kFrameShift - kFrameLen / 2 - cpad_w;
-        return rel >= 0 && rel + fr * kFrameShift + (kFrameLen - kFrameShift) <= N;
-      };
+      auto interior = [&](long long q0) { return mk.quad_interior(q0, frames[i], wav_lengths_host[i]); };
       long long g = f;
       while (g < f + nf) {                          // maximal runs of quads of one kind
         const bool in0 = interior(g);
         long long e = g + kQuadFrames;
         while (e < f + nf && interior(e) == in0) e += kQuadFrames;
         if (e > f + nf) e = f + nf;
-        push_one(dst, i, g, e - g, in0 ? 1 : 0);
+        dst.push_back(mk.frames(i, g, e - g, in0));
         g = e;
       }
     };
-    if (pad_rows_host) {
-      for (int i = 0; i < B; ++i) {
-        for (long long r = frames[i]; r < pad_rows_host[i]; r += 64) {
-          Span sp;
-          sp.wav_off = 0;
-          sp.out_row = out_rows_host[i] + r;
-          sp.nframes = 0;
-          sp.utt = i;
-          sp.t0 = static_cast<int>(r);
-          const long long left = pad_rows_host[i] - r;
-          sp.aux = static_cast<int>(left < 64 ? left : 64);
-          pool.push_back(sp);
-        }
-      }
-    }
+    if (pad_rows_host)
+      for (int i = 0; i < B; ++i) mk.zero_fill(pool, i, frames[i], pad_rows_host[i]);
     std::vector<std::vector<Span>> per_warp(static_cast<size_t>(W));
     long long quad_no = 0;      // quads dealt out so far
     for (int i = 0; i < B; ++i) {
@@ -1115,7 +1145,7 @@ int lidfe_plan_create_async(lidfe_handle h, lidfe_plan* out, int B, const long l
   }
   p->blk = b;
   {
-    std::lock_guard<std::mutex> g(*h->pool_mu);
+    std::lock_guard<std::mutex> g(h->pool_mu);
     ++h->live_plans;
   }
   const BlockLayout L = block_layout(b->Bc, b->Sc, b->Tc, b->Wc, h->n_out, static_cast<long long>(h->w_grid) * kWWarps);
@@ -1181,8 +1211,8 @@ int lidfe_plan_destroy(lidfe_plan p) {
   lidfe_ctx* h = p->ctx;
   bool last = false;
   if (p->blk) {
-    std::lock_guard<std::mutex> g(*h->pool_mu);
-    h->pool->push_back(p->blk);
+    std::lock_guard<std::mutex> g(h->pool_mu);
+    h->pool.push_back(p->blk);
     --h->live_plans;
     last = h->destroyed && h->live_plans == 0;
   }
@@ -1192,9 +1222,9 @@ int lidfe_plan_destroy(lidfe_plan p) {
 }
 int lidfe_pool_stats(lidfe_handle h, long long* blocks_allocated, long long* blocks_free) {
   if (!h || !blocks_allocated || !blocks_free) return LIDFE_E_NULL;
-  std::lock_guard<std::mutex> g(*h->pool_mu);
+  std::lock_guard<std::mutex> g(h->pool_mu);
   *blocks_allocated = h->blocks_allocated;
-  *blocks_free = static_cast<long long>(h->pool->size());
+  *blocks_free = static_cast<long long>(h->pool.size());
   return LIDFE_OK;
 }
 long long lidfe_plan_total_frames(lidfe_plan p) { return p ? p->total_frames : 0; }
@@ -1239,6 +1269,20 @@ static int launch_apply(lidfe_ctx* h, lidfe_plan p, float* feats, long long ld, 
   return LIDFE_OK;
 }
 
+// the wave_stages_kernel parameters every caller sets; the stages it does not name start off
+static WaveParams wave_params(lidfe_plan p, const void* in, int in_i16, float in_scale, float* out, int normalize) {
+  WaveParams W;
+  memset(&W, 0, sizeof(W));
+  W.in = in;
+  W.in_i16 = in_i16;
+  W.in_scale = in_scale;
+  W.out = out;
+  W.offsets = p->d_offsets;
+  W.lengths = p->d_lengths;
+  W.normalize = normalize;
+  return W;
+}
+
 // noise: kNoiseNone / kNoiseBank / kNoiseGauss (the wave_stages_kernel instantiation)
 static int run_wave(lidfe_plan p, const WaveParams& W, int noise, void* stream) {
   const dim3 grid(static_cast<unsigned>(p->B) * kWaveCluster);
@@ -1257,25 +1301,119 @@ static int launch_wave(lidfe_handle h, lidfe_plan p, const void* in, int in_i16,
   if (!h || !p || !in) return LIDFE_E_NULL;
   if (!out && !norm_out) return LIDFE_E_NULL;
   if (p->ctx != h || in == static_cast<const void*>(out)) return LIDFE_E_ARG;
-  WaveParams W;
-  W.in = in;
-  W.in_i16 = in_i16;
-  W.in_scale = in_scale;
-  W.out = out;
+  WaveParams W = wave_params(p, in, in_i16, in_scale, out, normalize);
   W.norm_out = norm_out;
-  W.offsets = p->d_offsets;
-  W.lengths = p->d_lengths;
-  W.normalize = normalize;
   W.dither = dither;
   W.noise = noise_dev;
   W.seed = h->cfg.seed;
   W.preemph = preemph;
-  W.bank = nullptr;
-  W.bank_len = 0;
-  W.noise_tab = nullptr;
-  W.snr_db = nullptr;
-  W.noise_seed = 0;
   return run_wave(p, W, kNoiseNone, stream);
+}
+
+// fbank_precise_kernel on the call's parameters: fp64 arithmetic on the same tables, statistics of this launch's parity
+static void launch_precise(const lidfe_ctx* h, lidfe_plan p, const FbankParams& P, cudaStream_t st) {
+  PreciseParams Q;
+  memset(&Q, 0, sizeof(Q));
+  Q.wav = P.wav;
+  Q.out = P.out;
+  Q.out_ld = P.out_ld;
+  Q.spans = P.spans;
+  Q.n_spans = P.n_spans;
+  Q.window = reinterpret_cast<const float*>(h->d_blob);
+  Q.mel_k0 = reinterpret_cast<const int*>(h->d_blob + h->k0_off);
+  Q.mel_w = reinterpret_cast<const float*>(h->d_blob + h->melw_off);
+  for (int b = 0; b < kBands; ++b) Q.band_taps[b] = h->band_taps[b];
+  Q.total_taps = h->total_taps;
+  Q.dct = h->cfg.n_ceps > 0 ? reinterpret_cast<const float*>(h->d_blob + h->dct_off) : nullptr;
+  Q.lifter = h->cfg.n_ceps > 0 ? reinterpret_cast<const float*>(h->d_blob + h->lifter_off) : nullptr;
+  Q.n_mels = P.n_mels;
+  Q.n_ceps = P.n_ceps;
+  Q.n_out = P.n_out;
+  Q.preemph = P.preemph;
+  Q.in_scale = P.in_scale;
+  Q.log_floor = P.log_floor;
+  Q.log_of_floor = P.log_of_floor;
+  Q.log_mul = (h->cfg.log_kind == LIDFE_LOG_DB10) ? 4.3429448190325182765 : 1.0;     // 10 / ln 10
+  Q.center = P.center;
+  Q.pad = P.pad;
+  Q.utt_offsets = P.utt_offsets;
+  Q.utt_lengths = P.utt_lengths;
+  Q.utt_max = P.utt_max + static_cast<long long>(P.parity & 1) * P.b_cap;
+  Q.utt_min = P.utt_min + static_cast<long long>(P.parity & 1) * P.b_cap;
+  Q.remove_dc = P.remove_dc;
+  Q.mode = P.mode;
+  Q.utt_stats = P.utt_stats + static_cast<long long>(P.parity & 1) * P.b_cap * 2 * h->n_out;
+  Q.stats_out = P.stats_out;
+  long long gp = p->n_spans * kMaxSpanTiles < static_cast<long long>(h->num_sms) * kPCtasPerSm ? p->n_spans * kMaxSpanTiles : static_cast<long long>(h->num_sms) * kPCtasPerSm;
+  if (gp < 1) gp = 1;
+  void (*pk)(const PreciseParams) =
+      (h->cfg.in_dtype == LIDFE_IN_I16) ? (Q.center ? fbank_precise_kernel<short, true> : fbank_precise_kernel<short, false>)
+                                        : (Q.center ? fbank_precise_kernel<float, true> : fbank_precise_kernel<float, false>);
+  pk<<<static_cast<unsigned>(gp), kPThreads, kPSmemBytes, st>>>(Q);
+}
+
+// The route's feature kernel, bracketed by an event pair between lidfe_profile_begin and lidfe_profile_end (every
+// prof_stride-th call).
+static int launch_fbank(lidfe_ctx* h, lidfe_plan p, const Route& r, FbankParams& F, cudaStream_t st) {
+  bool prof = h->prof_used + 2 <= static_cast<int>(h->prof_events.size());
+  if (prof) prof = (h->prof_calls++ % (h->prof_stride > 0 ? h->prof_stride : 1)) == 0;
+  if (prof) CU_TRY(cudaEventRecord(h->prof_events[h->prof_used], st));
+  if (r.fbank == kFbPrecise) {
+    launch_precise(h, p, F, st);
+  } else if (r.fbank == kFbWarp) {
+    F.wspans = p->d_wspans;
+    F.n_wspans = static_cast<int>(p->n_wspans);
+    F.w_first = p->d_w_first;
+    F.n_wstatic = p->n_wstatic;
+    F.w_tab_bytes = h->w_tab_bytes;
+    F.const_bytes = h->blob_bytes_fbank;
+    long long grid = (p->n_wspans + kWWarps - 1) / kWWarps;      // (never more warps than spans)
+    if (grid > h->w_grid || p->n_wstatic > 0) grid = h->w_grid;
+    if (grid < 1) grid = 1;
+    r.fn<<<static_cast<unsigned>(grid), kWThreads, h->w_smem, st>>>(F);
+  } else {
+    // the fbank-only variant of the two-kernel MFCC path runs 4 CTAs per SM; a static head of ~85 % of the spans is
+    // dealt out as consecutive runs
+    const long long cap = r.dct ? static_cast<long long>(h->num_sms) * 4 : h->grid_cap;
+    long long grid = p->n_spans < cap ? p->n_spans : cap;
+    if (grid < 1) grid = 1;
+    const long long ks = ((p->n_spans / grid) * 85) / 100;
+    F.k_static = static_cast<int>(ks < 1 ? 1 : ks);
+    r.fn<<<static_cast<unsigned>(grid), kThreads, r.dct ? h->smem_bytes_fbank : h->smem_bytes, st>>>(F);
+  }
+  g_launches.fetch_add(1);
+  CU_TRY(cudaGetLastError());
+  if (prof) {
+    CU_TRY(cudaEventRecord(h->prof_events[h->prof_used + 1], st));
+    h->prof_used += 2;
+  }
+  return LIDFE_OK;
+}
+
+// mfcc_dct_mma_kernel: the log-mel workspace's tiles x DCT x lifter into the call's output (P: the call's parameters)
+static int launch_dct(const lidfe_ctx* h, lidfe_plan p, const FbankParams& P, cudaStream_t st) {
+  DctParams D;
+  D.logmel = p->blk->d_logmel;
+  D.out = P.out;
+  D.out_ld = P.out_ld;
+  D.tiles = p->d_tiles;
+  D.n_tiles = static_cast<int>(p->n_tiles);
+  D.n_mels = h->cfg.n_mels;
+  D.n_ceps = h->cfg.n_ceps;
+  D.dct = reinterpret_cast<const float*>(h->d_blob + h->dct_off);
+  D.lifter = reinterpret_cast<const float*>(h->d_blob + h->lifter_off);
+  D.masks = P.masks;
+  D.n_masks = P.n_masks;
+  D.mode = P.mode;
+  D.stats_in = P.stats_in;
+  // every warp walks its own contiguous range of tiles; 2 CTAs of 8 warps per SM
+  long long gm = (p->n_tiles + kMmTM * kMmWarps - 1) / (kMmTM * kMmWarps);
+  if (gm > static_cast<long long>(h->num_sms) * 2) gm = static_cast<long long>(h->num_sms) * 2;
+  if (gm < 1) gm = 1;
+  mfcc_dct_mma_kernel<<<static_cast<unsigned>(gm), kMmThreads, kMmSmemBytes, st>>>(D);
+  g_launches.fetch_add(1);
+  CU_TRY(cudaGetLastError());
+  return LIDFE_OK;
 }
 
 static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, float* out_dev, long long out_ld,
@@ -1286,7 +1424,9 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
   if (out_ld < h->n_out || cmvn_mode < 0 || cmvn_mode > 4 || n_masks < 0 || n_masks > kMaxMasks) return LIDFE_E_ARG;
   if (cmvn_mode == LIDFE_CMVN_APPLY_GLOBAL && !stats_in_dev) return LIDFE_E_NULL;
   if (cmvn_mode == LIDFE_CMVN_ACCUM_GLOBAL && !stats_out_dev) return LIDFE_E_NULL;
+  if (raw && h->precise) return LIDFE_E_ARG;      // the precise kernel has no fused normalize_wav load
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const Route r = route_for(h, p, cmvn_mode, raw, masks_dev && n_masks > 0);
 
   if (raw) {   // statistics pre-pass of normalize_wav: (mean, std + 1e-6) per utterance; the fused kernel applies them
     const int rc = launch_wave(h, p, wav_dev, h->cfg.in_dtype == LIDFE_IN_I16 ? 1 : 0, h->cfg.in_scale, nullptr, p->d_utt_wnorm, 1,
@@ -1340,94 +1480,11 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
   P.stats_out = stats_out_dev;
   P.utt_stats = p->d_utt_stats;
 
-  if (h->precise) {
-    // precise mode: fp64 arithmetic in fbank_precise_kernel (statistics included), normalisation / masks in the apply kernel
-    if (raw) return LIDFE_E_ARG;
-    PreciseParams Q;
-    memset(&Q, 0, sizeof(Q));
-    Q.wav = wav_dev;
-    Q.out = out_dev;
-    Q.out_ld = out_ld;
-    Q.spans = p->d_spans;
-    Q.n_spans = static_cast<int>(p->n_spans);
-    Q.window = reinterpret_cast<const float*>(h->d_blob);
-    Q.mel_k0 = reinterpret_cast<const int*>(h->d_blob + h->k0_off);
-    Q.mel_w = reinterpret_cast<const float*>(h->d_blob + h->melw_off);
-    for (int b = 0; b < kBands; ++b) Q.band_taps[b] = h->band_taps[b];
-    Q.total_taps = h->total_taps;
-    Q.dct = h->cfg.n_ceps > 0 ? reinterpret_cast<const float*>(h->d_blob + h->dct_off) : nullptr;
-    Q.lifter = h->cfg.n_ceps > 0 ? reinterpret_cast<const float*>(h->d_blob + h->lifter_off) : nullptr;
-    Q.n_mels = h->cfg.n_mels;
-    Q.n_ceps = h->cfg.n_ceps;
-    Q.n_out = h->n_out;
-    Q.preemph = h->cfg.preemph;
-    Q.in_scale = h->cfg.in_scale;
-    Q.log_floor = h->cfg.log_floor;
-    Q.log_of_floor = P.log_of_floor;
-    Q.log_mul = (h->cfg.log_kind == LIDFE_LOG_DB10) ? 4.3429448190325182765 : 1.0;     // 10 / ln 10
-    Q.center = P.center;
-    Q.pad = P.pad;
-    Q.utt_offsets = p->d_offsets;
-    Q.utt_lengths = p->d_lengths;
-    Q.utt_max = p->d_utt_max + static_cast<long long>(P.parity & 1) * P.b_cap;
-    Q.utt_min = p->d_utt_min + static_cast<long long>(P.parity & 1) * P.b_cap;
-    Q.remove_dc = h->cfg.remove_dc;
-    Q.mode = cmvn_mode;
-    Q.utt_stats = p->d_utt_stats + static_cast<long long>(P.parity & 1) * P.b_cap * 2 * h->n_out;
-    Q.stats_out = stats_out_dev;
-    long long gp = p->n_spans * kMaxSpanTiles < static_cast<long long>(h->num_sms) * kPCtasPerSm ? p->n_spans * kMaxSpanTiles : static_cast<long long>(h->num_sms) * kPCtasPerSm;
-    if (gp < 1) gp = 1;
-    {
-      void (*pk)(const PreciseParams) =
-          (h->cfg.in_dtype == LIDFE_IN_I16) ? (Q.center ? fbank_precise_kernel<short, true> : fbank_precise_kernel<short, false>)
-                                            : (Q.center ? fbank_precise_kernel<float, true> : fbank_precise_kernel<float, false>);
-      pk<<<static_cast<unsigned>(gp), kPThreads, kPSmemBytes, st>>>(Q);
-    }
-    g_launches.fetch_add(1);
-    CU_TRY(cudaGetLastError());
-    if (cmvn_mode == LIDFE_CMVN_PER_UTT) return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 1, P.parity);
-    if (cmvn_mode == LIDFE_POST_TOPDB) return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 2, P.parity);
-    if (cmvn_mode == LIDFE_CMVN_APPLY_GLOBAL) return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, stats_in_dev, st, 1);
-    if (cmvn_mode == LIDFE_CMVN_NONE && masks_dev && n_masks > 0) return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 0);
-    CU_TRY(cudaEventRecord(p->blk->ev, st));
-    return LIDFE_OK;
-  }
-
-  // the warp-autonomous kernel takes every call inside its scope (see lidfe_fbank_warp.cuh)
-  const bool use_warp = h->warp_ok && !raw && p->d_wspans != nullptr &&
-                        (cmvn_mode != LIDFE_POST_TOPDB || h->std_mel == 2);
-  auto launch_warp = [&](FbankParams& F, bool profile) -> int {
-    F.wspans = p->d_wspans;
-    F.n_wspans = static_cast<int>(p->n_wspans);
-    F.w_tab_bytes = h->w_tab_bytes;
-    F.const_bytes = h->blob_bytes_fbank;
-    long long grid_w = (p->n_wspans + kWWarps - 1) / kWWarps;      // (never more warps than spans)
-    if (grid_w > h->w_grid || p->n_wstatic > 0) grid_w = h->w_grid;
-    if (grid_w < 1) grid_w = 1;
-    F.w_first = p->d_w_first;
-    F.n_wstatic = p->n_wstatic;
-    fbank_fn wf = pick_warp_kernel(h->cfg.in_dtype, h->std_mel,
-                                   (F.mode == LIDFE_CMVN_PER_UTT || F.mode == LIDFE_CMVN_ACCUM_GLOBAL) ? 1 : F.mode == LIDFE_POST_TOPDB ? 2 : 0);
-    bool prof = profile && h->prof_events && (h->prof_used + 2 <= static_cast<int>(h->prof_events->size()));
-    if (prof) prof = (h->prof_calls++ % (h->prof_stride > 0 ? h->prof_stride : 1)) == 0;
-    if (prof) CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used], st));
-    wf<<<static_cast<unsigned>(grid_w), kWThreads, h->w_smem, st>>>(F);
-    g_launches.fetch_add(1);
-    CU_TRY(cudaGetLastError());
-    if (prof) {
-      CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used + 1], st));
-      h->prof_used += 2;
-    }
-    return LIDFE_OK;
-  };
-
-  const bool mfcc2 = p->d_tiles && (cmvn_mode == LIDFE_CMVN_NONE || cmvn_mode == LIDFE_CMVN_APPLY_GLOBAL);
-  long long grid = p->n_spans < h->grid_cap ? p->n_spans : h->grid_cap;
-  if (grid < 1) grid = 1;
-  if (mfcc2) {
-    // MFCC without statistics: fbank-only kernel into the log-mel workspace, then the tensor-core DCT kernel
+  FbankParams F = P;
+  if (r.dct) {
+    // fbank-only: log-mels into the tile-blocked workspace, grown on demand and kept with the pooled block
     PlanBlock* b = p->blk;
-    if (b->logmel_tiles < p->n_tiles) {      // grown on demand, kept with the pooled block
+    if (b->logmel_tiles < p->n_tiles) {
       CU_TRY(cudaStreamSynchronize(st));
       cudaFree(b->d_logmel);
       b->d_logmel = nullptr;
@@ -1436,7 +1493,6 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
       CU_TRY(cudaMalloc(reinterpret_cast<void**>(&b->d_logmel), static_cast<size_t>(cap) * kTileFrames * h->cfg.n_mels * sizeof(float)));
       b->logmel_tiles = cap;
     }
-    FbankParams F = P;
     F.out = b->d_logmel;
     F.out_ld = h->cfg.n_mels;
     F.n_ceps = 0;
@@ -1446,82 +1502,19 @@ static int featurize_impl(lidfe_handle h, lidfe_plan p, const void* wav_dev, flo
     F.mode = LIDFE_CMVN_NONE;
     F.ws_blocked = 1;
     F.const_bytes = h->blob_bytes_fbank;
-    fbank_fn f2 = (h->cfg.in_dtype == LIDFE_IN_I16) ? pick_kernel_t<short>(false, h->std_mel)
-                                                     : pick_kernel_t<float>(false, h->std_mel);
-    long long g2 = p->n_spans < static_cast<long long>(h->num_sms) * 4 ? p->n_spans : static_cast<long long>(h->num_sms) * 4;
-    if (g2 < 1) g2 = 1;
-    F.k_static = static_cast<int>((p->n_spans / g2) * 85 / 100);
-    if (F.k_static < 1) F.k_static = 1;
-    if (use_warp) {
-      const int rcw = launch_warp(F, true);
-      if (rcw != LIDFE_OK) return rcw;
-    } else {
-      const bool prof2 = h->prof_events && (h->prof_used + 2 <= static_cast<int>(h->prof_events->size()));
-      if (prof2) CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used], st));
-      f2<<<static_cast<unsigned>(g2), kThreads, h->smem_bytes_fbank, st>>>(F);
-      g_launches.fetch_add(1);
-      CU_TRY(cudaGetLastError());
-      if (prof2) {
-        CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used + 1], st));
-        h->prof_used += 2;
-      }
-    }
-    DctParams D;
-    D.logmel = b->d_logmel;
-    D.out = out_dev;
-    D.out_ld = out_ld;
-    D.tiles = p->d_tiles;
-    D.n_tiles = static_cast<int>(p->n_tiles);
-    D.n_mels = h->cfg.n_mels;
-    D.n_ceps = h->cfg.n_ceps;
-    D.dct = reinterpret_cast<const float*>(h->d_blob + h->dct_off);
-    D.lifter = reinterpret_cast<const float*>(h->d_blob + h->lifter_off);
-    D.masks = masks_dev;
-    D.n_masks = masks_dev ? n_masks : 0;
-    D.mode = cmvn_mode;
-    D.stats_in = stats_in_dev;
-    // every warp walks its own contiguous range of tiles; 2 CTAs of 8 warps per SM
-    long long gm = (p->n_tiles + kMmTM * kMmWarps - 1) / (kMmTM * kMmWarps);
-    if (gm > static_cast<long long>(h->num_sms) * 2) gm = static_cast<long long>(h->num_sms) * 2;
-    if (gm < 1) gm = 1;
-    mfcc_dct_mma_kernel<<<static_cast<unsigned>(gm), kMmThreads, kMmSmemBytes, st>>>(D);
-    g_launches.fetch_add(1);
-    CU_TRY(cudaGetLastError());
+  }
+  int rc = launch_fbank(h, p, r, F, st);
+  if (rc == LIDFE_OK && r.dct) rc = launch_dct(h, p, P, st);
+  if (rc != LIDFE_OK) return rc;
+
+  if (r.apply == kApplyNone) {
     CU_TRY(cudaEventRecord(p->blk->ev, st));
     return LIDFE_OK;
   }
-
-  if (use_warp && h->cfg.n_ceps == 0) {
-    const int rcw = launch_warp(P, true);
-    if (rcw != LIDFE_OK) return rcw;
-    if (cmvn_mode == LIDFE_POST_TOPDB)
-      return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 2, P.parity);
-    if (cmvn_mode == LIDFE_CMVN_PER_UTT)
-      return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, 1, P.parity);
-    CU_TRY(cudaEventRecord(p->blk->ev, st));
-    return LIDFE_OK;
-  }
-
-  // static head of the schedule: ~85 % of the spans are dealt out as consecutive runs
-  {
-    const long long ks = ((p->n_spans / grid) * 85) / 100;
-    P.k_static = static_cast<int>(ks < 1 ? 1 : ks);
-  }
-  fbank_fn fn = pick_kernel(h);
-  bool prof = h->prof_events && (h->prof_used + 2 <= static_cast<int>(h->prof_events->size()));
-  if (prof) prof = (h->prof_calls++ % (h->prof_stride > 0 ? h->prof_stride : 1)) == 0;
-  if (prof) CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used], st));
-  fn<<<static_cast<unsigned>(grid), kThreads, h->smem_bytes, st>>>(P);
-  g_launches.fetch_add(1);
-  CU_TRY(cudaGetLastError());
-  if (prof) {
-    CU_TRY(cudaEventRecord((*h->prof_events)[h->prof_used + 1], st));
-    h->prof_used += 2;
-  }
-  if (cmvn_mode == LIDFE_CMVN_PER_UTT || cmvn_mode == LIDFE_POST_TOPDB)
-    return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, nullptr, st, cmvn_mode == LIDFE_CMVN_PER_UTT ? 1 : 2, P.parity);
-  CU_TRY(cudaEventRecord(p->blk->ev, st));
-  return LIDFE_OK;
+  const bool parity = r.apply == kApplyUtt || r.apply == kApplyTopDb;
+  const int normalize = r.apply == kApplyTopDb ? 2 : r.apply == kApplyMasks ? 0 : 1;
+  return launch_apply(h, p, out_dev, out_ld, masks_dev, n_masks, r.apply == kApplyGlobal ? stats_in_dev : nullptr, st,
+                      normalize, parity ? P.parity : -1);
 }
 
 int lidfe_featurize(lidfe_handle h, lidfe_plan p, const void* wav_dev, float* out_dev, long long out_ld,
@@ -1565,13 +1558,16 @@ int lidfe_cmvn_apply(lidfe_handle h, lidfe_plan p, float* feats_dev, long long l
 
 int lidfe_profile_begin(lidfe_handle h, int max_launches) {
   if (!h) return LIDFE_E_NULL;
-  if (max_launches <= 0 || h->prof_events) return LIDFE_E_ARG;
-  h->prof_events = new (std::nothrow) std::vector<cudaEvent_t>(static_cast<size_t>(max_launches) * 2);
-  if (!h->prof_events) return LIDFE_E_NOMEM;
+  if (max_launches <= 0 || !h->prof_events.empty()) return LIDFE_E_ARG;
+  try {
+    h->prof_events.assign(static_cast<size_t>(max_launches) * 2, nullptr);
+  } catch (const std::bad_alloc&) {
+    return LIDFE_E_NOMEM;
+  }
   h->prof_used = 0;
   h->prof_calls = 0;
   if (h->prof_stride <= 0) h->prof_stride = 1;
-  for (auto& ev : *h->prof_events) CU_TRY(cudaEventCreate(&ev));
+  for (auto& ev : h->prof_events) CU_TRY(cudaEventCreate(&ev));
   return LIDFE_OK;
 }
 
@@ -1584,19 +1580,18 @@ int lidfe_profile_set_stride(lidfe_handle h, int stride) {
 
 int lidfe_profile_end(lidfe_handle h, float* ms_host, int capacity, int* n_out) {
   if (!h || !n_out) return LIDFE_E_NULL;
-  if (!h->prof_events) return LIDFE_E_ARG;
+  if (h->prof_events.empty()) return LIDFE_E_ARG;
   const int n = h->prof_used / 2;
   int rc = LIDFE_OK;
   for (int i = 0; i < n && rc == LIDFE_OK; ++i) {
-    cudaError_t e = cudaEventSynchronize((*h->prof_events)[2 * i + 1]);
+    cudaError_t e = cudaEventSynchronize(h->prof_events[2 * i + 1]);
     float ms = 0.f;
-    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, (*h->prof_events)[2 * i], (*h->prof_events)[2 * i + 1]);
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, h->prof_events[2 * i], h->prof_events[2 * i + 1]);
     if (e != cudaSuccess) rc = static_cast<int>(e);
     if (ms_host && i < capacity) ms_host[i] = ms;
   }
-  for (auto& ev : *h->prof_events) cudaEventDestroy(ev);
-  delete h->prof_events;
-  h->prof_events = nullptr;
+  for (cudaEvent_t ev : h->prof_events) cudaEventDestroy(ev);
+  h->prof_events.clear();
   h->prof_used = 0;
   *n_out = n;
   return rc;
@@ -1628,15 +1623,7 @@ int lidfe_add_noise(lidfe_handle h, lidfe_plan p, const void* wav_in_dev, int in
   if (bank_dev && !noise_tab_dev) return LIDFE_E_NULL;
   if (p->ctx != h || wav_in_dev == static_cast<const void*>(wav_out_dev) || (in_i16 != 0 && in_i16 != 1)) return LIDFE_E_ARG;
   if (bank_dev && (bank_len <= 0 || bank_dev == wav_out_dev)) return LIDFE_E_ARG;
-  WaveParams W;
-  memset(&W, 0, sizeof(W));
-  W.in = wav_in_dev;
-  W.in_i16 = in_i16;
-  W.in_scale = in_scale;
-  W.out = wav_out_dev;
-  W.offsets = p->d_offsets;
-  W.lengths = p->d_lengths;
-  W.normalize = normalize ? 1 : 0;
+  WaveParams W = wave_params(p, wav_in_dev, in_i16, in_scale, wav_out_dev, normalize ? 1 : 0);
   W.bank = bank_dev;
   W.bank_len = bank_len;
   W.noise_tab = noise_tab_dev;

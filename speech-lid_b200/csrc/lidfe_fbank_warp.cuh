@@ -22,12 +22,9 @@
 //     are folded into lane-owned fp64 accumulators in the warp's shared memory every kFoldQuads quads; they leave the
 //     warp with fp64 atomics when the utterance changes (per-utterance mode) or once per CTA at the end (global mode).
 //     The statistics-free instantiation (kStats = false) carries none of those registers.
-// Scope: KALDI framing (kStdMel 0 / 1) and the reference's default branch -- CENTER framing, HTK mel, 10 log10, per-utterance
-// extrema for AmplitudeToDB(top_db) (kStdMel 2) with a pad of a multiple of 16 bytes of input (4 float / 8 int16 samples)
-// --, 16-byte aligned utterances, cmvn modes none / per-utterance statistics /
-// global apply / global accumulate / top_db, fbank output (the MFCC two-kernel path uses it with the tile-blocked workspace
-// layout).  Everything else (in-kernel dither / normalize_wav, in-kernel DCT, unaligned offsets, generic CENTER configs) stays
-// with fbank_kernel.
+// Scope: route_for in lidfe_abi.cu decides which calls run here (handle_can_warp, plan_can_warp); fbank_kernel takes the
+// rest.  kStdMel 0 / 1 serve KALDI framing, kStdMel 2 the reference's default branch (CENTER framing, HTK mel, 10 log10,
+// per-utterance extrema for AmplitudeToDB(top_db)); the MFCC two-kernel path uses the tile-blocked workspace layout.
 #pragma once
 #include "lidfe_kernels.cuh"
 

@@ -3,7 +3,7 @@ fp64 evaluation of the same operation.
 
 liblidfe.so compiles fbank_warp_kernel<TIn, kStdMel, kStats>, fbank_kernel<TIn, kMfcc, kStdMel> and
 fbank_precise_kernel<TIn, kCenter> for several template arguments.  The input type, the mel bank, the statistics, the
-framing, the pad and the alignment choose one of them at run time (lidfe_create's warp_ok, featurize_impl).  Each row of
+framing, the pad and the alignment choose one of them at run time (route_for in lidfe_abi.cu).  Each row of
 ROUTES names a configuration, a call and the exact kernels that call must launch; the GPU test checks that those kernels
 ran (torch.profiler) and that what they computed matches the fp64 references of oracle.frontend_oracle:
 
@@ -48,12 +48,13 @@ def PR(t, center):
     return "fbank_precise_kernel<%s, %s>" % (t, "true" if center else "false")
 
 
-def _route(rid, kw, mode, kernels, env=None, raw=False, abi_ceps=0):
+def _route(rid, kw, mode, kernels, env=None, raw=False, abi_ceps=0, shift=0):
     """kw: FrontEnd kwargs.  mode: none / utt / accum / apply / topdb (the C ABI's cmvn modes; every call goes through
     lidfe_featurize, so the melspec rows may use the modes FrontEnd.featurize_packed refuses).  env: LIDFE_WARP_KERNEL at
     creation.  raw: lidfe_featurize_raw (normalize_wav fused into the load).  abi_ceps: a melspec handle re-created with
-    that many cepstra, which FrontEnd(kind="melspec_db") never builds."""
-    return dict(id=rid, kw=kw, mode=mode, kernels=frozenset(kernels), env=env, raw=raw, abi_ceps=abi_ceps)
+    that many cepstra, which FrontEnd(kind="melspec_db") never builds.  shift: every utterance starts that many samples
+    past a 16-byte boundary of the packed buffer."""
+    return dict(id=rid, kw=kw, mode=mode, kernels=frozenset(kernels), env=env, raw=raw, abi_ceps=abi_ceps, shift=shift)
 
 
 _I16 = dict(in_dtype=torch.int16, in_scale=I16_SCALE)
@@ -77,11 +78,14 @@ ROUTES = [
     _route("k80_cta", {}, "none", [CTA(F32, False, 1)], env="0"),
     _route("k80_cta_utt", {}, "utt", [CTA(F32, False, 1), APPLY], env="0"),
     _route("k80_raw", {}, "none", [WAVE0, CTA(F32, False, 1)], raw=True),
+    _route("k80_unaligned", {}, "none", [CTA(F32, False, 1)], shift=1),
+    _route("k80_dither", dict(dither=0.05, seed=0x1234567811), "none", [CTA(F32, False, 1)]),
     _route("k80_i16_raw", _I16, "none", [WAVE0, CTA(I16, False, 1)], raw=True),
     _route("k40_cta", dict(n_mels=40), "none", [CTA(F32, False, 0)], env="0"),
     _route("k40_i16_cta", dict(n_mels=40, **_I16), "none", [CTA(I16, False, 0)], env="0"),
     _route("mfcc40", dict(n_ceps=40), "none", [W(F32, 1, 0), DCT]),
     _route("mfcc40_i16", dict(n_ceps=40, **_I16), "none", [W(I16, 1, 0), DCT]),
+    _route("mfcc40_raw", dict(n_ceps=40), "none", [WAVE0, CTA(F32, False, 1), DCT], raw=True),
     _route("mfcc40_utt", dict(n_ceps=40), "utt", [CTA(F32, True, 1), APPLY]),
     _route("mfcc40_i16_utt", dict(n_ceps=40, **_I16), "utt", [CTA(I16, True, 1), APPLY]),
     _route("mfcc60", dict(n_ceps=60), "none", [CTA(F32, True, 1)]),
@@ -94,6 +98,7 @@ ROUTES = [
     _route("mel_p300", dict(pad=300, **_MEL), "topdb", [W(F32, 2, 2), APPLY]),
     _route("mel_topdb20", dict(pad=0, top_db=20.0, **_MEL), "topdb", [W(F32, 2, 2), APPLY]),
     _route("mel_p2", dict(pad=2, **_MEL), "topdb", [CTA(F32, False, 2), APPLY]),
+    _route("mel_p0_unaligned", dict(pad=0, **_MEL), "topdb", [CTA(F32, False, 2), APPLY], shift=1),
     _route("mel_n64", dict(pad=0, n_mels=64, **_MEL), "topdb", [CTA(F32, False, 0), APPLY]),
     _route("mel_i16_p0", dict(pad=0, **_MEL, **_I16), "topdb", [W(I16, 2, 2), APPLY]),
     _route("mel_i16_p4", dict(pad=4, **_MEL, **_I16), "topdb", [CTA(I16, False, 2), APPLY]),
@@ -273,6 +278,17 @@ def _modes():
             "accum": _lib.CMVN_ACCUM_GLOBAL, "topdb": _lib.POST_TOPDB}
 
 
+def _plan(fe, route, lens, padded):
+    """fe.make_plan; a route with a shift starts every utterance that many samples past its 16-byte boundary."""
+    if not route["shift"]:
+        return fe.make_plan(lens, padded=padded)
+    offsets, pos = [], 0
+    for n in lens:
+        offsets.append(pos + route["shift"])
+        pos += (route["shift"] + n + fe.align - 1) // fe.align * fe.align
+    return fe.make_plan(lens, padded=padded, offsets=offsets)
+
+
 def _call(fe, route, plan, packed, mode, ld=None, out=None, masks=None, stats_in=None, stats_out=None):
     """One lidfe_featurize(_raw) call; returns the (rows, ld) output."""
     from speech_lid_b200 import _lib
@@ -345,21 +361,26 @@ def _check_raw(lid, route, fe, wavs, kinds, plan, packed, raw):
     lin = None
     if fe.n_ceps and not kw.get("precise"):
         # the device's own log-mels (same configuration without cepstra) x DCT x lifter in fp64
-        fb_route = dict(route, abi_ceps=0, kw={k: v for k, v in kw.items() if k != "n_ceps"}, raw=False)
+        fb_route = dict(route, abi_ceps=0, kw={k: v for k, v in kw.items() if k != "n_ceps"})
         fb = _frontend(lid, fb_route)
-        plan_f = fb.make_plan(plan.lengths, padded=True)
+        plan_f = _plan(fb, fb_route, plan.lengths, True)
         logmel = _call(fb, fb_route, plan_f, packed, "none").double()
         from speech_lid_b200 import tables
         lin = (logmel @ tables.dct_matrix(fe.n_ceps, fe.n_mels).to(fe.device).double()) * \
             tables.lifter(fe.n_ceps, 22.0).to(fe.device).double()
         lin = lin.cpu()
+    if kw.get("dither"):
+        # in-kernel dither: the references see wav + dither * U, U the device's own draw (as in test_gpu_round2.py)
+        u = fe.wave_stages(torch.zeros(plan.total_samples, device=fe.device), plan, dither=1.0).cpu()
+        amp = torch.tensor(kw["dither"], dtype=torch.float32)
+        wavs = [x + amp * u[o:o + x.shape[-1]] for x, o in zip(wavs, plan.offsets)]
     for i, (x, kind) in enumerate(zip(wavs, kinds)):
         got = _rows(raw, plan, i).cpu()
         what = "%s utt %d (%s, %d samples)" % (route["id"], i, kind, x.shape[-1])
         assert torch.isfinite(got).all(), what
         ref, tru = _references(route, fe, x)
         assert got.shape == ref.shape == tru.shape, (what, got.shape, ref.shape)
-        if kind == "zeros" and not fe.n_ceps:
+        if kind == "zeros" and not fe.n_ceps and not kw.get("dither"):
             floor = -100.0 if melspec else float(torch.tensor(O.EPS32).log())
             assert torch.all(got == floor), "%s: silence is not exactly %r" % (what, floor)
             assert torch.equal(got, ref), what
@@ -426,8 +447,8 @@ def test_route(lid, route):
     mode = route["mode"]
     stat_mode = mode in ("utt", "accum")          # fp64 atomics: the sums' order varies between launches
     tol = 2e-6 if stat_mode else 0.0
-    plan = fe.make_plan(lens, padded=True)
-    plan_p = fe.make_plan(lens, padded=False)
+    plan = _plan(fe, route, lens, True)
+    plan_p = _plan(fe, route, lens, False)
     assert plan.frames == [fe.num_frames(n) for n in lens]
     packed = fe.pack(wavs, plan)
     packed_p = fe.pack(wavs, plan_p)
@@ -440,7 +461,7 @@ def test_route(lid, route):
         raw = _call(fe, route, plan, packed, "accum")
     elif mode == "topdb":
         fe_inf = _frontend(lid, route, top_db=float("inf"))      # same kernel; the clamp never bites
-        raw = _call(fe_inf, route, fe_inf.make_plan(lens, padded=True), packed, "topdb")
+        raw = _call(fe_inf, route, _plan(fe_inf, route, lens, True), packed, "topdb")
     else:       # apply
         raw = _call(fe, route, plan, packed, "none")
         stats_in = O.cmvn_stats([_rows(raw, plan, i).cpu() for i in range(len(lens))]).to(fe.device)
