@@ -113,13 +113,7 @@ __global__ void __launch_bounds__(kWThreads, kWCtasPerSm) fbank_warp_kernel(cons
   }
   if (kSums)
     for (int e = lane; e < 2 * kMaxMels; e += 32) acc_s[e] = 0.0;
-  if (mode == 2 && tid < n_out) {
-    const double n = P.stats_in[2 * n_out];
-    const double mean = P.stats_in[tid] / n;
-    double var = (P.stats_in[n_out + tid] - P.stats_in[tid] * mean) / (n - 1.0);
-    var = var > 0.0 ? var : 0.0;
-    sm_norm[tid] = make_float2(static_cast<float>(mean), static_cast<float>(1.0 / (sqrt(var) + 1e-9)));
-  }
+  if (mode == 2 && tid < n_out) sm_norm[tid] = global_cmvn(P, n_out, tid);
   __syncthreads();
 
   // ---- this warp's schedule: its static run of spans [w_first[gw], w_first[gw + 1]), then claims from the pool ----------

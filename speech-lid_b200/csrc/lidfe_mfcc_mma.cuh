@@ -120,16 +120,7 @@ __global__ void __launch_bounds__(kMmThreads, 2) mfcc_dct_mma_kernel(const __gri
   }
   if (tid < kDctMaxCeps) {
     s_lift[tid] = tid < nc ? P.lifter[tid] : 0.f;
-    float mean = 0.f, inv = 1.f;
-    if (P.mode == 2 && tid < nc) {
-      const double n = P.stats_in[2 * nc];
-      const double mu = P.stats_in[tid] / n;
-      double var = (P.stats_in[nc + tid] - P.stats_in[tid] * mu) / (n - 1.0);
-      var = var > 0.0 ? var : 0.0;
-      mean = static_cast<float>(mu);
-      inv = static_cast<float>(1.0 / (sqrt(var) + 1e-9));
-    }
-    s_norm[tid] = make_float2(mean, inv);
+    s_norm[tid] = (P.mode == 2 && tid < nc) ? global_cmvn(P, nc, tid) : make_float2(0.f, 1.f);
   }
   __syncthreads();
 
