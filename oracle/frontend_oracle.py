@@ -379,6 +379,37 @@ def truth64_melspec_db(x: torch.Tensor, pad: int = 0, top_db: Optional[float] = 
     return torch.maximum(db, db.max() - top_db)
 
 
+def truth64_resample(x: torch.Tensor, kernel32: torch.Tensor, width: int, orig: int, new: int) -> torch.Tensor:
+    """``resample`` of one utterance in float64 on the fp32 FIR bank ``kernel32`` ((new/g, 2 width + orig/g), g the gcd):
+    output sample i * new + p is  sum_k kernel32[p][k] * xpad[i * orig + k],  xpad = x with ``width`` zeros in front and
+    width + orig behind, cut to ceil(new * n / orig) samples.  Runs on x's device."""
+    g = math.gcd(int(orig), int(new))
+    orig, new = int(orig) // g, int(new) // g
+    w = x.reshape(-1).double()
+    k = kernel32.to(w.device).double()
+    assert k.shape[0] == new and k.shape[1] == 2 * width + orig
+    xp = torch.nn.functional.pad(w, (width, width + orig))
+    y = (xp.unfold(0, k.shape[1], orig) @ k.T).reshape(-1)
+    return y[:-(-new * w.numel() // orig)]
+
+
+def truth64_s3prl_fbank(x: torch.Tensor, fbank_size: int = 80, n_fft: int = 640, normalize: bool = True) -> torch.Tensor:
+    """``s3prl_fbank`` in float64 on the reference's fp32 tables (``torch.hann_window(n_fft)``, ``melscale_fbanks``):
+    spectrogram (center=False, hop n_fft / 2, power 2) -> HTK mel -> 10 log10(max(., 1e-10)) -> (x - mean) / (std + 1e-9)
+    with one mean / unbiased std over the whole spectrogram.  (frames, fbank_size), on x's device."""
+    w = x.reshape(-1).double()
+    window = torch.hann_window(n_fft).double().to(w.device)
+    spec = torch.stft(w, n_fft=n_fft, hop_length=n_fft // 2, win_length=n_fft, window=window, center=False,
+                      normalized=False, onesided=True, return_complex=True)
+    power = spec.real ** 2 + spec.imag ** 2                                      # (n_fft/2+1, frames)
+    fb = htk_mel_fbanks(n_fft // 2 + 1, 0.0, 8000.0, fbank_size, 16000).double().to(w.device)
+    db = 10.0 * torch.log10((power.T @ fb).clamp_min(1e-10))
+    if not normalize:
+        return db
+    std, mean = torch.std_mean(db)
+    return (db - mean) / (std + 1e-9)
+
+
 # --------------------------------------------------------------------------------------
 # Synthetic inputs (SURVEY.md §8d).  Deterministic; used by tests, golden generation and bench.
 # --------------------------------------------------------------------------------------

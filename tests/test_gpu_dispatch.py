@@ -123,13 +123,13 @@ ROUTES = [
 OTHER_KERNELS = {
     "cmvn_apply_kernel": "tests/test_gpu_dispatch.py (second stage, masks, strided rows)",
     "mfcc_dct_mma_kernel": "tests/test_gpu_dispatch.py, test_gpu_parity.py::test_generic_kernel_variant_configs",
-    "resample_kernel": "test_gpu_round2.py::test_resampler_kernels_agree_tcgen05_fp32",
-    "resample_tc_kernel": "test_gpu_round2.py::test_resampler_kernels_agree_tcgen05_fp32",
+    "resample_kernel": "test_gpu_gemm_routes.py::test_gemm_route",
+    "resample_tc_kernel": "test_gpu_gemm_routes.py::test_gemm_route",
     "wave_stages_kernel<0>": "test_gpu_parity.py::test_wave_stages, tests/test_gpu_dispatch.py (raw rows)",
     "wave_stages_kernel<1>": "test_gpu_noise.py (noise bank)",
     "wave_stages_kernel<2>": "test_gpu_noise.py (Gaussian noise)",
-    "stft_mel_db_kernel": "test_gpu_round2.py::test_s3prl_fbank_variant_matches_reference_module",
-    "scalar_norm_kernel": "test_gpu_round2.py::test_s3prl_fbank_variant_matches_reference_module",
+    "stft_mel_db_kernel": "test_gpu_gemm_routes.py::test_gemm_route (S3prlFBank rows)",
+    "scalar_norm_kernel": "test_gpu_gemm_routes.py::test_gemm_route (S3prlFBank rows)",
     "h2d_gather_kernel": "test_gpu_precise.py::test_h2d_gather_kernel_and_its_fallback",
     "fp32_probe_kernel": "bench roofline probe only",
 }

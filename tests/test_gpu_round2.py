@@ -68,20 +68,6 @@ def fe(lid):
     return lid.FrontEnd(n_mels=80)
 
 
-def _fresh(ctor, env, *args, **kw):
-    """An object created under temporary environment switches (they are read once, at creation)."""
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        return ctor(*args, **kw)
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-
-
 def _fresh_frontend(lid, env, **kw):
     """A FrontEnd created under temporary environment switches (they are read once, at lidfe_create)."""
     old = {k: os.environ.get(k) for k in env}
@@ -294,50 +280,6 @@ def test_s3prl_fbank_variant_matches_reference_module(lid):
         assert float((o.cpu() - want).abs().max() / want.abs().max()) <= 1e-4, w.numel()
     with pytest.raises(RuntimeError):
         fb.forward_list([torch.randn(639)])
-
-
-def _cuda_kernels(fn):
-    """Names of the CUDA kernels that fn() launches (torch.profiler, CUDA activities)."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        out = fn()
-        torch.cuda.synchronize()
-    return out, {e.name for e in prof.events()}
-
-
-@gpu
-@pytest.mark.parametrize("orig", [44100, 22050, 25000, 15000])
-def test_resampler_kernels_agree_tcgen05_fp32(lid, orig):
-    """Row f4: the two kernels behind lidfe_resample -- resample_tc_kernel (tcgen05 + TMEM, 3 x TF32, what a Resampler
-    runs on sm_100 whenever the reduced output rate is a multiple of 16) and the FP32 resample_kernel -- against an fp64
-    evaluation of the same polyphase sum with the same fp32 FIR bank (ta: functional/functional.py
-    _apply_sinc_resample_kernel), on ragged utterances: shorter than one tile, one sample, exact multiples of the period,
-    several 128-frame tiles (the persistent CTA walks them through both TMEM accumulator buffers and wraps the 3-stage
-    pipeline many times).  25 kHz has 16 phases (one 16-column phase tile), 15 kHz 29 taps (a second, all-zero tap
-    block)."""
-    import math
-    g = torch.Generator().manual_seed(orig)
-    lens = [int(orig * s) for s in (0.05, 0.31, 1.0, 2.57, 0.011, 6.3)] + [441, 1, 44101, 441 * 128, 441 * 128 + 1]
-    wavs = [torch.randn(n, generator=g) for n in lens]
-    outs = {}
-    for kind, kernel in (("tc", "resample_tc_kernel"), ("fp32", "resample_kernel")):
-        rs = lid.Resampler(orig, 16000) if kind == "tc" else _fresh(lid.Resampler, {"LIDFE_RESAMPLE_TC": "0"}, orig, 16000)
-        gg = math.gcd(rs.orig_freq, rs.new_freq)
-        o_red = rs.orig_freq // gg
-        k64 = rs.kernel.double()
-        dev = [w.cuda() for w in wavs]
-        res, names = _cuda_kernels(lambda: rs.resample_list(dev))
-        ran_tc = any("resample_tc_kernel" in n for n in names)
-        assert ran_tc == (kind == "tc") and any(kernel in n for n in names), (kind, names)
-        for w, o in zip(wavs, res):
-            x = torch.nn.functional.pad(w.double(), (rs.width, rs.width + o_red))
-            want = (x.unfold(0, k64.shape[1], o_red) @ k64.T).reshape(-1)[:rs.out_len(w.numel())]
-            assert o.numel() == want.numel(), (kind, w.numel())
-            assert float((o.double().cpu() - want).abs().max()) <= 1e-5, (kind, w.numel())
-        outs[kind] = [o.cpu() for o in res]
-    worst = max(float((a - b).abs().max()) for a, b in zip(outs["tc"], outs["fp32"]))
-    assert worst <= 2e-6, worst
 
 
 @gpu

@@ -98,3 +98,67 @@ def test_truth64_mfcc_is_the_oracle_in_fp64(speech, n_ceps, n_mels, preemph):
            ) * O.kaldi_lifter(n_ceps, 22.0).double()
     assert _norm_rel(O.kaldi_mfcc(speech, num_ceps=n_ceps, n_mels=n_mels, preemph=preemph), tru) <= FP32_DISTANCE
     assert math.isfinite(float(tru.abs().max()))
+
+
+# ---- the windowed-GEMM family (tests/test_gpu_gemm_routes.py): resampler and wav2vec-exp FBank ------------------------
+@pytest.mark.parametrize("orig,new", [(44100, 16000), (22050, 16000), (48000, 16000), (8000, 16000), (16000, 44100),
+                                      (88200, 16000)])
+def test_truth64_resample_is_the_oracle_in_fp64(speech, orig, new):
+    kernel, width, _, _ = O.sinc_resample_kernel(orig, new)
+    x = speech[0]
+    tru = O.truth64_resample(x, kernel[:, 0], width, orig, new)
+    ref = O.resample(x, orig, new)
+    assert tru.dtype == torch.float64 and tru.shape == ref.shape
+    assert _norm_rel(ref, tru) <= FP32_DISTANCE
+    # torchaudio's formulation -- a strided conv1d of the padded waveform -- evaluated in float64
+    g = math.gcd(orig, new)
+    xp = torch.nn.functional.pad(x.double(), (width, width + orig // g))
+    conv = torch.nn.functional.conv1d(xp[None, None], kernel.double(), stride=orig // g)[0].T.reshape(-1)[:tru.numel()]
+    assert float((conv - tru).abs().max()) <= 1e-13 * float(tru.abs().max())
+    # every argument matters: the bank, its width, each rate, and the samples themselves
+    other_k, other_w, _, _ = O.sinc_resample_kernel(orig + 50, new)
+    if other_k.shape[0] == kernel.shape[0] and other_k.shape[2] == kernel.shape[2]:
+        assert _norm_rel(O.truth64_resample(x, other_k[:, 0], other_w, orig, new), tru) > 1e-6
+    assert _norm_rel(O.truth64_resample(x, kernel[:, 0] * (1 + 1e-3), width, orig, new), tru) > 1e-4
+    y = x.clone()
+    y[len(y) // 2] += 1.0
+    assert not torch.equal(O.truth64_resample(y, kernel[:, 0], width, orig, new), tru)
+    with pytest.raises(AssertionError):              # a bank of another width or rate pair is refused, not misread
+        O.truth64_resample(x, kernel[:, 0], width + 1, orig, new)
+    with pytest.raises(AssertionError):
+        O.truth64_resample(x, kernel[:, 0], width, orig, new * 2 + 1)
+    assert O.truth64_resample(x[:1], kernel[:, 0], width, orig, new).numel() == -(-(new // g) // (orig // g))
+
+
+@pytest.mark.parametrize("fbank_size,n_fft", [(80, 640), (80, 320), (40, 640), (128, 640), (1, 640), (80, 2048),
+                                              (80, 64), (80, 4)])
+def test_truth64_s3prl_fbank_is_the_oracle_in_fp64(speech, fbank_size, n_fft):
+    x = speech[0]
+    raw = O.truth64_s3prl_fbank(x, fbank_size, n_fft, False)
+    norm = O.truth64_s3prl_fbank(x, fbank_size, n_fft, True)
+    std, mean = torch.std_mean(raw)
+    assert torch.equal(norm, (raw - mean) / (std + 1e-9))
+    for tru, normalize in ((raw, False), (norm, True)):
+        ref = O.s3prl_fbank(x, fbank_size, n_fft, normalize).T
+        assert tru.dtype == torch.float64 and tru.shape == ref.shape == (O.s3prl_fbank_num_frames(x.numel(), n_fft),
+                                                                         fbank_size)
+        # normalising divides the dB values' fp32 error by their std: the distance scales with it
+        dist = FP32_DISTANCE * (float(raw.abs().max() / std / norm.abs().max()) if normalize else 1.0)
+        assert _norm_rel(ref, tru) <= dist, (normalize, _norm_rel(ref, tru), dist)
+    if fbank_size > 1 and n_fft >= 64:
+        assert _norm_rel(O.truth64_s3prl_fbank(x, fbank_size - 1 if fbank_size > 2 else 3, n_fft, False)[:, -1:],
+                         raw[:, -1:]) > 1e-3
+    if n_fft >= 64:
+        other = O.truth64_s3prl_fbank(x, fbank_size, n_fft - 2, False)
+        assert other.shape != raw.shape or _norm_rel(other, raw) > 1e-4
+    if n_fft == 4:                      # three bins under 80 triangles: empty filters floor at exactly -100 dB
+        assert bool((raw == -100.0).all(0).any())
+
+
+def test_truth64_s3prl_fbank_silence_and_one_value():
+    z = O.truth64_s3prl_fbank(torch.zeros(6400), 80, 640, False)
+    assert torch.equal(z, torch.full((19, 80), -100.0, dtype=torch.float64))
+    assert torch.equal(O.truth64_s3prl_fbank(torch.zeros(6400), 80, 640, True), torch.zeros(19, 80, dtype=torch.float64))
+    one = O.truth64_s3prl_fbank(torch.randn(640, generator=torch.Generator().manual_seed(2)), 1, 640, True)
+    assert one.shape == (1, 1) and bool(torch.isnan(one).all())            # torch.std of one value
+    assert bool(torch.isnan(O.s3prl_fbank(torch.randn(640), 1, 640)).all())
